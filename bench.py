@@ -2,6 +2,7 @@
 """bench.py — the hot path of spalinalg on B200, BASELINE.json's metric.
 
   python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload NAME]
+                  [--dump-outputs DIR]
 
 ONE workload at every N: config 5 of BASELINE.json (banded, offsets -4..+4, n = 1e8, 9e8 stored
 entries, f64; 12.4 GB algorithmic per product, inputs far larger than L2, so no flush is needed).
@@ -25,6 +26,11 @@ changes every step with one rank delayed).  The line also carries, as named extr
 transposes + Gustavson) on the host: the oracle's line-by-line port (the reference is Rust; no rustc
 in this image: cpu_baseline.kind = "port"), one core because the reference is single-threaded, on a
 bounded sample of the same workload (the same banded matrix at n = 1e7).
+
+--dump-outputs DIR writes the product of the last timed step, y, as DIR/y.npy (f64): every row while y
+has at most DUMP_ROWS of them, else a fixed sample (the first and last 4096 rows and a seeded uniform
+draw), whose row numbers go to DIR/y_rows.npy.  Matrix and x are deterministic, so two builds run with
+the same arguments can be compared output for output.
 """
 from __future__ import annotations
 
@@ -277,6 +283,41 @@ def x_values(torch, wl, lo, hi):
     return (1.0 / (1.0 + (idx % 97))).to(torch.float64)
 
 
+DUMP_ROWS = 1 << 21      # rows of y --dump-outputs writes at most: 16 MB of f64 values, 16 MB of row numbers
+
+
+def dump_rows(n):
+    """Rows of y that --dump-outputs writes, ascending: all n while n <= DUMP_ROWS, else the first and last
+    4096 rows and a seeded uniform draw, the same in every build and at every rank count."""
+    if n <= DUMP_ROWS:
+        return np.arange(n)
+    edges = np.concatenate([np.arange(4096), np.arange(n - 4096, n)])
+    return np.unique(np.concatenate([edges, np.random.default_rng(0).integers(0, n, DUMP_ROWS - edges.size)]))
+
+
+def last_step_output(torch, dist, y, n, r0, rank, world):
+    """(rows, y[rows]) of the whole product, rows = dump_rows(n), gathered bit for bit from the row blocks
+    [r0, r1) of sharding.row_partition that the ranks hold."""
+    from spalinalg_b200 import sharding
+    rows = dump_rows(n)
+    bounds = np.searchsorted(rows, [sharding.row_partition(n, world, g)[0] for g in range(world)] + [n])
+    counts = np.diff(bounds)
+    mine = torch.zeros(int(counts.max()), dtype=y.dtype, device=y.device)
+    mine[:counts[rank]] = y[torch.from_numpy(rows[bounds[rank]:bounds[rank + 1]] - r0).to(y.device)]
+    parts = [mine]
+    if world > 1:
+        parts = [torch.empty_like(mine) for _ in range(world)]
+        dist.all_gather(parts, mine)
+    return rows, torch.cat([p[:c] for p, c in zip(parts, counts)]).cpu().numpy()
+
+
+def write_outputs(path, n, rows, y):
+    os.makedirs(path, exist_ok=True)
+    np.save(os.path.join(path, "y.npy"), y)
+    if rows.size < n:
+        np.save(os.path.join(path, "y_rows.npy"), rows.astype(np.float64))      # exact below 2^53
+
+
 def parity_check(torch, dist, sp, spd, ctx, rank, world):
     """A small problem sharded over the SAME ranks, against the CPU oracle (the checker, never the thing
     measured): sharded assembly bit-exact, sharded SpMV within 1e-12, sharded add bit-exact, and the
@@ -358,7 +399,13 @@ def main():
     ap.add_argument("--workload", default="auto", choices=["auto"] + list(WORKLOADS))
     ap.add_argument("--kernel", default="auto")       # auto | vectorN | stream | merge  (N = 1 only)
     ap.add_argument("--no-extras", action="store_true", help="skip secondary metrics / cpu baseline / parity check")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write y of the last timed step as DIR/y.npy (a fixed sample of its rows when "
+                                                          "it is large, their numbers in DIR/y_rows.npy)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the device product (--impl ours)")
     args.warmup = max(args.warmup, 3)
 
     if args.impl == "reference":
@@ -489,6 +536,7 @@ def main():
     value = bytes_total / (ms_step * 1e-3) / 1e9
     if xv is not None:
         xv.check()
+    dumped = last_step_output(torch, dist, y, n, r0, rank, world) if args.dump_outputs else None
 
     # SpMV-kernel-only time on this rank (roofline of the dominant kernel)
     barrier()
@@ -609,6 +657,8 @@ def main():
         if cpu:
             line["cpu_baseline"] = cpu
         line.update(extras)
+        if dumped is not None:
+            write_outputs(args.dump_outputs, n, *dumped)
         print(json.dumps(line), flush=True)
     if world > 1:
         dist.barrier()
