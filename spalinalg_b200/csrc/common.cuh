@@ -39,6 +39,8 @@ constexpr int kNumSmFallback = 148;
 // 32-bit positions: kernels step a position by up to a tile (<= 65536 entries) past the last entry
 // before testing it, so entry counts stay that far below 2^32.
 constexpr uint64_t kMaxEntries = (1ull << 32) - 65536;
+// longest row whose column offsets the SpMV plan keeps as the matrix's row pattern (spl_mat::pattern_off)
+constexpr uint32_t kPatternMax = 64;
 
 }  // namespace spl
 
@@ -126,6 +128,16 @@ struct spl_mat {
     // tile's first stored entry (same layout, one more slot per CTA)
     uint32_t *stream_cta_rows = nullptr, *stream_xhi = nullptr, *stream_xlo0 = nullptr, *stream_tile_lo = nullptr;
     uint32_t stream_rows = 0, stream_cap = 0, stream_grid = 0, stream_max_tiles = 0;
+    // row pattern (plan; depends on ptr and ind only): pattern_len = K = max_row_len when 0 < K <= kPatternMax and
+    // some row r at or after nrows / 2 has K entries; pattern_off[j] = ind[ptr[r] + j] - r (mod 2^32) for the first
+    // such r (a shard's local matrix: local rows, global columns, offsets shifted by its first row).  A stream
+    // tile is regular when each of its rows r has K entries at columns r + pattern_off[j]: the stream kernel
+    // then fetches its values only.  stream_tile_reg[slot] = 1 for a regular tile (layout of stream_tile_lo),
+    // stream_regular = how many tiles of the grid are regular.
+    uint32_t pattern_off[spl::kPatternMax] = {};
+    uint32_t pattern_len = 0;
+    uint32_t *stream_tile_reg = nullptr;
+    uint32_t stream_regular = 0;
 
     // CSR form of a CSC matrix (same matrix, other format), built by the first product y = A x on it
     // and kept: products on a CscMatrix then run the row kernels at full speed and in the reference's

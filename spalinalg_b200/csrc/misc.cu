@@ -240,6 +240,7 @@ void free_mat(spl_ctx *ctx, spl_mat *m) {
     dfree(ctx, m->stream_cta_rows);
     dfree(ctx, m->stream_xlo0);
     dfree(ctx, m->stream_tile_lo);
+    dfree(ctx, m->stream_tile_reg);
     delete m;
 }
 

@@ -544,14 +544,23 @@ __global__ void stream_partition_kernel(const uint32_t *__restrict__ ptr, uint32
     if (b < grid) atomicMax(max_tiles, (first_row(b + 1) - r0 + rows_per_tile - 1) / rows_per_tile);
 }
 
+// The matrix's row pattern as a kernel parameter (spl_mat::pattern_off / pattern_len; len 0: none).
+struct RowPattern {
+    uint32_t off[kPatternMax];
+    uint32_t len;
+};
+
 // Per CTA b, slots [b * (max_tiles + 1) ...]: tile_lo[k] = position of tile k's first stored entry
 // (k = number of tiles: the end of the range); xhi[k] = 1 + the largest column of tile k (rows are
 // column-sorted: the last entry of a row), 0 if the tile has no entry; xlo0[b] = the smallest column of
-// the CTA's first tile.
+// the CTA's first tile.  With a row pattern: reg[k] = 1 when tile k is regular (every row r has pat.len
+// entries at columns r + pat.off[j]), and *regular counts the regular tiles of the grid.  reg and xhi
+// arrive zeroed.
 __global__ void stream_edges_kernel(const uint32_t *__restrict__ ptr, const uint32_t *__restrict__ ind,
                                     const uint32_t *__restrict__ cta_rows, uint32_t rows_per_tile, uint32_t max_tiles,
                                     uint32_t *__restrict__ tile_lo, uint32_t *__restrict__ xhi,
-                                    uint32_t *__restrict__ xlo0) {
+                                    uint32_t *__restrict__ xlo0, const __grid_constant__ RowPattern pat,
+                                    uint32_t *__restrict__ reg, uint32_t *__restrict__ regular) {
     const uint32_t b = blockIdx.x;
     const uint32_t rs = cta_rows[b], re = cta_rows[b + 1];
     const size_t base = (size_t)b * (max_tiles + 1);
@@ -561,40 +570,63 @@ __global__ void stream_edges_kernel(const uint32_t *__restrict__ ptr, const uint
     }
     for (uint32_t r = rs + threadIdx.x; r < re; r += blockDim.x) {
         const uint32_t lo = ptr[r], hi = ptr[r + 1];
-        if (hi == lo) continue;
         const uint32_t k = (r - rs) / rows_per_tile;
+        if (pat.len) {                                  // reg[] holds "irregular" until the pass below
+            bool fits = hi - lo == pat.len;
+            for (uint32_t j = 0; fits && j < pat.len; ++j) fits = ind[lo + j] == r + pat.off[j];
+            if (!fits) reg[base + k] = 1u;
+        }
+        if (hi == lo) continue;
         atomicMax(xhi + base + k, ind[hi - 1] + 1u);
         if (k == 0) atomicMin(xlo0 + b, ind[lo]);
     }
+    if (!pat.len) return;
+    __syncthreads();
+    const uint32_t ntiles = (re - rs + rows_per_tile - 1) / rows_per_tile;
+    uint32_t count = 0;
+    for (uint32_t k = threadIdx.x; k < ntiles; k += blockDim.x) {
+        const uint32_t fits = reg[base + k] ^ 1u;
+        reg[base + k] = fits;
+        count += fits;
+    }
+    if (count) atomicAdd(regular, count);
 }
 
 constexpr int ST_CONSUMERS = 256;
 
 // TIGHT: registers held to 56 so that four CTAs fit on an SM; otherwise three CTAs with room for
 // eight f64 gathers and values in flight per lane.
-template <typename T, int LPR, int U, bool TIGHT, typename XG>
+// PAT: the grid has regular tiles (stream_edges_kernel).  Their columns and row starts follow from the row
+// number and the row pattern, so the producer fetches only their values; the consumers take column
+// r + pat.off[j] for position j of row r, and everything else runs as on any tile (same bits).
+template <typename T, int LPR, int U, bool TIGHT, bool PAT, typename XG>
 __global__ void __launch_bounds__(ST_CONSUMERS + 32, TIGHT ? 4 : 3)
 spmv_stream_kernel(uint32_t nrows, const uint32_t *__restrict__ ptr, const uint32_t *__restrict__ ind,
                    const T *__restrict__ val, const XG xg, T *__restrict__ y, const uint32_t *__restrict__ cta_rows,
                    const uint32_t *__restrict__ tile_lo, const uint32_t *__restrict__ xhi,
                    const uint32_t *__restrict__ xlo0, uint32_t max_tiles, uint32_t cap, uint32_t stages,
-                   const T *__restrict__ x_edge, uint32_t x_lo, uint32_t x_hi, int l2_hint) {
+                   const T *__restrict__ x_edge, uint32_t x_lo, uint32_t x_hi, int l2_hint,
+                   const uint32_t *__restrict__ tile_reg, const __grid_constant__ RowPattern pat) {
     constexpr uint32_t CONS = ST_CONSUMERS;
     constexpr uint32_t R = CONS / LPR;
     constexpr uint32_t PTRS = R + 4;           // pointer slots per stage: R + 1 needed, whole 16-byte units
     extern __shared__ __align__(128) unsigned char st_raw[];
-    // per stage: [cap] indices, [cap] values, [PTRS] row pointers; then the barriers
+    // per stage: [cap] indices, [cap] values, [PTRS] row pointers; then the barriers; with PAT one word per
+    // stage (the first entry position of a regular tile, ~0 for any other) and the row pattern
     uint32_t *s_ind = reinterpret_cast<uint32_t *>(st_raw);
     T *s_val = reinterpret_cast<T *>(st_raw + (size_t)stages * cap * sizeof(uint32_t));
     uint32_t *s_ptr = reinterpret_cast<uint32_t *>(st_raw + (size_t)stages * cap * (sizeof(uint32_t) + sizeof(T)));
     uint64_t *full = reinterpret_cast<uint64_t *>(s_ptr + (size_t)stages * PTRS);
     uint64_t *empty = full + stages;
+    uint32_t *s_reg_lo = reinterpret_cast<uint32_t *>(empty + stages);
+    uint32_t *s_pat = s_reg_lo + stages;
     if (threadIdx.x == 0) {
         for (uint32_t s = 0; s < stages; ++s) {
             mbar_init(full + s, 1);
             mbar_init(empty + s, CONS / 32);
         }
     }
+    if (PAT && threadIdx.x < pat.len) s_pat[threadIdx.x] = pat.off[threadIdx.x];
     __syncthreads();
     const uint32_t rs = __ldg(cta_rows + blockIdx.x), re = __ldg(cta_rows + blockIdx.x + 1);
     const uint32_t ntiles = (re - rs + R - 1) / R;
@@ -603,7 +635,7 @@ spmv_stream_kernel(uint32_t nrows, const uint32_t *__restrict__ ptr, const uint3
         // ---- producer: one thread, up to S tiles ahead of the consumers ----
         if (threadIdx.x != CONS || ntiles == 0) return;
         const size_t base = (size_t)blockIdx.x * (max_tiles + 1);
-        const uint32_t *t_lo = tile_lo + base, *t_xhi = xhi + base;
+        const uint32_t *t_lo = tile_lo + base, *t_xhi = xhi + base, *t_reg = tile_reg + base;
         uint32_t s = 0, phase = 0;
         uint32_t edge = __ldg(xlo0 + blockIdx.x);                 // x below this is somebody else's first touch
         uint32_t lo = __ldg(t_lo);
@@ -613,16 +645,20 @@ spmv_stream_kernel(uint32_t nrows, const uint32_t *__restrict__ ptr, const uint3
             if (k >= stages) mbar_wait(empty + s, phase ^ 1u);     // the consumers are done with this stage
             const uint32_t za = lo & ~3u, zb = (hi + 3u) & ~3u;    // 16-byte aligned superset; the arrays carry slack
             const uint32_t cnt = zb - za;
+            // a regular tile: no pointer or index slice, its first entry position goes through the stage
+            const bool regular = PAT && __ldg(t_reg + k);
+            if (PAT) s_reg_lo[s] = regular ? lo : ~0u;             // published by the arrive below (release)
             const uint32_t r0 = rs + k * R;                        // multiple of 4
             const uint32_t left = (nrows + 1u - r0 + 3u) & ~3u;    // pointer entries from r0 to the end (+ slack)
-            const uint32_t np = left < PTRS ? left : PTRS;
-            mbar_expect_tx(full + s, cnt * (uint32_t)(sizeof(uint32_t) + sizeof(T)) + np * (uint32_t)sizeof(uint32_t));
-            tma_bulk_g2s(s_ptr + (size_t)s * PTRS, ptr + r0, np * (uint32_t)sizeof(uint32_t), full + s);
+            const uint32_t np = regular ? 0u : left < PTRS ? left : PTRS;
+            const uint32_t ni = regular ? 0u : cnt;
+            mbar_expect_tx(full + s, ni * (uint32_t)sizeof(uint32_t) + cnt * (uint32_t)sizeof(T) + np * (uint32_t)sizeof(uint32_t));
+            if (np) tma_bulk_g2s(s_ptr + (size_t)s * PTRS, ptr + r0, np * (uint32_t)sizeof(uint32_t), full + s);
             if (cnt && l2_hint) {
-                tma_bulk_g2s_hint(s_ind + (size_t)s * cap, ind + za, cnt * (uint32_t)sizeof(uint32_t), full + s, pol);
+                if (ni) tma_bulk_g2s_hint(s_ind + (size_t)s * cap, ind + za, ni * (uint32_t)sizeof(uint32_t), full + s, pol);
                 tma_bulk_g2s_hint(s_val + (size_t)s * cap, val + za, cnt * (uint32_t)sizeof(T), full + s, pol);
             } else if (cnt) {
-                tma_bulk_g2s(s_ind + (size_t)s * cap, ind + za, cnt * (uint32_t)sizeof(uint32_t), full + s);
+                if (ni) tma_bulk_g2s(s_ind + (size_t)s * cap, ind + za, ni * (uint32_t)sizeof(uint32_t), full + s);
                 tma_bulk_g2s(s_val + (size_t)s * cap, val + za, cnt * (uint32_t)sizeof(T), full + s);
             }
             if (x_edge && x1 > edge) {                             // leading edge of x -> L2
@@ -654,16 +690,23 @@ spmv_stream_kernel(uint32_t nrows, const uint32_t *__restrict__ ptr, const uint3
         const uint32_t *ci = s_ind + (size_t)s * cap;
         const T *cv = s_val + (size_t)s * cap;
         const uint32_t r = rs + k * R + rl;
-        const uint32_t za = cp[0] & ~3u;
-        uint32_t p0 = 0, e = 0;
-        if (r < re) { p0 = cp[rl] - za; e = cp[rl + 1] - za; }
+        // column of stage position j: cb[j] + cadd (a regular tile: cb = the pattern moved to the row's start)
+        const uint32_t *cb = ci;
+        uint32_t cadd = 0, p0 = 0, e = 0;
+        const uint32_t reg_lo = PAT ? s_reg_lo[s] : ~0u;
+        if (reg_lo != ~0u) {
+            if (r < re) { p0 = (reg_lo & 3u) + rl * pat.len; e = p0 + pat.len; cb = s_pat - p0; cadd = r; }
+        } else {
+            const uint32_t za = cp[0] & ~3u;
+            if (r < re) { p0 = cp[rl] - za; e = cp[rl + 1] - za; }
+        }
         T acc = (T)0;
         auto row_sum = [&](auto gather) {
             for (uint32_t j = p0 + sub; j < e; j += U * LPR) {
                 uint32_t c[U];
                 T xv[U], v[U];
 #pragma unroll
-                for (int u = 0; u < U; ++u) c[u] = j + u * LPR < e ? ci[j + u * LPR] : 0xffffffffu;
+                for (int u = 0; u < U; ++u) c[u] = j + u * LPR < e ? cb[j + u * LPR] + cadd : 0xffffffffu;
 #pragma unroll
                 for (int u = 0; u < U; ++u) xv[u] = c[u] != 0xffffffffu ? gather(c[u]) : (T)0;
 #pragma unroll
@@ -673,7 +716,7 @@ spmv_stream_kernel(uint32_t nrows, const uint32_t *__restrict__ ptr, const uint3
             }
         };
         // the row's columns are sorted: first and last entry bound them
-        if (e <= p0 || xg.all_local(ci[p0], ci[e - 1])) row_sum([&](uint32_t c) { return xg.local(c); });
+        if (e <= p0 || xg.all_local(cb[p0] + cadd, cb[e - 1] + cadd)) row_sum([&](uint32_t c) { return xg.local(c); });
         else row_sum([&](uint32_t c) { return xg(c); });
         __syncwarp();
         if (lane_id() == 0) mbar_arrive(empty + s);
@@ -692,6 +735,12 @@ inline int env_int(const char *name, int fallback) {
 inline int stream_consumers() { return ST_CONSUMERS; }
 inline size_t stream_stage_bytes(const spl_mat *a) {
     return (size_t)a->stream_cap * (4 + a->vsize()) + ((size_t)a->stream_rows + 4) * 4;
+}
+RowPattern row_pattern(const spl_mat *a) {
+    RowPattern p{};
+    std::memcpy(p.off, a->pattern_off, sizeof(p.off));
+    p.len = a->pattern_len;
+    return p;
 }
 
 // Largest window of R rows -> stage capacity in entries (0: a tile does not fit in shared memory).
@@ -720,7 +769,8 @@ void stream_partition(spl_ctx *ctx, spl_mat *a, uint32_t grid) {
     if (a->stream_grid == grid) return;
     SPL_CUDA(cudaStreamSynchronize(ctx->stream));                  // nobody is reading the old arrays
     dfree(ctx, a->stream_cta_rows); dfree(ctx, a->stream_xhi); dfree(ctx, a->stream_xlo0); dfree(ctx, a->stream_tile_lo);
-    a->stream_cta_rows = a->stream_xhi = a->stream_xlo0 = a->stream_tile_lo = nullptr;
+    dfree(ctx, a->stream_tile_reg);
+    a->stream_cta_rows = a->stream_xhi = a->stream_xlo0 = a->stream_tile_lo = a->stream_tile_reg = nullptr;
     a->stream_cta_rows = dalloc<uint32_t>(ctx, (size_t)grid + 1);
     SPL_CUDA(cudaMemsetAsync(ctx->d_scratch + 1, 0, sizeof(uint32_t), ctx->stream));
     stream_partition_kernel<<<div_up((uint64_t)grid + 1, 128), 128, 0, ctx->stream>>>(
@@ -734,61 +784,97 @@ void stream_partition(spl_ctx *ctx, spl_mat *a, uint32_t grid) {
     a->stream_xhi = dalloc<uint32_t>(ctx, slots);
     a->stream_tile_lo = dalloc<uint32_t>(ctx, slots);
     a->stream_xlo0 = dalloc<uint32_t>(ctx, grid);
+    a->stream_tile_reg = dalloc<uint32_t>(ctx, slots);
     SPL_CUDA(cudaMemsetAsync(a->stream_xhi, 0, sizeof(uint32_t) * slots, ctx->stream));
     SPL_CUDA(cudaMemsetAsync(a->stream_xlo0, 0xff, sizeof(uint32_t) * (size_t)grid, ctx->stream));
+    SPL_CUDA(cudaMemsetAsync(a->stream_tile_reg, 0, sizeof(uint32_t) * slots, ctx->stream));
+    SPL_CUDA(cudaMemsetAsync(ctx->d_scratch + 1, 0, sizeof(uint32_t), ctx->stream));
     stream_edges_kernel<<<grid, 256, 0, ctx->stream>>>(a->ptr, a->ind, a->stream_cta_rows, a->stream_rows, max_tiles,
-                                                      a->stream_tile_lo, a->stream_xhi, a->stream_xlo0);
+                                                      a->stream_tile_lo, a->stream_xhi, a->stream_xlo0, row_pattern(a),
+                                                      a->stream_tile_reg, ctx->d_scratch + 1);
     check_launch(ctx, "stream_edges");
-    SPL_CUDA(cudaStreamSynchronize(ctx->stream));                  // visible to any other stream from here on
+    read_back(ctx, ctx->d_scratch + 1, &a->stream_regular, 1);    // synchronises: visible to any other stream from here on
     a->stream_grid = grid;
+}
+
+// Sets the kernel's dynamic shared memory to `smem` and returns how many of its CTAs fit on an SM (cached per
+// instantiation).
+template <typename K>
+uint32_t stream_resident(K k, size_t smem, std::atomic<size_t> &smem_set, std::atomic<uint64_t> &occ_cache) {
+    if (smem > smem_set.load(std::memory_order_relaxed)) {
+        SPL_CUDA(cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+        smem_set.store(smem, std::memory_order_relaxed);
+    }
+    uint64_t oc = occ_cache.load(std::memory_order_relaxed);     // (smem << 8) | resident CTAs
+    if ((oc >> 8) != smem) {
+        int resident = 0;
+        SPL_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&resident, k, ST_CONSUMERS + 32, smem));
+        SPL_REQUIRE(resident >= 1, SPL_ERR_CUDA, "stream SpMV: no CTA fits on an SM");
+        oc = ((uint64_t)smem << 8) | (uint64_t)resident;
+        occ_cache.store(oc, std::memory_order_relaxed);
+    }
+    return (uint32_t)(oc & 0xff);
 }
 
 // x_edge: array indexable by column over [x_lo, x_hi) in local memory (the whole x, or this rank's own
 // slice of a sharded x with the pointer moved back by the slice's first column), or NULL
 template <typename T, int LPR, int U, bool TIGHT, typename XG>
 void launch_stream(spl_ctx *ctx, const spl_mat *a, const XG &xg, T *y, const T *x_edge, uint32_t x_lo, uint32_t x_hi) {
-    auto k = spmv_stream_kernel<T, LPR, U, TIGHT, XG>;
+    auto k_csr = spmv_stream_kernel<T, LPR, U, TIGHT, false, XG>;
+    auto k_pat = spmv_stream_kernel<T, LPR, U, TIGHT, true, XG>;
     constexpr int CONS = ST_CONSUMERS;
     // shape (measured, profiles/r2_spmv_notes.md): three stages, three CTAs of 64 registers per SM; a
     // deeper ring or a fourth, register-starved CTA does not pay
     const size_t stage_bytes = stream_stage_bytes(a);
     const uint32_t stages = (uint32_t)std::max(2, env_int("SPL_STREAM_STAGES", 3));
-    const size_t smem = stages * stage_bytes + 2 * stages * sizeof(uint64_t);
-    SPL_REQUIRE(smem <= 227 * 1024, SPL_ERR_UNSUPPORTED, "stream SpMV: the stages do not fit in shared memory");
-    static std::atomic<size_t> smem_set{0};                       // per instantiation
-    if (smem > smem_set.load(std::memory_order_relaxed)) {
-        SPL_CUDA(cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-        smem_set.store(smem, std::memory_order_relaxed);
-    }
-    static std::atomic<uint64_t> occ_cache{0};                    // (smem << 8) | resident CTAs
-    uint64_t oc = occ_cache.load(std::memory_order_relaxed);
-    if ((oc >> 8) != smem) {
-        int resident = 0;
-        SPL_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&resident, k, CONS + 32, smem));
-        SPL_REQUIRE(resident >= 1, SPL_ERR_CUDA, "stream SpMV: no CTA fits on an SM");
-        oc = ((uint64_t)smem << 8) | (uint64_t)resident;
-        occ_cache.store(oc, std::memory_order_relaxed);
-    }
-    const uint32_t resident = (uint32_t)(oc & 0xff);
+    const size_t smem_csr = stages * stage_bytes + 2 * stages * sizeof(uint64_t);
+    const size_t smem_pat = smem_csr + (stages + kPatternMax) * sizeof(uint32_t);
+    SPL_REQUIRE(smem_csr <= 227 * 1024, SPL_ERR_UNSUPPORTED, "stream SpMV: the stages do not fit in shared memory");
+    static std::atomic<size_t> smem_set_csr{0}, smem_set_pat{0};
+    static std::atomic<uint64_t> occ_csr{0}, occ_pat{0};
+    // the grid is the CSR kernel's: a matrix without regular tiles runs exactly that kernel, and the
+    // partition (with the regular tiles) does not depend on which of the two kernels runs
+    const uint32_t resident = stream_resident(k_csr, smem_csr, smem_set_csr, occ_csr);
     uint32_t ctas = (uint32_t)env_int("SPL_STREAM_CTAS", 0);
     if (ctas == 0 || ctas > resident) ctas = resident;
     const uint32_t grid = (uint32_t)ctx->num_sms * ctas;
     stream_partition(ctx, const_cast<spl_mat *>(a), grid);
+    // regular tiles: the pattern kernel, on the same grid (SPL_STREAM_PATTERN=0 turns it off for A/B measurements).
+    // It may need fewer registers than the CSR kernel (C1: 56 against 63), so one more of its CTAs could fit on
+    // an SM; programmatic dependent launch then places the next product's CTAs there early, which was measured
+    // slower (C1, one L2-resident copy: 12.7 against 11.0 us per product, profiles/r3_spmv_notes.md).  Its shared
+    // memory is padded so that exactly the grid's CTAs per SM fit, as with the CSR kernel.
+    bool pat = a->stream_regular && env_int("SPL_STREAM_PATTERN", 1) != 0;
+    size_t smem_pat_run = smem_pat;
+    if (pat) {
+        static const size_t sm_bytes = [] {
+            int dev = 0, per_sm = 0, reserved = 0;
+            cudaGetDevice(&dev);
+            cudaDeviceGetAttribute(&per_sm, cudaDevAttrMaxSharedMemoryPerMultiprocessor, dev);
+            cudaDeviceGetAttribute(&reserved, cudaDevAttrReservedSharedMemoryPerBlock, dev);
+            return ((size_t)per_sm << 16) | (size_t)reserved;
+        }();
+        const size_t per_sm = sm_bytes >> 16, reserved = sm_bytes & 0xffff;
+        const size_t one_more = per_sm / (ctas + 1) + 1;            // ctas + 1 CTAs of this size do not fit
+        if (one_more > reserved) smem_pat_run = std::max(smem_pat, std::min<size_t>(one_more - reserved, 227 * 1024));
+        pat = smem_pat_run <= 227 * 1024 && stream_resident(k_pat, smem_pat_run, smem_set_pat, occ_pat) >= ctas;
+    }
     cudaLaunchConfig_t cfg{};
     cfg.gridDim = dim3(grid);
     cfg.blockDim = dim3(CONS + 32);
-    cfg.dynamicSmemBytes = smem;
+    cfg.dynamicSmemBytes = pat ? smem_pat_run : smem_csr;
     cfg.stream = ctx->stream;
     cudaLaunchAttribute attr[1];
     attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
     attr[0].val.programmaticStreamSerializationAllowed = 1;
     cfg.attrs = attr;
     cfg.numAttrs = (ctx->pdl_prev && !std::getenv("SPL_NO_PDL")) ? 1 : 0;     // only behind another stream-kernel product
-    SPL_CUDA(cudaLaunchKernelEx(&cfg, k, a->nrows, (const uint32_t *)a->ptr, (const uint32_t *)a->ind,
+    SPL_CUDA(cudaLaunchKernelEx(&cfg, pat ? k_pat : k_csr, a->nrows, (const uint32_t *)a->ptr, (const uint32_t *)a->ind,
                                 static_cast<const T *>(a->val), xg, y, (const uint32_t *)a->stream_cta_rows,
                                 (const uint32_t *)a->stream_tile_lo, (const uint32_t *)a->stream_xhi,
                                 (const uint32_t *)a->stream_xlo0, a->stream_max_tiles, a->stream_cap, stages,
-                                x_edge, x_lo, x_hi, env_int("SPL_STREAM_L2HINT", 1)));
+                                x_edge, x_lo, x_hi, env_int("SPL_STREAM_L2HINT", 1),
+                                (const uint32_t *)a->stream_tile_reg, row_pattern(a)));
     check_launch(ctx, "spmv_stream");
     ctx->pdl_chain = true;
 }
@@ -1250,6 +1336,38 @@ __global__ void max_row_len_kernel(const uint32_t *__restrict__ ptr, const uint3
     }
 }
 
+// *row = the first row in [from, nrows) with `len` entries (stays ~0 if there is none)
+__global__ void pattern_row_kernel(const uint32_t *__restrict__ ptr, uint32_t from, uint32_t nrows, uint32_t len,
+                                   uint32_t *row) {
+    for (uint64_t r = from + (uint64_t)blockIdx.x * blockDim.x + threadIdx.x; r < nrows;
+         r += (uint64_t)gridDim.x * blockDim.x) {
+        if (ptr[r + 1] - ptr[r] == len) {        // a thread's first hit is its smallest: the minimum over threads is the first
+            atomicMin(row, (uint32_t)r);
+            return;
+        }
+    }
+}
+
+// The row pattern (spl_mat::pattern_off): the column offsets of the first row at or after nrows / 2 with the
+// longest length, taken from the middle because the first rows of bands and stencils are boundary rows.
+void plan_pattern(spl_ctx *ctx, spl_mat *a) {
+    a->pattern_len = 0;
+    const uint32_t len = a->max_row_len;
+    if (len == 0 || len > kPatternMax) return;
+    SPL_CUDA(cudaMemsetAsync(ctx->d_scratch, 0xff, sizeof(uint32_t), ctx->stream));
+    const uint32_t from = a->nrows / 2;
+    pattern_row_kernel<<<std::min<unsigned>(div_up(a->nrows - from, 256), (unsigned)ctx->num_sms * 8u), 256, 0, ctx->stream>>>(
+        a->ptr, from, a->nrows, len, ctx->d_scratch);
+    check_launch(ctx, "pattern_row");
+    uint32_t row = 0, p = 0;
+    read_back(ctx, ctx->d_scratch, &row, 1);
+    if (row == ~0u) return;
+    read_back(ctx, a->ptr + row, &p, 1);
+    read_back(ctx, a->ind + p, a->pattern_off, (int)len);
+    for (uint32_t j = 0; j < len; ++j) a->pattern_off[j] -= row;
+    a->pattern_len = len;
+}
+
 }  // namespace
 
 void spmv_plan(spl_ctx *ctx, spl_mat *a) {
@@ -1278,8 +1396,10 @@ void spmv_plan(spl_ctx *ctx, spl_mat *a) {
     if (mean > 12.0) lanes = 4;
     while (lanes < 32 && lanes * 10 < mean) lanes *= 2;
     a->plan_lanes = lanes;
-    // stream kernel: the largest window of 256 / lanes rows sizes its shared-memory stages
+    // stream kernel: the largest window of 256 / lanes rows sizes its shared-memory stages; tiles that follow
+    // the row pattern stream their values only
     stream_capacity(ctx, a, (uint32_t)stream_consumers() / (uint32_t)lanes);
+    plan_pattern(ctx, a);
     // merge-path tile starts (matrix-only data, cached)
     const int ipt = a->dtype == SPL_F64 ? merge_ipt<double>() : merge_ipt<float>();
     const uint32_t items = MG_THREADS * ipt;
