@@ -20,7 +20,9 @@
 //   * the COMPUTE warps own a fixed range of rows per CTA, keep the row sums in shared memory, and
 //     walk the blocks in order: block 0 needs only the rank's own slice and runs while the first
 //     slices are in flight; before block b they wait (acquire) for the counters of its slices.
-//     Transfer and math overlap block by block, and y is written once.
+//     Transfer and math overlap block by block, and y is written once.  A tile producer warp feeds
+//     them the tiles of the stream kernel (stream_tile.cuh: same tile, same row loop, same bits per
+//     block); the copies and the folded flag barrier use the primitives of ptx.cuh.
 // All CTAs are resident at once (cooperative launch: the grid is what fits), so the waits cannot
 // deadlock.  Row sums add the blocks in ring order, not in ascending column order: tolerance parity
 // (1e-12 / 1e-5), like every multi-lane kernel.
@@ -28,6 +30,8 @@
 #include <cstdlib>
 
 #include "kernels.cuh"
+#include "ptx.cuh"
+#include "stream_tile.cuh"
 
 namespace spl {
 
@@ -49,14 +53,7 @@ struct GatherBarrier {
     uint32_t *failed;
 };
 
-__device__ __forceinline__ unsigned long long global_timer_ns() {
-    unsigned long long t;
-    asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(t));
-    return t;
-}
-
-constexpr int GF_THREADS = 256;  // consumer threads of a CTA; one warp more feeds them tiles, another copies x
-constexpr int GF_CTA = GF_THREADS + 64;
+constexpr int GF_CTA = TILE_CONSUMERS + 64;      // the consumers, one warp that feeds them tiles, one that copies x
 constexpr uint32_t GF_CHUNK = 4096;      // bytes per bulk copy of x: 5 x 4 KB in flight per CTA, ~9 MB on the chip — beside the
                                          // product's gathers an NVLink read takes ~15 us, and 4 MB in flight gave 240 GB/s
 constexpr int GF_STAGES = 6;             // x ring slots per CTA
@@ -69,41 +66,6 @@ struct GatherBlocks {
     int n;
 };
 
-__device__ __forceinline__ uint32_t ld_acquire_gpu(const uint32_t *p) {
-    uint32_t v;
-    asm volatile("ld.acquire.gpu.global.u32 %0, [%1];" : "=r"(v) : "l"(p) : "memory");
-    return v;
-}
-__device__ __forceinline__ uint32_t gf_smem(const void *p) { return (uint32_t)__cvta_generic_to_shared(p); }
-__device__ __forceinline__ void gf_mbar_init(uint64_t *bar, uint32_t count) {
-    asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(gf_smem(bar)), "r"(count));
-}
-__device__ __forceinline__ void gf_mbar_wait(uint64_t *bar, uint32_t parity) {
-    asm volatile(
-        "{\n.reg .pred q;\nGFW_%=:\nmbarrier.try_wait.parity.shared::cta.b64 q, [%0], %1;\n@q bra GFD_%=;\nbra GFW_%=;\nGFD_%=:\n}\n" ::"r"(
-            gf_smem(bar)),
-        "r"(parity)
-        : "memory");
-}
-__device__ __forceinline__ void gf_mbar_arrive(uint64_t *bar) {
-    asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(gf_smem(bar)) : "memory");
-}
-__device__ __forceinline__ void gf_expect_tx(uint64_t *bar, uint32_t bytes) {
-    asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(gf_smem(bar)), "r"(bytes) : "memory");
-}
-__device__ __forceinline__ void gf_g2s(void *dst_smem, const void *src, uint32_t bytes, uint64_t *bar) {
-    asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];" ::"r"(gf_smem(dst_smem)),
-                 "l"(src), "r"(bytes), "r"(gf_smem(bar))
-                 : "memory");
-}
-__device__ __forceinline__ void gf_g2s_stream(void *dst_smem, const void *src, uint32_t bytes, uint64_t *bar, uint64_t policy) {
-    asm volatile(
-        "cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes.L2::cache_hint [%0], [%1], %2, [%3], %4;" ::"r"(
-            gf_smem(dst_smem)),
-        "l"(src), "r"(bytes), "r"(gf_smem(bar)), "l"(policy)
-        : "memory");
-}
-
 // ---- the copy warp of one CTA ----
 template <typename T>
 __device__ void gather_copy_warp(const GatherPeers &gp, T *x_full, uint32_t *ready, const GatherBarrier &gb,
@@ -112,25 +74,14 @@ __device__ void gather_copy_warp(const GatherPeers &gp, T *x_full, uint32_t *rea
     const unsigned lane = threadIdx.x & 31u;
     const unsigned long long cta = blockIdx.x, ncta = gridDim.x;
     if (gb.flags_mine) {
-        if (cta == 0 && (int)lane < G && (int)lane != gp.rank) {
-            // fused barrier, arrival: this rank's published slice is final (stream order put its writers before us)
-            __threadfence_system();
-            asm volatile("st.release.sys.global.u32 [%0], %1;" ::"l"(gb.flags[lane] + gp.rank), "r"(gb.epoch) : "memory");
-        }
+        // fused barrier, arrival: this rank's published slice is final (stream order put its writers before us)
+        if (cta == 0 && (int)lane < G && (int)lane != gp.rank) flag_arrive(gb.flags[lane], gp.rank, gb.epoch);
         __syncwarp();
     }
     // fused barrier, wait: rank g's slice is final once its epoch shows up in this rank's flag block; waited for
     // slice by slice, so a late peer delays only its own slice
     auto wait_owner = [&](int g) {
-        if (!gb.flags_mine) return;
-        const unsigned long long t0 = global_timer_ns();
-        for (;;) {
-            uint32_t v;
-            asm volatile("ld.acquire.sys.global.u32 %0, [%1];" : "=r"(v) : "l"(gb.flags_mine + g) : "memory");
-            if ((int32_t)(v - gb.epoch) >= 0) break;
-            if (global_timer_ns() - t0 > gb.timeout_ns) { atomicExch(gb.failed, 1u); break; }
-            __nanosleep(100);
-        }
+        if (gb.flags_mine) flag_wait(gb.flags_mine + g, gb.epoch, gb.timeout_ns, 100, gb.failed);
     };
     // chunks of the bulk path per slice (ring offset k = 1..G-1): whole 16-byte units of slices whose two ends are
     // 16-byte aligned (IPC blocks are; slice starts of an f32 vector need not be); the rest goes element by element
@@ -158,9 +109,8 @@ __device__ void gather_copy_warp(const GatherPeers &gp, T *x_full, uint32_t *rea
     }
     __syncwarp();
     if (lane == 0) {
-        for (int s = 0; s < GF_STAGES; ++s)
-            asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(gf_smem(full + s)), "r"(1u));
-        asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+        for (int s = 0; s < GF_STAGES; ++s) mbar_init(full + s, 1);
+        mbar_init_fence();
         const unsigned long long total = cum[G - 1];
         const unsigned long long mine = total > cta ? (total - cta + ncta - 1) / ncta : 0;
         int kl = 1, ks = 1, ksig = 1, kw = 0;
@@ -185,11 +135,8 @@ __device__ void gather_copy_warp(const GatherPeers &gp, T *x_full, uint32_t *rea
                 const unsigned long long off = (c - cum[kl - 1]) * GF_CHUNK;
                 const uint32_t len = (uint32_t)(b16 - off < GF_CHUNK ? b16 - off : GF_CHUNK);
                 const int s = (int)(i % GF_STAGES);
-                asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(gf_smem(full + s)), "r"(len) : "memory");
-                asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];" ::"r"(
-                                 gf_smem(ring + (size_t)s * GF_CHUNK)),
-                             "l"(src + off), "r"(len), "r"(gf_smem(full + s))
-                             : "memory");
+                mbar_expect_tx(full + s, len);
+                tma_bulk_g2s(ring + (size_t)s * GF_CHUNK, src + off, len, full + s);
             }
             if (i >= (unsigned long long)GF_AHEAD) {
                 const unsigned long long j = i - GF_AHEAD, c = cta + j * ncta;
@@ -200,28 +147,22 @@ __device__ void gather_copy_warp(const GatherPeers &gp, T *x_full, uint32_t *rea
                 const uint32_t len = (uint32_t)(b16 - off < GF_CHUNK ? b16 - off : GF_CHUNK);
                 const int s = (int)(j % GF_STAGES);
                 const uint32_t parity = (uint32_t)((j / GF_STAGES) & 1);
-                asm volatile(
-                    "{\n.reg .pred q;\nGFW_%=:\nmbarrier.try_wait.parity.shared::cta.b64 q, [%0], %1;\n@q bra GFD_%=;\nbra GFW_%=;\nGFD_%=:\n}\n" ::"r"(
-                        gf_smem(full + s)),
-                    "r"(parity)
-                    : "memory");
-                asm volatile("cp.async.bulk.global.shared::cta.bulk_group [%0], [%1], %2;" ::"l"(dst + off),
-                             "r"(gf_smem(ring + (size_t)s * GF_CHUNK)), "r"(len)
-                             : "memory");
-                asm volatile("cp.async.bulk.commit_group;" ::: "memory");
+                mbar_wait(full + s, parity);
+                tma_bulk_s2g(dst + off, ring + (size_t)s * GF_CHUNK, len);
+                bulk_commit();
                 if (c + ncta >= cum[ks]) {
                     // this CTA's last chunk of the slice: wait until its stores are WRITTEN (the loads ahead keep flying —
                     // bulk groups count stores only), then say so.  Slices that lie wholly below the next chunk hold
                     // nothing of this CTA that is still in flight
-                    asm volatile("cp.async.bulk.wait_group 0;" ::: "memory");
+                    bulk_wait_all();
                     __threadfence();
                     for (; ksig < G && cum[ksig] <= c + ncta; ++ksig) atomicAdd(ready + ksig, 1u);
                 } else {
-                    asm volatile("cp.async.bulk.wait_group.read 1;" ::: "memory");   // every store but the newest has left its slot
+                    bulk_wait_read_but_one();            // every store but the newest has left its slot
                 }
             }
         }
-        asm volatile("cp.async.bulk.wait_group 0;" ::: "memory");
+        bulk_wait_all();
         __threadfence();
         for (; ksig < G; ++ksig) atomicAdd(ready + ksig, 1u);
     }
@@ -242,8 +183,7 @@ spmv_gather_fused_kernel(uint32_t nloc, const uint32_t *__restrict__ bptr, uint3
                          const uint32_t *__restrict__ bind, const T *__restrict__ bval, GatherPeers gp, GatherBlocks gk,
                          T *x_full, T *__restrict__ y, uint32_t *ready, uint32_t target, GatherShape sh, GatherBarrier gb,
                          unsigned long long *timeline) {
-    constexpr uint32_t R = GF_THREADS / LPR;      // rows per tile: LPR lanes per row, U gathers per lane and pass
-    constexpr uint32_t PTRS = R + 4;              // pointer slots per stage: R + 1 needed, whole 16-byte units
+    constexpr uint32_t R = tile_rows(LPR), PTRS = tile_ptr_slots(R);
     extern __shared__ __align__(128) unsigned char gf_raw[];
     uint32_t *s_ind = reinterpret_cast<uint32_t *>(gf_raw);
     T *s_val = reinterpret_cast<T *>(gf_raw + sh.off_val);
@@ -259,12 +199,12 @@ spmv_gather_fused_kernel(uint32_t nloc, const uint32_t *__restrict__ bptr, uint3
     const uint32_t ntiles = (re - rs + R - 1) / R;          // 0 for a CTA without rows (it still copies x)
     const uint32_t nb = (uint32_t)gk.n;
 
-    if (threadIdx.x >= GF_THREADS + 32) {
+    if (threadIdx.x >= TILE_CONSUMERS + 32) {
         // ---- warp 9: this CTA's share of the peers' slices of x ----
         if (gp.world > 1) gather_copy_warp<T>(gp, x_full, ready, gb, gf_raw + sh.off_ring, xfull, timeline);
         return;
     }
-    if (threadIdx.x >= GF_THREADS) {
+    if (threadIdx.x >= TILE_CONSUMERS) {
         // ---- warp 8: feeds the consumers.  All lanes fetch the tile bounds of every block (one round trip), then one
         // thread issues the bulk copies of each tile's row pointers, indices and values, `stages` tiles ahead; the
         // matrix does not depend on x, so the tiles of block b are in shared memory before its slices have landed ----
@@ -277,23 +217,22 @@ spmv_gather_fused_kernel(uint32_t nloc, const uint32_t *__restrict__ bptr, uint3
         }
         if (lane == 0) {
             for (uint32_t s = 0; s < sh.stages; ++s) {
-                gf_mbar_init(full + s, 1);
-                gf_mbar_init(empty + s, GF_THREADS / 32);
+                mbar_init(full + s, 1);
+                mbar_init(empty + s, TILE_CONSUMERS / 32);
             }
-            asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+            mbar_init_fence();
         }
         __syncwarp();
-        asm volatile("bar.arrive 2, %0;" ::"n"(GF_THREADS + 32) : "memory");      // barriers are live: consumers may wait on them
+        asm volatile("bar.arrive 2, %0;" ::"n"(TILE_CONSUMERS + 32) : "memory");      // barriers are live: consumers may wait on them
         if (lane != 0) return;
-        uint64_t pol;
-        asm volatile("createpolicy.fractional.L2::evict_first.b64 %0, 1.0;" : "=l"(pol));
+        const uint64_t pol = l2_policy_evict_first();
         uint32_t s = 0, phase = 0, i = 0;
         for (uint32_t k = 0; k < nb; ++k)
             for (uint32_t t = 0; t < ntiles; ++t, ++i) {
                 const uint32_t lo = s_tlo[k * (ntiles + 1) + t], hi = s_tlo[k * (ntiles + 1) + t + 1];
-                if (i >= sh.stages) gf_mbar_wait(empty + s, phase ^ 1u);
-                const uint32_t za = lo & ~3u, zb = (hi + 3u) & ~3u;           // 16-byte aligned superset; the arrays carry slack
-                uint32_t cnt = zb - za;
+                if (i >= sh.stages) mbar_wait(empty + s, phase ^ 1u);
+                const uint32_t za = slice_lo(lo);
+                uint32_t cnt = slice_hi(hi) - za;
                 if (cnt > sh.cap) {                        // tile_entries_max was too small: never overrun the stage — the
                     atomicExch(gb.failed, 1u);             // tile is cut (the consumers clamp too) and y comes back as NaN
                     cnt = sh.cap;
@@ -301,25 +240,25 @@ spmv_gather_fused_kernel(uint32_t nloc, const uint32_t *__restrict__ bptr, uint3
                 const uint32_t r0 = rs + t * R;
                 const uint32_t left = (pstride - r0) & ~3u;                   // pointer entries from r0 to the end of the block's array
                 const uint32_t np = left < PTRS ? left : PTRS;
-                gf_expect_tx(full + s, cnt * (uint32_t)(sizeof(uint32_t) + sizeof(T)) + np * (uint32_t)sizeof(uint32_t));
-                gf_g2s(s_ptr + (size_t)s * PTRS, bptr + (size_t)k * pstride + r0, np * (uint32_t)sizeof(uint32_t), full + s);
+                mbar_expect_tx(full + s, cnt * (uint32_t)(sizeof(uint32_t) + sizeof(T)) + np * (uint32_t)sizeof(uint32_t));
+                tma_bulk_g2s(s_ptr + (size_t)s * PTRS, bptr + (size_t)k * pstride + r0, np * (uint32_t)sizeof(uint32_t), full + s);
                 if (cnt) {
-                    gf_g2s_stream(s_ind + (size_t)s * sh.cap, bind + za, cnt * (uint32_t)sizeof(uint32_t), full + s, pol);
-                    gf_g2s_stream(s_val + (size_t)s * sh.cap, bval + za, cnt * (uint32_t)sizeof(T), full + s, pol);
+                    tma_bulk_g2s_hint(s_ind + (size_t)s * sh.cap, bind + za, cnt * (uint32_t)sizeof(uint32_t), full + s, pol);
+                    tma_bulk_g2s_hint(s_val + (size_t)s * sh.cap, bval + za, cnt * (uint32_t)sizeof(T), full + s, pol);
                 }
                 if (++s == sh.stages) { s = 0; phase ^= 1u; }
             }
         return;
     }
 
-    // ---- consumers: LPR lanes per row, exactly as in the unsharded stream kernel (spmv.cu) — pointers, indices and
-    // values come from shared memory, only x from global memory, and the warps run on their own (no CTA barrier).
+    // ---- consumers: LPR lanes per row (tile_row_sum) — pointers, indices and values come from shared memory, only x
+    // from global memory, and the warps run on their own (no CTA barrier).
     // A row's running sum lives in y itself: the same lanes own the row in every block, and shared memory spent on
     // sums would come out of the L1 that holds the gathers in flight.  Measured alternatives (entries dealt to the
     // lanes with eight gathers each, four rows per lane, products summed in a second pass) kept more gathers in flight
     // and were all slower: profiles/r2_spmv_notes.md ----
     if (ntiles == 0) return;
-    asm volatile("bar.sync 2, %0;" ::"n"(GF_THREADS + 32) : "memory");
+    asm volatile("bar.sync 2, %0;" ::"n"(TILE_CONSUMERS + 32) : "memory");
     const T *own = static_cast<const T *>(gp.slice[gp.rank]) - gp.start[gp.rank];
     const uint32_t lane = threadIdx.x & 31u, rl = threadIdx.x / LPR, sub = threadIdx.x % LPR;
     const bool stamp = timeline && c == 0 && threadIdx.x == 0;
@@ -334,39 +273,24 @@ spmv_gather_fused_kernel(uint32_t nloc, const uint32_t *__restrict__ bptr, uint3
         }
         if (stamp) timeline[2 + 3 * k] = global_timer_ns();                                           // its slices have landed
         for (uint32_t t = 0; t < ntiles; ++t) {
-            gf_mbar_wait(full + s, phase);
+            mbar_wait(full + s, phase);
             const uint32_t *cp = s_ptr + (size_t)s * PTRS;
             const uint32_t *ci = s_ind + (size_t)s * sh.cap;
             const T *cv = s_val + (size_t)s * sh.cap;
             const uint32_t r = rs + t * R + rl;
-            const uint32_t za = cp[0] & ~3u;
+            const uint32_t za = slice_lo(cp[0]);
             uint32_t p0 = 0, e = 0;
             if (r < re) { p0 = min(cp[rl] - za, sh.cap); e = min(cp[rl + 1] - za, sh.cap); }      // never past the stage
             T prev = (T)0;
             if (k > 0 && sub == 0 && r < re) prev = y[r];              // in flight with the gathers
             T acc = (T)0;
-            auto row_sum = [&](auto gather) {
-                for (uint32_t j = p0 + sub; j < e; j += U * LPR) {
-                    uint32_t col[U];
-                    T xv[U], v[U];
-#pragma unroll
-                    for (int u = 0; u < U; ++u) col[u] = j + u * LPR < e ? ci[j + u * LPR] : 0xffffffffu;
-#pragma unroll
-                    for (int u = 0; u < U; ++u) xv[u] = col[u] != 0xffffffffu ? gather(col[u]) : (T)0;
-#pragma unroll
-                    for (int u = 0; u < U; ++u) v[u] = j + u * LPR < e ? cv[j + u * LPR] : (T)0;
-#pragma unroll
-                    for (int u = 0; u < U; ++u) acc += j + u * LPR < e ? v[u] * xv[u] : (T)0;          // 0, never 0 * inf
-                }
-            };
             // block 0 reads the published slice (constant for the whole kernel); x_full is written by this very kernel,
             // behind the acquire that let this block start: L2 loads
-            if (k == 0) row_sum([&](uint32_t col) { return __ldg(own + col); });
-            else row_sum([&](uint32_t col) { return __ldcg(x_full + col); });
+            if (k == 0) tile_row_sum<T, LPR, U>(acc, ci, 0, cv, p0, e, sub, [&](uint32_t col) { return __ldg(own + col); });
+            else tile_row_sum<T, LPR, U>(acc, ci, 0, cv, p0, e, sub, [&](uint32_t col) { return __ldcg(x_full + col); });
             __syncwarp();
-            if (lane == 0) gf_mbar_arrive(empty + s);
-#pragma unroll
-            for (int o = LPR / 2; o > 0; o >>= 1) acc += __shfl_xor_sync(0xffffffffu, acc, o);
+            if (lane == 0) mbar_arrive(empty + s);
+            acc = row_lanes_sum<LPR>(acc);
             if (sub == 0 && r < re) y[r] = prev + acc;
             if (++s == sh.stages) { s = 0; phase ^= 1u; }
         }
@@ -394,9 +318,9 @@ bool spmv_gather_fused_t(size_t smem_per_sm, spl_ctx *ctx, uint32_t nloc, const 
                          const T *bval, const uint32_t *tile_caps, const GatherPeers &gp, const GatherBlocks &gk, T *x_full,
                          T *y, uint32_t *ready, uint32_t epoch, const GatherBarrier &gb, unsigned long long *timeline) {
     auto k = spmv_gather_fused_kernel<T, LPR, U>;
-    constexpr uint32_t R = GF_THREADS / LPR;
+    constexpr uint32_t R = tile_rows(LPR);
     static_assert(R == 64 || R == 128 || R == 256, "tile rows");
-    const uint32_t cap = (tile_caps[R == 64 ? 0 : R == 128 ? 1 : 2] + 6u + 3u) & ~3u;
+    const uint32_t cap = stage_capacity(tile_caps[R == 64 ? 0 : R == 128 ? 1 : 2]);
     const char *pc = std::getenv("SPL_GATHER_CTAS_PER_SM");          // measurement knobs
     const char *ps = std::getenv("SPL_GATHER_STAGES");
     const int most = pc ? std::max(1, std::atoi(pc)) : 3;
@@ -413,7 +337,7 @@ bool spmv_gather_fused_t(size_t smem_per_sm, spl_ctx *ctx, uint32_t nloc, const 
         sh.off_val = (uint32_t)o;
         o += (size_t)stages * cap * sizeof(T);
         sh.off_ptr = (uint32_t)o;
-        o += (size_t)stages * (R + 4) * sizeof(uint32_t);
+        o += (size_t)stages * tile_ptr_slots(R) * sizeof(uint32_t);
         o = (o + 127) & ~(size_t)127;
         sh.off_ring = (uint32_t)o;
         o += GF_RING;

@@ -5,13 +5,14 @@
 // mapping is a full-bandwidth NVLink path.  spl_spmv_peer then gathers x straight from the
 // owning slice, so the "exchange" of the sharded SpMV is part of the kernel's loads.  The only
 // thing left between iterations is ordering: a rank's writes to its slice must be visible before
-// a peer's next kernel reads them.  peer_barrier_kernel does that on the device: release-store of
-// the epoch into every peer's flag block, acquire-spin on the own block, bounded by a timeout so
-// a missing peer can never hang the GPU.
+// a peer's next kernel reads them.  peer_barrier_kernel does that on the device with the flag
+// barrier of ptx.cuh: release-store of the epoch into every peer's flag block, acquire-spin on the
+// own block, bounded by a timeout so a missing peer can never hang the GPU.
 #include <algorithm>
 #include <cstdlib>
 
 #include "kernels.cuh"
+#include "ptx.cuh"
 
 namespace spl {
 
@@ -21,30 +22,12 @@ struct FlagBlocks {
     uint32_t *block[SPL_MAX_PEERS];
 };
 
-__device__ __forceinline__ uint64_t global_timer_ns() {
-    uint64_t t;
-    asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(t));
-    return t;
-}
-
 __global__ void peer_barrier_kernel(FlagBlocks f, int world, int rank, uint32_t epoch,
                                     uint64_t timeout_ns, uint32_t *timed_out) {
     const int g = threadIdx.x;
     if (g >= world || g == rank) return;
-    __threadfence_system();                      // earlier kernels' writes to this rank's slice
-    asm volatile("st.release.sys.global.u32 [%0], %1;" ::"l"(f.block[g] + rank), "r"(epoch) : "memory");
-    const uint64_t t0 = global_timer_ns();
-    const uint32_t *mine = f.block[rank] + g;
-    for (;;) {
-        uint32_t v;
-        asm volatile("ld.acquire.sys.global.u32 %0, [%1];" : "=r"(v) : "l"(mine) : "memory");
-        if ((int32_t)(v - epoch) >= 0) break;
-        if (global_timer_ns() - t0 > timeout_ns) {
-            atomicExch(timed_out, 1u);
-            break;
-        }
-        __nanosleep(200);
-    }
+    flag_arrive(f.block[g], rank, epoch);        // earlier kernels' writes to this rank's slice are visible
+    flag_wait(f.block[rank] + g, epoch, timeout_ns, 200, timed_out);
 }
 
 // Barrier + halo in one launch.  Threads 0..world-1 run the flag protocol above; once every peer has
@@ -67,21 +50,8 @@ peer_barrier_halo_kernel(FlagBlocks f, int world, int rank, uint32_t epoch, uint
     __syncthreads();
     const int g = threadIdx.x;
     if (g < world && g != rank) {
-        __threadfence_system();
-        asm volatile("st.release.sys.global.u32 [%0], %1;" ::"l"(f.block[g] + rank), "r"(epoch) : "memory");
-        const uint64_t t0 = global_timer_ns();
-        const uint32_t *mine = f.block[rank] + g;
-        for (;;) {
-            uint32_t v;
-            asm volatile("ld.acquire.sys.global.u32 %0, [%1];" : "=r"(v) : "l"(mine) : "memory");
-            if ((int32_t)(v - epoch) >= 0) break;
-            if (global_timer_ns() - t0 > timeout_ns) {
-                atomicExch(timed_out, 1u);
-                s_failed = 1;
-                break;
-            }
-            __nanosleep(200);
-        }
+        flag_arrive(f.block[g], rank, epoch);
+        if (!flag_wait(f.block[rank] + g, epoch, timeout_ns, 200, timed_out)) s_failed = 1;
     }
     __syncthreads();
     if (s_failed) return;                        // the product behind this writes NaN (XPeer / status call)
@@ -118,8 +88,6 @@ struct PullSlices {
 constexpr uint32_t PULL_CHUNK = 16384;
 constexpr int PULL_STAGES = 6, PULL_AHEAD = 4;     // loads run 4 chunks in front of the stores (STAGES >= AHEAD + 2)
 constexpr int PULL_THREADS = 128;
-
-__device__ __forceinline__ uint32_t peer_smem(const void *p) { return (uint32_t)__cvta_generic_to_shared(p); }
 
 __global__ void __launch_bounds__(PULL_THREADS) peer_pull_kernel(PullSlices ps, unsigned char *__restrict__ dst) {
     extern __shared__ __align__(128) unsigned char pull_ring[];
@@ -161,9 +129,8 @@ __global__ void __launch_bounds__(PULL_THREADS) peer_pull_kernel(PullSlices ps, 
         ++np;
     }
     if (threadIdx.x != 0 || np == 0) return;
-    for (int s = 0; s < PULL_STAGES; ++s)
-        asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(peer_smem(full + s)), "r"(1u));
-    asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+    for (int s = 0; s < PULL_STAGES; ++s) mbar_init(full + s, 1);
+    mbar_init_fence();
     // chunk id c = j * np + k: chunk j of peer k, so all peers (all links) move at once; ids past a short slice are skipped
     const unsigned long long total = most * np;
     auto locate = [&](unsigned long long c, int &k, unsigned long long &off, uint32_t &len) {
@@ -181,11 +148,8 @@ __global__ void __launch_bounds__(PULL_THREADS) peer_pull_kernel(PullSlices ps, 
         const bool more = cl < total;
         if (more) {
             const int s = (int)(issued % PULL_STAGES);
-            asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(peer_smem(full + s)), "r"(len) : "memory");
-            asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];" ::"r"(
-                             peer_smem(pull_ring + (size_t)s * PULL_CHUNK)),
-                         "l"(src[k] + off), "r"(len), "r"(peer_smem(full + s))
-                         : "memory");
+            mbar_expect_tx(full + s, len);
+            tma_bulk_g2s(pull_ring + (size_t)s * PULL_CHUNK, src[k] + off, len, full + s);
             ++issued;
             cl += gridDim.x;
         }
@@ -194,23 +158,17 @@ __global__ void __launch_bounds__(PULL_THREADS) peer_pull_kernel(PullSlices ps, 
             for (;; cs += gridDim.x) { locate(cs, k2, off2, len2); if (len2) break; }
             const int s = (int)(stored % PULL_STAGES);
             const uint32_t parity = (uint32_t)((stored / PULL_STAGES) & 1);
-            asm volatile(
-                "{\n.reg .pred q;\nPLW_%=:\nmbarrier.try_wait.parity.shared::cta.b64 q, [%0], %1;\n@q bra PLD_%=;\nbra PLW_%=;\nPLD_%=:\n}\n" ::"r"(
-                    peer_smem(full + s)),
-                "r"(parity)
-                : "memory");
-            asm volatile("cp.async.bulk.global.shared::cta.bulk_group [%0], [%1], %2;" ::"l"(out[k2] + off2),
-                         "r"(peer_smem(pull_ring + (size_t)s * PULL_CHUNK)), "r"(len2)
-                         : "memory");
-            asm volatile("cp.async.bulk.commit_group;" ::: "memory");
-            asm volatile("cp.async.bulk.wait_group.read 1;" ::: "memory");   // every store but the newest has left its slot
+            mbar_wait(full + s, parity);
+            tma_bulk_s2g(out[k2] + off2, pull_ring + (size_t)s * PULL_CHUNK, len2);
+            bulk_commit();
+            bulk_wait_read_but_one();                   // every store but the newest has left its slot
             ++stored;
             cs += gridDim.x;
         } else if (!more) {
             break;
         }
     }
-    asm volatile("cp.async.bulk.wait_group 0;" ::: "memory");
+    bulk_wait_all();
 }
 
 }  // namespace

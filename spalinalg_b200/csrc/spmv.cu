@@ -27,8 +27,10 @@
 #include <cstring>
 
 #include "kernels.cuh"
+#include "ptx.cuh"
 #include "radix_sort.cuh"
 #include "scan.cuh"
+#include "stream_tile.cuh"
 
 namespace spl {
 
@@ -107,29 +109,28 @@ spmv_vector_kernel(uint32_t nrows, const uint32_t *__restrict__ ptr,
             for (int u = 0; u < U; ++u) acc += p + u * LPR < e ? v[u] * xv[u] : (T)0;   // 0, never 0 * inf
         }
     }
-#pragma unroll
-    for (int o = LPR / 2; o > 0; o >>= 1) acc += __shfl_xor_sync(0xffffffffu, acc, o);
+    acc = row_lanes_sum<LPR>(acc);
     if (sub == 0 && row < nrows) y[row] = xg.poisoned() ? (T)NAN : acc;
 }
 
+// rows [r0, r1) of A: y[r0, r1)
 template <typename T, int LPR, typename XG>
-void launch_vector(spl_ctx *ctx, const spl_mat *a, const XG &xg, T *y) {
-    const uint64_t threads = (uint64_t)a->nrows * LPR;
-    const unsigned grid = div_up(threads, 256);
-    spmv_vector_kernel<T, LPR, XG><<<grid, 256, 0, ctx->stream>>>(a->nrows, a->ptr, a->ind,
-                                                                  static_cast<const T *>(a->val), xg, y);
+void launch_vector(spl_ctx *ctx, const spl_mat *a, const XG &xg, T *y, uint32_t r0, uint32_t r1) {
+    const uint64_t threads = (uint64_t)(r1 - r0) * LPR;
+    spmv_vector_kernel<T, LPR, XG><<<div_up(threads, 256), 256, 0, ctx->stream>>>(
+        r1 - r0, a->ptr + r0, a->ind, static_cast<const T *>(a->val), xg, y + r0);
     check_launch(ctx, "spmv_vector");
 }
 
 template <typename T, typename XG>
-void spmv_vector(spl_ctx *ctx, const spl_mat *a, const XG &xg, T *y, int lanes) {
+void spmv_vector(spl_ctx *ctx, const spl_mat *a, const XG &xg, T *y, int lanes, uint32_t r0, uint32_t r1) {
     switch (lanes) {
-        case 1: launch_vector<T, 1>(ctx, a, xg, y); break;
-        case 2: launch_vector<T, 2>(ctx, a, xg, y); break;
-        case 4: launch_vector<T, 4>(ctx, a, xg, y); break;
-        case 8: launch_vector<T, 8>(ctx, a, xg, y); break;
-        case 16: launch_vector<T, 16>(ctx, a, xg, y); break;
-        case 32: launch_vector<T, 32>(ctx, a, xg, y); break;
+        case 1: launch_vector<T, 1>(ctx, a, xg, y, r0, r1); break;
+        case 2: launch_vector<T, 2>(ctx, a, xg, y, r0, r1); break;
+        case 4: launch_vector<T, 4>(ctx, a, xg, y, r0, r1); break;
+        case 8: launch_vector<T, 8>(ctx, a, xg, y, r0, r1); break;
+        case 16: launch_vector<T, 16>(ctx, a, xg, y, r0, r1); break;
+        case 32: launch_vector<T, 32>(ctx, a, xg, y, r0, r1); break;
         default: throw Error{SPL_ERR_ARG, "lanes per row must be 1, 2, 4, 8, 16 or 32"};
     }
 }
@@ -277,42 +278,6 @@ __global__ void merge_partition_kernel(const uint32_t *__restrict__ ptr, uint32_
     tile_rows[t] = (uint32_t)lo;
 }
 
-
-// ---- TMA (cp.async.bulk) + mbarrier: the contiguous col/val slice of a tile goes global ->
-// shared memory as two bulk copies issued by one thread; no registers, no per-lane loads.
-__device__ __forceinline__ uint32_t smem_u32(const void *p) {
-    return (uint32_t)__cvta_generic_to_shared(p);
-}
-__device__ __forceinline__ void mbar_init(uint64_t *bar, uint32_t count) {
-    asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(smem_u32(bar)), "r"(count));
-    asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-}
-__device__ __forceinline__ void mbar_expect_tx(uint64_t *bar, uint32_t bytes) {
-    asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(smem_u32(bar)), "r"(bytes)
-                 : "memory");
-}
-__device__ __forceinline__ void tma_bulk_g2s(void *dst_smem, const void *src_gmem, uint32_t bytes,
-                                             uint64_t *bar) {
-    asm volatile(
-        "cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];" ::"r"(
-            smem_u32(dst_smem)),
-        "l"(src_gmem), "r"(bytes), "r"(smem_u32(bar))
-        : "memory");
-}
-__device__ __forceinline__ void mbar_wait(uint64_t *bar, uint32_t parity) {
-    asm volatile(
-        "{\n"
-        ".reg .pred p;\n"
-        "WAIT_%=:\n"
-        "mbarrier.try_wait.parity.shared::cta.b64 p, [%0], %1;\n"
-        "@p bra DONE_%=;\n"
-        "bra WAIT_%=;\n"
-        "DONE_%=:\n"
-        "}\n" ::"r"(smem_u32(bar)),
-        "r"(parity)
-        : "memory");
-}
-
 template <typename T, int IPT>
 __global__ void __launch_bounds__(MG_THREADS)
 spmv_merge_kernel(uint32_t nrows, uint32_t nnz, const uint32_t *__restrict__ ptr,
@@ -339,7 +304,10 @@ spmv_merge_kernel(uint32_t nrows, uint32_t nnz, const uint32_t *__restrict__ ptr
     // (1a) TMA: the 16-byte aligned superset [za, zb) of the tile's slice, one bulk copy per array
     const uint32_t za = z0 & ~3u, zb = (z1 + 3u) & ~3u;     // arrays carry 16 entries of slack
     const uint32_t shift = z0 - za;
-    if (threadIdx.x == 0) mbar_init(&s_bar, 1);
+    if (threadIdx.x == 0) {
+        mbar_init(&s_bar, 1);
+        mbar_init_fence();
+    }
     __syncthreads();
     if (threadIdx.x == 0 && zb > za) {
         mbar_expect_tx(&s_bar, (zb - za) * (uint32_t)(sizeof(uint32_t) + sizeof(T)));
@@ -481,31 +449,9 @@ void spmv_merge(spl_ctx *ctx, const spl_mat *a, const T *x, T *y) {
 //   * lanes take the entries of a row exactly as the vector kernel does, so the two kernels give the
 //     same bits; with one lane per row the row sum runs in ascending column order: bit-identical to
 //     the reference's `&A * &X` (src/csr/ops/mul.rs:25-40).
+// The tile layout and the consumers' row loop are those of stream_tile.cuh (shared with the fused
+// gather kernel, gather.cu); the copy and barrier primitives are those of ptx.cuh.
 constexpr uint32_t kStreamXEdgeMax = 1u << 15;     // longest leading edge of x one tile prefetches (elements)
-
-// L2 eviction policy for the matrix stream: read once, so it should not push x (re-read by other
-// tiles) out of L2
-__device__ __forceinline__ uint64_t l2_policy_evict_first() {
-    uint64_t p;
-    asm volatile("createpolicy.fractional.L2::evict_first.b64 %0, 1.0;" : "=l"(p));
-    return p;
-}
-__device__ __forceinline__ void tma_bulk_g2s_hint(void *dst_smem, const void *src_gmem, uint32_t bytes, uint64_t *bar,
-                                                  uint64_t policy) {
-    asm volatile(
-        "cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes.L2::cache_hint [%0], [%1], %2, [%3], %4;" ::"r"(
-            smem_u32(dst_smem)),
-        "l"(src_gmem), "r"(bytes), "r"(smem_u32(bar)), "l"(policy)
-        : "memory");
-}
-__device__ __forceinline__ void mbar_arrive(uint64_t *bar) {
-    asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(smem_u32(bar)) : "memory");
-}
-__device__ __forceinline__ void l2_prefetch_bulk(const void *gmem, uint32_t bytes) {
-    asm volatile("cp.async.bulk.prefetch.L2.global [%0], %1;" ::"l"(gmem), "r"(bytes) : "memory");
-}
-__device__ __forceinline__ void griddep_wait() { asm volatile("griddepcontrol.wait;" ::: "memory"); }
-__device__ __forceinline__ void griddep_launch() { asm volatile("griddepcontrol.launch_dependents;" ::: "memory"); }
 
 // largest number of stored entries in any window of `rows` consecutive rows (bounds every tile)
 __global__ void stream_window_kernel(const uint32_t *__restrict__ ptr, uint32_t nrows, uint32_t rows,
@@ -592,24 +538,21 @@ __global__ void stream_edges_kernel(const uint32_t *__restrict__ ptr, const uint
     if (count) atomicAdd(regular, count);
 }
 
-constexpr int ST_CONSUMERS = 256;
-
 // TIGHT: registers held to 56 so that four CTAs fit on an SM; otherwise three CTAs with room for
 // eight f64 gathers and values in flight per lane.
 // PAT: the grid has regular tiles (stream_edges_kernel).  Their columns and row starts follow from the row
 // number and the row pattern, so the producer fetches only their values; the consumers take column
 // r + pat.off[j] for position j of row r, and everything else runs as on any tile (same bits).
 template <typename T, int LPR, int U, bool TIGHT, bool PAT, typename XG>
-__global__ void __launch_bounds__(ST_CONSUMERS + 32, TIGHT ? 4 : 3)
+__global__ void __launch_bounds__(TILE_CONSUMERS + 32, TIGHT ? 4 : 3)
 spmv_stream_kernel(uint32_t nrows, const uint32_t *__restrict__ ptr, const uint32_t *__restrict__ ind,
                    const T *__restrict__ val, const XG xg, T *__restrict__ y, const uint32_t *__restrict__ cta_rows,
                    const uint32_t *__restrict__ tile_lo, const uint32_t *__restrict__ xhi,
                    const uint32_t *__restrict__ xlo0, uint32_t max_tiles, uint32_t cap, uint32_t stages,
                    const T *__restrict__ x_edge, uint32_t x_lo, uint32_t x_hi, int l2_hint,
                    const uint32_t *__restrict__ tile_reg, const __grid_constant__ RowPattern pat) {
-    constexpr uint32_t CONS = ST_CONSUMERS;
-    constexpr uint32_t R = CONS / LPR;
-    constexpr uint32_t PTRS = R + 4;           // pointer slots per stage: R + 1 needed, whole 16-byte units
+    constexpr uint32_t CONS = TILE_CONSUMERS;
+    constexpr uint32_t R = tile_rows(LPR), PTRS = tile_ptr_slots(R);
     extern __shared__ __align__(128) unsigned char st_raw[];
     // per stage: [cap] indices, [cap] values, [PTRS] row pointers; then the barriers; with PAT one word per
     // stage (the first entry position of a regular tile, ~0 for any other) and the row pattern
@@ -625,6 +568,7 @@ spmv_stream_kernel(uint32_t nrows, const uint32_t *__restrict__ ptr, const uint3
             mbar_init(full + s, 1);
             mbar_init(empty + s, CONS / 32);
         }
+        mbar_init_fence();
     }
     if (PAT && threadIdx.x < pat.len) s_pat[threadIdx.x] = pat.off[threadIdx.x];
     __syncthreads();
@@ -643,8 +587,7 @@ spmv_stream_kernel(uint32_t nrows, const uint32_t *__restrict__ ptr, const uint3
         for (uint32_t k = 0; k < ntiles; ++k) {
             const uint32_t hi = __ldg(t_lo + k + 1), x1 = __ldg(t_xhi + k);     // consecutive words: L1 hits
             if (k >= stages) mbar_wait(empty + s, phase ^ 1u);     // the consumers are done with this stage
-            const uint32_t za = lo & ~3u, zb = (hi + 3u) & ~3u;    // 16-byte aligned superset; the arrays carry slack
-            const uint32_t cnt = zb - za;
+            const uint32_t za = slice_lo(lo), cnt = slice_hi(hi) - za;
             // a regular tile: no pointer or index slice, its first entry position goes through the stage
             const bool regular = PAT && __ldg(t_reg + k);
             if (PAT) s_reg_lo[s] = regular ? lo : ~0u;             // published by the arrive below (release)
@@ -697,31 +640,18 @@ spmv_stream_kernel(uint32_t nrows, const uint32_t *__restrict__ ptr, const uint3
         if (reg_lo != ~0u) {
             if (r < re) { p0 = (reg_lo & 3u) + rl * pat.len; e = p0 + pat.len; cb = s_pat - p0; cadd = r; }
         } else {
-            const uint32_t za = cp[0] & ~3u;
+            const uint32_t za = slice_lo(cp[0]);
             if (r < re) { p0 = cp[rl] - za; e = cp[rl + 1] - za; }
         }
         T acc = (T)0;
-        auto row_sum = [&](auto gather) {
-            for (uint32_t j = p0 + sub; j < e; j += U * LPR) {
-                uint32_t c[U];
-                T xv[U], v[U];
-#pragma unroll
-                for (int u = 0; u < U; ++u) c[u] = j + u * LPR < e ? cb[j + u * LPR] + cadd : 0xffffffffu;
-#pragma unroll
-                for (int u = 0; u < U; ++u) xv[u] = c[u] != 0xffffffffu ? gather(c[u]) : (T)0;
-#pragma unroll
-                for (int u = 0; u < U; ++u) v[u] = j + u * LPR < e ? cv[j + u * LPR] : (T)0;
-#pragma unroll
-                for (int u = 0; u < U; ++u) acc += j + u * LPR < e ? v[u] * xv[u] : (T)0;      // 0, never 0 * inf
-            }
-        };
         // the row's columns are sorted: first and last entry bound them
-        if (e <= p0 || xg.all_local(cb[p0] + cadd, cb[e - 1] + cadd)) row_sum([&](uint32_t c) { return xg.local(c); });
-        else row_sum([&](uint32_t c) { return xg(c); });
+        if (e <= p0 || xg.all_local(cb[p0] + cadd, cb[e - 1] + cadd))
+            tile_row_sum<T, LPR, U>(acc, cb, cadd, cv, p0, e, sub, [&](uint32_t c) { return xg.local(c); });
+        else
+            tile_row_sum<T, LPR, U>(acc, cb, cadd, cv, p0, e, sub, [&](uint32_t c) { return xg(c); });
         __syncwarp();
         if (lane_id() == 0) mbar_arrive(empty + s);
-#pragma unroll
-        for (int o = LPR / 2; o > 0; o >>= 1) acc += __shfl_xor_sync(0xffffffffu, acc, o);
+        acc = row_lanes_sum<LPR>(acc);
         if (sub == 0 && r < re) y[r] = xg.poisoned() ? (T)NAN : acc;
         if (++s == stages) { s = 0; phase ^= 1u; }
     }
@@ -732,9 +662,8 @@ inline int env_int(const char *name, int fallback) {
     return e ? std::atoi(e) : fallback;
 }
 
-inline int stream_consumers() { return ST_CONSUMERS; }
 inline size_t stream_stage_bytes(const spl_mat *a) {
-    return (size_t)a->stream_cap * (4 + a->vsize()) + ((size_t)a->stream_rows + 4) * 4;
+    return (size_t)a->stream_cap * (4 + a->vsize()) + (size_t)tile_ptr_slots(a->stream_rows) * 4;
 }
 RowPattern row_pattern(const spl_mat *a) {
     RowPattern p{};
@@ -757,7 +686,7 @@ void stream_capacity(spl_ctx *ctx, spl_mat *a, uint32_t rows_per_tile) {
     check_launch(ctx, "stream_window");
     uint32_t max_window = 0;
     read_back(ctx, ctx->d_scratch + 1, &max_window, 1);
-    const uint32_t cap = (max_window + 6u + 3u) & ~3u;            // the 16-byte aligned superset of the largest slice
+    const uint32_t cap = stage_capacity(max_window);
     // three stages of it (with the pointer slices) must fit beside the barriers
     if (3 * ((size_t)cap * (4 + a->vsize()) + ((size_t)rows_per_tile + 4) * 4) + 64 <= 226 * 1024) a->stream_cap = cap;
 }
@@ -808,7 +737,7 @@ uint32_t stream_resident(K k, size_t smem, std::atomic<size_t> &smem_set, std::a
     uint64_t oc = occ_cache.load(std::memory_order_relaxed);     // (smem << 8) | resident CTAs
     if ((oc >> 8) != smem) {
         int resident = 0;
-        SPL_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&resident, k, ST_CONSUMERS + 32, smem));
+        SPL_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&resident, k, TILE_CONSUMERS + 32, smem));
         SPL_REQUIRE(resident >= 1, SPL_ERR_CUDA, "stream SpMV: no CTA fits on an SM");
         oc = ((uint64_t)smem << 8) | (uint64_t)resident;
         occ_cache.store(oc, std::memory_order_relaxed);
@@ -822,7 +751,7 @@ template <typename T, int LPR, int U, bool TIGHT, typename XG>
 void launch_stream(spl_ctx *ctx, const spl_mat *a, const XG &xg, T *y, const T *x_edge, uint32_t x_lo, uint32_t x_hi) {
     auto k_csr = spmv_stream_kernel<T, LPR, U, TIGHT, false, XG>;
     auto k_pat = spmv_stream_kernel<T, LPR, U, TIGHT, true, XG>;
-    constexpr int CONS = ST_CONSUMERS;
+    constexpr int CONS = TILE_CONSUMERS;
     // shape (measured, profiles/r2_spmv_notes.md): three stages, three CTAs of 64 registers per SM; a
     // deeper ring or a fourth, register-starved CTA does not pay
     const size_t stage_bytes = stream_stage_bytes(a);
@@ -923,7 +852,7 @@ void spmv_peer_t(spl_ctx *ctx, const spl_mat *a, const PeerX &px, T *y, int lane
     const XPeer<T> xg = make_xpeer<T>(ctx, px);
     if (a->plan_kernel == SPL_SPMV_STREAM && !std::getenv("SPL_PEER_VECTOR"))   // leading-edge prefetch inside the own slice
         spmv_stream<T>(ctx, a, xg, y, xg.mine - xg.my_start, xg.my_start, xg.my_start + xg.my_len);
-    else spmv_vector<T>(ctx, a, xg, y, lanes);
+    else spmv_vector<T>(ctx, a, xg, y, lanes, 0, a->nrows);
 }
 
 // ------------------------------------------------------------------ nnz-split kernel
@@ -1398,7 +1327,7 @@ void spmv_plan(spl_ctx *ctx, spl_mat *a) {
     a->plan_lanes = lanes;
     // stream kernel: the largest window of 256 / lanes rows sizes its shared-memory stages; tiles that follow
     // the row pattern stream their values only
-    stream_capacity(ctx, a, (uint32_t)stream_consumers() / (uint32_t)lanes);
+    stream_capacity(ctx, a, tile_rows(lanes));
     plan_pattern(ctx, a);
     // merge-path tile starts (matrix-only data, cached)
     const int ipt = a->dtype == SPL_F64 ? merge_ipt<double>() : merge_ipt<float>();
@@ -1424,7 +1353,7 @@ void spmv_plan(spl_ctx *ctx, spl_mat *a) {
     a->plan_kernel = skewed ? SPL_SPMV_SPLIT : SPL_SPMV_VECTOR;
     // regular rows, a tile fits in shared memory and there is at least a tile per resident CTA: the
     // persistent stream kernel (same bits as the vector kernel: same lanes, same order)
-    if (!skewed && a->stream_cap && (uint64_t)a->nrows * lanes >= (uint64_t)ctx->num_sms * 3u * ST_CONSUMERS)
+    if (!skewed && a->stream_cap && (uint64_t)a->nrows * lanes >= (uint64_t)ctx->num_sms * 3u * TILE_CONSUMERS)
         a->plan_kernel = SPL_SPMV_STREAM;
     // the plan arrays were written on this context's stream: make them visible to any other stream
     SPL_CUDA(cudaStreamSynchronize(ctx->stream));
@@ -1524,10 +1453,10 @@ void spmv(spl_ctx *ctx, const spl_mat *a, const void *x, void *y, int kernel, in
     if (kernel == SPL_SPMV_STREAM) {
         spl_mat *m = const_cast<spl_mat *>(a);
         spmv_plan(ctx, m);
-        if (a->stream_rows != (uint32_t)stream_consumers() / (uint32_t)a->plan_lanes) {     // measurement knob changed
+        if (a->stream_rows != tile_rows(a->plan_lanes)) {     // measurement knob changed
             std::lock_guard<std::mutex> lock(m->plan_mu);
             SPL_CUDA(cudaStreamSynchronize(ctx->stream));
-            stream_capacity(ctx, m, (uint32_t)stream_consumers() / (uint32_t)a->plan_lanes);
+            stream_capacity(ctx, m, tile_rows(a->plan_lanes));
         }
         SPL_REQUIRE(a->nnz == 0 || a->stream_cap, SPL_ERR_UNSUPPORTED,
                     "stream SpMV: a tile of rows does not fit in shared memory (skewed rows: use SPLIT)");
@@ -1557,8 +1486,8 @@ void spmv(spl_ctx *ctx, const spl_mat *a, const void *x, void *y, int kernel, in
         return;
     }
     if (kernel == SPL_SPMV_VECTOR) {
-        if (a->dtype == SPL_F32) spmv_vector<float>(ctx, a, XLocal<float>{(const float *)x}, (float *)y, lanes);
-        else spmv_vector<double>(ctx, a, XLocal<double>{(const double *)x}, (double *)y, lanes);
+        if (a->dtype == SPL_F32) spmv_vector<float>(ctx, a, XLocal<float>{(const float *)x}, (float *)y, lanes, 0, a->nrows);
+        else spmv_vector<double>(ctx, a, XLocal<double>{(const double *)x}, (double *)y, lanes, 0, a->nrows);
         return;
     }
     if (kernel == SPL_SPMV_MERGE) {
@@ -1615,26 +1544,6 @@ __global__ void chunk_need_kernel(const uint32_t *__restrict__ ptr, const uint32
     if (lane_id() == 0 && m && r < nrows) atomicMax(need + (uint32_t)(r / rows_per_chunk), m);
 }
 
-template <typename T, int LPR, typename XG>
-void launch_vector_rows(spl_ctx *ctx, const spl_mat *a, const XG &xg, T *y, uint32_t r0, uint32_t r1) {
-    const uint64_t threads = (uint64_t)(r1 - r0) * LPR;
-    spmv_vector_kernel<T, LPR, XG><<<div_up(threads, 256), 256, 0, ctx->stream>>>(
-        r1 - r0, a->ptr + r0, a->ind, static_cast<const T *>(a->val), xg, y + r0);
-    check_launch(ctx, "spmv_vector");
-}
-
-template <typename T, typename XG>
-void spmv_vector_rows(spl_ctx *ctx, const spl_mat *a, const XG &xg, T *y, int lanes, uint32_t r0, uint32_t r1) {
-    switch (lanes) {
-        case 1: launch_vector_rows<T, 1>(ctx, a, xg, y, r0, r1); break;
-        case 2: launch_vector_rows<T, 2>(ctx, a, xg, y, r0, r1); break;
-        case 4: launch_vector_rows<T, 4>(ctx, a, xg, y, r0, r1); break;
-        case 8: launch_vector_rows<T, 8>(ctx, a, xg, y, r0, r1); break;
-        case 16: launch_vector_rows<T, 16>(ctx, a, xg, y, r0, r1); break;
-        default: launch_vector_rows<T, 32>(ctx, a, xg, y, r0, r1); break;
-    }
-}
-
 void plan_pipeline(spl_ctx *ctx, spl_mat *a) {
     constexpr int K = spl_ctx::kPipeChunks;
     std::lock_guard<std::mutex> lock(a->plan_mu);
@@ -1654,6 +1563,23 @@ void plan_pipeline(spl_ctx *ctx, spl_mat *a) {
     a->pipe_state.store(1, std::memory_order_release);
 }
 
+// The upload and download streams of the host-vector products and the events that order them against the compute
+// stream, created on first use.
+void pipe_streams(spl_ctx *ctx) {
+    if (ctx->up_stream) return;
+    SPL_CUDA(cudaStreamCreateWithFlags(&ctx->up_stream, cudaStreamNonBlocking));
+    SPL_CUDA(cudaStreamCreateWithFlags(&ctx->down_stream, cudaStreamNonBlocking));
+    for (cudaEvent_t &e : ctx->pipe_ev) SPL_CUDA(cudaEventCreateWithFlags(&e, cudaEventDisableTiming));
+}
+
+// Pageable host memory makes every cudaMemcpyAsync block the host: copies overlap only with pinned memory.
+bool is_pinned(const void *p) {
+    cudaPointerAttributes at{};
+    const bool ok = cudaPointerGetAttributes(&at, p) == cudaSuccess && at.type == cudaMemoryTypeHost;
+    cudaGetLastError();
+    return ok;
+}
+
 }  // namespace
 
 bool spmv_host_pipelined(spl_ctx *ctx, const spl_mat *a, const void *x_host, void *y_host, void *x_dev,
@@ -1662,22 +1588,12 @@ bool spmv_host_pipelined(spl_ctx *ctx, const spl_mat *a, const void *x_host, voi
     a = csr_form(ctx, a);
     const size_t vs = a->vsize();
     if ((size_t)a->nrows * vs < (1u << 20) || a->nnz == 0) return false;      // small: one copy each way
-    {   // pageable host memory makes every cudaMemcpyAsync block the host: nothing would overlap
-        cudaPointerAttributes ax{}, ay{};
-        const bool okx = cudaPointerGetAttributes(&ax, x_host) == cudaSuccess && ax.type == cudaMemoryTypeHost;
-        const bool oky = cudaPointerGetAttributes(&ay, y_host) == cudaSuccess && ay.type == cudaMemoryTypeHost;
-        cudaGetLastError();
-        if (!okx || !oky) return false;
-    }
+    if (!is_pinned(x_host) || !is_pinned(y_host)) return false;               // nothing would overlap
     spl_mat *m = const_cast<spl_mat *>(a);
     spmv_plan(ctx, m);
     if (a->plan_kernel != SPL_SPMV_VECTOR) return false;                      // skewed rows: whole-matrix kernels
     if (!a->pipe_state.load(std::memory_order_acquire)) plan_pipeline(ctx, m);
-    if (!ctx->up_stream) {
-        SPL_CUDA(cudaStreamCreateWithFlags(&ctx->up_stream, cudaStreamNonBlocking));
-        SPL_CUDA(cudaStreamCreateWithFlags(&ctx->down_stream, cudaStreamNonBlocking));
-        for (cudaEvent_t &e : ctx->pipe_ev) SPL_CUDA(cudaEventCreateWithFlags(&e, cudaEventDisableTiming));
-    }
+    pipe_streams(ctx);
     cudaEvent_t *up_ev = ctx->pipe_ev, *run_ev = ctx->pipe_ev + K;
     cudaEvent_t start_ev = ctx->pipe_ev[2 * K], end_ev = ctx->pipe_ev[2 * K + 1];
     const unsigned char *xh = static_cast<const unsigned char *>(x_host);
@@ -1700,9 +1616,9 @@ bool spmv_host_pipelined(spl_ctx *ctx, const spl_mat *a, const void *x_host, voi
         SPL_CUDA(cudaEventRecord(up_ev[c], ctx->up_stream));
         SPL_CUDA(cudaStreamWaitEvent(ctx->stream, up_ev[c], 0));
         if (a->dtype == SPL_F32)
-            spmv_vector_rows<float>(ctx, a, XLocal<float>{(const float *)x_dev}, (float *)y_dev, a->plan_lanes, r0, r1);
+            spmv_vector<float>(ctx, a, XLocal<float>{(const float *)x_dev}, (float *)y_dev, a->plan_lanes, r0, r1);
         else
-            spmv_vector_rows<double>(ctx, a, XLocal<double>{(const double *)x_dev}, (double *)y_dev, a->plan_lanes, r0, r1);
+            spmv_vector<double>(ctx, a, XLocal<double>{(const double *)x_dev}, (double *)y_dev, a->plan_lanes, r0, r1);
         SPL_CUDA(cudaEventRecord(run_ev[c], ctx->stream));
         SPL_CUDA(cudaStreamWaitEvent(ctx->down_stream, run_ev[c], 0));
         SPL_CUDA(cudaMemcpyAsync(yh + (size_t)r0 * vs, yd + (size_t)r0 * vs, (size_t)(r1 - r0) * vs,
@@ -1744,11 +1660,7 @@ void spmv_peer_host(spl_ctx *ctx, const spl_mat *a, const PeerX &px, void *const
     const size_t vs = a->vsize();
     const uint32_t my_len = px.start[px.rank + 1] - px.start[px.rank];
     unsigned char *x_slice = static_cast<unsigned char *>(const_cast<void *>(px.slice[px.rank]));
-    if (!ctx->up_stream) {
-        SPL_CUDA(cudaStreamCreateWithFlags(&ctx->up_stream, cudaStreamNonBlocking));
-        SPL_CUDA(cudaStreamCreateWithFlags(&ctx->down_stream, cudaStreamNonBlocking));
-        for (cudaEvent_t &e : ctx->pipe_ev) SPL_CUDA(cudaEventCreateWithFlags(&e, cudaEventDisableTiming));
-    }
+    pipe_streams(ctx);
     cudaEvent_t *run_ev = ctx->pipe_ev + K;
     cudaEvent_t start_ev = ctx->pipe_ev[2 * K], end_ev = ctx->pipe_ev[2 * K + 1], up_ev = ctx->pipe_ev[0];
     // upload behind whatever the compute stream did to the slice before (a previous product may still gather from
@@ -1761,21 +1673,15 @@ void spmv_peer_host(spl_ctx *ctx, const spl_mat *a, const PeerX &px, void *const
     SPL_CUDA(cudaEventRecord(up_ev, ctx->up_stream));
     SPL_CUDA(cudaStreamWaitEvent(ctx->stream, up_ev, 0));
     peer_barrier(ctx, px.world, px.rank, flag_ptrs, epoch, timeout_ms);
-    const bool pinned = [&] {
-        cudaPointerAttributes ay{};
-        const bool ok = cudaPointerGetAttributes(&ay, y_host_local) == cudaSuccess && ay.type == cudaMemoryTypeHost;
-        cudaGetLastError();
-        return ok;
-    }();
-    const int chunks = (pinned && (size_t)a->nrows * vs >= (1u << 20)) ? K : 1;
+    const int chunks = (is_pinned(y_host_local) && (size_t)a->nrows * vs >= (1u << 20)) ? K : 1;
     const uint32_t per = (uint32_t)((((uint64_t)a->nrows + chunks - 1) / chunks + 255) / 256 * 256);
     unsigned char *yd = static_cast<unsigned char *>(y_dev), *yh = static_cast<unsigned char *>(y_host_local);
     for (int c = 0; c < chunks; ++c) {
         const uint32_t r0 = (uint32_t)std::min<uint64_t>((uint64_t)c * per, a->nrows);
         const uint32_t r1 = (uint32_t)std::min<uint64_t>((uint64_t)(c + 1) * per, a->nrows);
         if (r1 <= r0) continue;
-        if (a->dtype == SPL_F32) spmv_vector_rows<float>(ctx, a, make_xpeer<float>(ctx, px), (float *)y_dev, a->plan_lanes, r0, r1);
-        else spmv_vector_rows<double>(ctx, a, make_xpeer<double>(ctx, px), (double *)y_dev, a->plan_lanes, r0, r1);
+        if (a->dtype == SPL_F32) spmv_vector<float>(ctx, a, make_xpeer<float>(ctx, px), (float *)y_dev, a->plan_lanes, r0, r1);
+        else spmv_vector<double>(ctx, a, make_xpeer<double>(ctx, px), (double *)y_dev, a->plan_lanes, r0, r1);
         SPL_CUDA(cudaEventRecord(run_ev[c], ctx->stream));
         SPL_CUDA(cudaStreamWaitEvent(ctx->down_stream, run_ev[c], 0));
         SPL_CUDA(cudaMemcpyAsync(yh + (size_t)r0 * vs, yd + (size_t)r0 * vs, (size_t)(r1 - r0) * vs,
