@@ -21,8 +21,10 @@
  *  - Limits: dims below 2^32 (device indices are 32 bit).  Positions are 32 bit on the fast
  *    paths; a CsrMatrix / CscMatrix with 2^32 - 65536 stored entries or more ("wide") keeps a 64-bit
  *    pointer array on the device and supports construction + validation, SpMV, transpose, CSR<->CSC,
- *    download and chunked iteration; COO assembly, add/sub/mul/neg and the sharded calls answer
- *    SPL_ERR_UNSUPPORTED for it (COO length and intermediate products stay below 2^32 - 65536).
+ *    download and chunked iteration, and COO assembly produces it from 2^32 - 65536 triplets or more
+ *    (fewer than that per row of a CSR, per column of a CSC result).  Add/sub/mul/neg and the sharded
+ *    calls answer SPL_ERR_UNSUPPORTED for it (their lengths and intermediate products stay below
+ *    2^32 - 65536).
  */
 #ifndef SPL_H
 #define SPL_H
@@ -113,7 +115,14 @@ uint64_t spl_launch_count(const spl_ctx *ctx);
  *   impl From<&DokMatrix<T>> for CscMatrix<T>   src/csc/conv/dok.rs:3-76
  * (keys unique, explicit zeros kept).  Host SoA arrays of length len; the bound
  * checks of CooMatrix::push (src/coo.rs:431-435) are re-checked on the device
- * (SPL_ERR_ARG).  nrows, ncols must be > 0 (src/coo.rs:105-106). */
+ * (SPL_ERR_ARG).  nrows, ncols must be > 0 (src/coo.rs:105-106).
+ * len may be 2^32 - 65536 or more: the list is then assembled in buckets of whole rows (CSR) / columns
+ * (CSC), each assembled as a shorter list and the parts stitched, with the same result bit for bit.  The
+ * result is wide (64-bit pointers) when it keeps 2^32 - 65536 entries or more, else an ordinary matrix.
+ * One row (CSR) / column (CSC) with 2^32 - 65536 triplets or more gives SPL_ERR_UNSUPPORTED.  Bucket size
+ * follows the device memory free at the call; the peak is the input + one bucket's scratch (about
+ * 3 (8 + V) bytes per triplet) + the parts so far, and at the end the input + the parts + the output.
+ * The host front uploads such a list through a fixed staging buffer. */
 int spl_mat_from_coo(spl_ctx *ctx, int format, int dtype, uint64_t nrows, uint64_t ncols,
                      uint64_t len, const uint64_t *row, const uint64_t *col, const void *val,
                      int dedup, int dropzero, spl_mat **out);
@@ -139,8 +148,8 @@ int spl_mat_from_coo_dev(spl_ctx *ctx, int format, int dtype, uint64_t nrows, ui
  *   spl_coo_invalidate get_mut / iter_mut                src/coo.rs:408-412, 514-518: the caller is about to
  *                     write values through the host pointers from entry `first` on; what the copy
  *                     stream already took from there is sent again at the next conversion
- *   spl_mat_from_coo_builder   From<&CooMatrix> for CsrMatrix / CscMatrix (as spl_mat_from_coo);
- *                     the builder stays valid and can be pushed to and converted again. */
+ *   spl_mat_from_coo_builder   From<&CooMatrix> for CsrMatrix / CscMatrix (as spl_mat_from_coo, any
+ *                     length); the builder stays valid and can be pushed to and converted again. */
 typedef struct spl_coo spl_coo;
 int spl_coo_create(spl_ctx *ctx, int dtype, uint64_t nrows, uint64_t ncols, uint64_t capacity,
                    spl_coo **out);

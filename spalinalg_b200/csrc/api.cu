@@ -212,10 +212,9 @@ int spl_mat_from_coo_dev(spl_ctx *ctx, int format, int dtype, uint64_t nrows, ui
     *out = nullptr;
     check_enums(format, dtype);
     check_dims(ctx, nrows, ncols);
-    SPL_REQUIRE(len < kMaxEntries, SPL_ERR_UNSUPPORTED, "COO length must be below 2^32 - 65536");
     SPL_REQUIRE(len == 0 || (row_dev && col_dev && val_dev), SPL_ERR_ARG, "NULL COO array");
-    *out = assemble_from_coo_dev(ctx, format, dtype, (uint32_t)nrows, (uint32_t)ncols, (uint32_t)len,
-                                 row_dev, col_dev, val_dev, dedup, dropzero);
+    *out = assemble_from_coo_any(ctx, format, dtype, (uint32_t)nrows, (uint32_t)ncols, len, row_dev, col_dev,
+                                 val_dev, dedup, dropzero);
     publish_mat(ctx, *out);
     API_END(ctx)
 }
@@ -228,12 +227,23 @@ int spl_mat_from_coo(spl_ctx *ctx, int format, int dtype, uint64_t nrows, uint64
     *out = nullptr;
     check_enums(format, dtype);
     check_dims(ctx, nrows, ncols);
-    SPL_REQUIRE(len < kMaxEntries, SPL_ERR_UNSUPPORTED, "COO length must be below 2^32 - 65536");
     SPL_REQUIRE(len == 0 || (row && col && val), SPL_ERR_ARG, "NULL COO array");
     const size_t vs = dtype == SPL_F32 ? 4 : 8;
     Tmp<uint32_t> r32(ctx, len), c32(ctx, len);
     Tmp<unsigned char> v(ctx, len * vs);
-    if (len) {
+    if (assemble_is_bucketed(len)) {       // long lists: the indices narrow through a fixed staging buffer
+        constexpr uint64_t kChunk = 1ull << 26;
+        Tmp<uint64_t> stage(ctx, std::min(kChunk, len));
+        SPL_CUDA(cudaMemsetAsync(ctx->d_scratch, 0, sizeof(uint32_t), ctx->stream));
+        for (uint64_t at = 0; at < len; at += kChunk) {
+            const uint64_t cnt = std::min(kChunk, len - at);
+            SPL_CUDA(cudaMemcpyAsync(stage, row + at, cnt * 8, cudaMemcpyHostToDevice, ctx->stream));
+            narrow_u64(ctx, stage, r32 + at, cnt, nrows, ctx->d_scratch);
+            SPL_CUDA(cudaMemcpyAsync(stage, col + at, cnt * 8, cudaMemcpyHostToDevice, ctx->stream));
+            narrow_u64(ctx, stage, c32 + at, cnt, ncols, ctx->d_scratch);
+        }
+        SPL_CUDA(cudaMemcpyAsync(v, val, len * vs, cudaMemcpyHostToDevice, ctx->stream));
+    } else if (len) {
         Tmp<uint64_t> wide(ctx, len);
         SPL_CUDA(cudaMemsetAsync(ctx->d_scratch, 0, sizeof(uint32_t), ctx->stream));
         SPL_CUDA(cudaMemcpyAsync(wide, row, len * 8, cudaMemcpyHostToDevice, ctx->stream));
@@ -243,8 +253,8 @@ int spl_mat_from_coo(spl_ctx *ctx, int format, int dtype, uint64_t nrows, uint64
         SPL_CUDA(cudaMemcpyAsync(v, val, len * vs, cudaMemcpyHostToDevice, ctx->stream));
     }
     // bounds (CooMatrix::push, src/coo.rs:432-433) are re-checked on the narrowed arrays
-    *out = assemble_from_coo_dev(ctx, format, dtype, (uint32_t)nrows, (uint32_t)ncols, (uint32_t)len,
-                                 r32, c32, v, dedup, dropzero);
+    *out = assemble_from_coo_any(ctx, format, dtype, (uint32_t)nrows, (uint32_t)ncols, len, r32, c32, v, dedup,
+                                 dropzero);
     publish_mat(ctx, *out);
     API_END(ctx)
 }

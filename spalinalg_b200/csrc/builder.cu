@@ -70,10 +70,8 @@ void release(spl_coo *b) {
 // Grows host and device storage to at least `want` entries (amortised doubling, like Vec).
 void reserve(spl_coo *b, uint64_t want) {
     if (want <= b->cap) return;
-    SPL_REQUIRE(want < kMaxEntries, SPL_ERR_UNSUPPORTED, "COO length must be below 2^32 - 65536");
     uint64_t cap = b->cap ? b->cap : kMinCapacity;
     while (cap < want) cap *= 2;
-    if (cap >= kMaxEntries) cap = kMaxEntries - 1;
     const size_t vs = b->vsize();
     uint64_t *hr = nullptr, *hc = nullptr;
     unsigned char *hv = nullptr, *dv = nullptr;
@@ -310,8 +308,8 @@ int spl_mat_from_coo_builder(spl_ctx *ctx, spl_coo *b, int format, int dedup, in
             ctx->launches += b->copy->launches - b->counted_launches;
             b->counted_launches = b->copy->launches;
         }
-        *out = assemble_from_coo_dev(ctx, format, b->dtype, (uint32_t)b->nrows, (uint32_t)b->ncols,
-                                     (uint32_t)b->len, b->d_row, b->d_col, b->d_val, dedup, dropzero);
+        *out = assemble_from_coo_any(ctx, format, b->dtype, (uint32_t)b->nrows, (uint32_t)b->ncols, b->len,
+                                     b->d_row, b->d_col, b->d_val, dedup, dropzero);
         publish_mat(ctx, *out);
     } catch (const spl::Error &e) {
         ctx->last_error = e.msg;

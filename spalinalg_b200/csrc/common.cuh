@@ -267,6 +267,17 @@ __device__ __forceinline__ uint32_t upper_bound_u32(const uint32_t *__restrict__
     return lo;
 }
 
+// first index in [lo, hi) with a[idx] > key  (a non-decreasing), 64-bit positions
+__device__ __forceinline__ uint64_t upper_bound_u64(const uint64_t *__restrict__ a, uint64_t lo, uint64_t hi,
+                                                    uint64_t key) {
+    while (lo < hi) {
+        const uint64_t mid = lo + ((hi - lo) >> 1);
+        if (__ldg(a + mid) <= key) lo = mid + 1;
+        else hi = mid;
+    }
+    return lo;
+}
+
 // Streaming load (SASS LDG.E.NA, L1::no_allocate) for data a kernel reads exactly once with fully
 // coalesced warps — the col/val stream of the nnz-split and merge SpMV kernels — so that it does
 // not push the reusable x out of L1.  Measured on B200 (profiles/r1_spmv_notes.md): +6 % on the

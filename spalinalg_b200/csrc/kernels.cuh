@@ -10,6 +10,14 @@ namespace spl {
 spl_mat *assemble_from_coo_dev(spl_ctx *ctx, int format, int dtype, uint32_t nrows, uint32_t ncols,
                                uint32_t len, const uint32_t *row, const uint32_t *col,
                                const void *val, int dedup, int dropzero);
+// wide_assemble.cu — the assembly entry of every COO front (spl_mat_from_coo{,_dev}, the builder):
+// lists below 2^32 - 65536 triplets go to assemble_from_coo_dev unchanged; longer ones (or longer than
+// SPL_ASSEMBLE_BUCKET_MAX when that is set) are assembled in buckets of whole majors, and the result is
+// wide when it keeps 2^32 - 65536 entries or more.
+bool assemble_is_bucketed(uint64_t len);
+spl_mat *assemble_from_coo_any(spl_ctx *ctx, int format, int dtype, uint32_t nrows, uint32_t ncols,
+                               uint64_t len, const uint32_t *row, const uint32_t *col,
+                               const void *val, int dedup, int dropzero);
 // Shared tail of assembly and SpGEMM: sorted (key = major << minor_bits | minor, value) records
 // -> in-order segmented sum, optional zero drop, compaction, pointer array.  `vals` is updated
 // in place.  key64 selects uint64 keys, else uint32.
@@ -123,6 +131,9 @@ void wide_spmv(spl_ctx *ctx, const spl_mat *a, const void *x, void *y);
 spl_mat *wide_regroup(spl_ctx *ctx, const spl_mat *in, int out_format, uint32_t out_rows, uint32_t out_cols);
 void wide_entry_range(spl_ctx *ctx, const spl_mat *m, uint64_t start, uint32_t count, uint64_t *major_out,
                       uint64_t *minor_out);
+// out[i] = in[0] + ... + in[i - 1] for i in [0, n] (64-bit sums of 32-bit counts)
+void wide_exclusive_scan(spl_ctx *ctx, const uint32_t *in, uint32_t n, uint64_t *out);
+uint32_t wide_max_u32(spl_ctx *ctx, const uint32_t *a, uint32_t n);      // largest of a[0..n), 0 if n == 0
 void free_mat(spl_ctx *ctx, spl_mat *m);
 
 }  // namespace spl

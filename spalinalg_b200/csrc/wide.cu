@@ -7,7 +7,8 @@
 // below: validation (CsrMatrix::new, src/csr.rs:144-156), SpMV (the vector kernel with 64-bit
 // positions), transpose / CSR<->CSC (src/csr.rs:358-406, src/csc/conv/csr.rs:3-53: histogram +
 // 64-bit exclusive scan + scatter + per-segment repair, the reference's own three steps),
-// download and the chunks of iter().  Everything else on the path (assembly, add/sub, mul) answers
+// download and the chunks of iter().  COO assembly of such a matrix (2^32 - 65536 triplets or more)
+// runs in wide_assemble.cu on the scan below.  Everything else on the path (add/sub, mul) answers
 // SPL_ERR_UNSUPPORTED for a wide operand.
 #include <algorithm>
 
@@ -18,15 +19,6 @@ namespace spl {
 namespace {
 
 constexpr uint32_t kWideRepairMax = 256;      // longest output segment the transpose's repair pass ranks
-
-__device__ __forceinline__ uint64_t upper_bound_u64(const uint64_t *__restrict__ a, uint64_t lo, uint64_t hi, uint64_t key) {
-    while (lo < hi) {
-        const uint64_t mid = lo + ((hi - lo) >> 1);
-        if (__ldg(a + mid) <= key) lo = mid + 1;
-        else hi = mid;
-    }
-    return lo;
-}
 
 // ---- validation (assertions 7, 8, 9 of CsrMatrix::new) ---------------------------------------
 __global__ void wide_validate_ptr_kernel(const uint64_t *__restrict__ ptr, uint32_t nmajor, uint32_t *fail) {
@@ -214,6 +206,8 @@ wide_scan_downsweep_kernel(const uint32_t *__restrict__ in, uint32_t n, const un
     if (n > 0 && base <= (uint64_t)n - 1 && (uint64_t)n - 1 < base + WS_IPT) out[n] = run;
 }
 
+}  // namespace
+
 void wide_exclusive_scan(spl_ctx *ctx, const uint32_t *in, uint32_t n, uint64_t *out) {
     const unsigned tiles = div_up(n, WS_TILE);
     Tmp<unsigned long long> sums(ctx, tiles + 1);
@@ -224,6 +218,19 @@ void wide_exclusive_scan(spl_ctx *ctx, const uint32_t *in, uint32_t n, uint64_t 
     wide_scan_downsweep_kernel<<<tiles, WS_THREADS, 0, ctx->stream>>>(in, n, sums, out);
     check_launch(ctx, "wide_scan_downsweep");
 }
+
+uint32_t wide_max_u32(spl_ctx *ctx, const uint32_t *a, uint32_t n) {
+    if (n == 0) return 0;
+    const unsigned sgrid = (unsigned)ctx->num_sms * 16u;
+    SPL_CUDA(cudaMemsetAsync(ctx->d_scratch, 0, sizeof(uint32_t), ctx->stream));
+    wide_max_kernel<<<std::min<unsigned>(div_up(n, 256), sgrid), 256, 0, ctx->stream>>>(a, n, ctx->d_scratch);
+    check_launch(ctx, "wide_max");
+    uint32_t m = 0;
+    read_back(ctx, ctx->d_scratch, &m, 1);
+    return m;
+}
+
+namespace {
 
 template <typename VB, int LPR>
 __global__ void __launch_bounds__(256)
@@ -295,13 +302,9 @@ void wide_recompress_t(spl_ctx *ctx, const spl_mat *in, spl_mat *out) {
     const unsigned sgrid = (unsigned)ctx->num_sms * 16u;
     Tmp<uint32_t> counts(ctx, nminor);
     SPL_CUDA(cudaMemsetAsync(counts, 0, sizeof(uint32_t) * (size_t)nminor, ctx->stream));
-    SPL_CUDA(cudaMemsetAsync(ctx->d_scratch, 0, sizeof(uint32_t), ctx->stream));
     wide_minor_count_kernel<<<sgrid, 256, 0, ctx->stream>>>(in->ind, nnz, counts);
     check_launch(ctx, "wide_minor_count");
-    wide_max_kernel<<<std::min<unsigned>(div_up(nminor, 256), sgrid), 256, 0, ctx->stream>>>(counts, nminor, ctx->d_scratch);
-    check_launch(ctx, "wide_max");
-    uint32_t longest = 0;
-    read_back(ctx, ctx->d_scratch, &longest, 1);
+    const uint32_t longest = wide_max_u32(ctx, counts, nminor);
     SPL_REQUIRE(longest <= kWideRepairMax, SPL_ERR_UNSUPPORTED,
                 "transpose of a matrix with 2^32 or more entries: output segments longer than 256 entries are not supported");
     wide_exclusive_scan(ctx, counts, nminor, out->ptr64);

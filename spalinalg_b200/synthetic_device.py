@@ -56,6 +56,43 @@ def banded_device(torch, n, r0, r1, offsets, dtype, chunk=1 << 24):
     return rowptr, torch.cat(col_parts), torch.cat(val_parts)
 
 
+def band_value(torch, i, d):
+    """A[i, i + d] of scrambled_band_coo_device, f64 (int64 tensors i, d)."""
+    return 1.0 / (1.0 + d.abs().double()) + (i % 7).double() * 1e-3
+
+
+def scrambled_band_coo_device(torch, n, half, dtype, spare=0, a=1_000_000_007, b=12_345, chunk=1 << 25):
+    """Triplets of the n x n band with diagonals -half..half (A[i, i+d] = band_value), one per cell, in an
+    order scrambled by the bijection e = (a p + b) mod (2 half + 1) n of the slot index (a coprime to the
+    slot count): slot e is cell (e // (2 half + 1), e % (2 half + 1) - half), slots outside the matrix are
+    skipped.  Every stretch of the list gathers from the whole matrix.  int32 row, int32 col, values, with
+    `spare` unset slots at the end for the caller.  Returns (row, col, val, number of band cells)."""
+    import math
+    w = 2 * half + 1
+    slots = w * n
+    assert math.gcd(a, slots) == 1 and a * slots < 2 ** 63
+    cells = w * n - half * (half + 1)
+    row = torch.empty(cells + spare, device="cuda", dtype=torch.int32)
+    col = torch.empty(cells + spare, device="cuda", dtype=torch.int32)
+    val = torch.empty(cells + spare, device="cuda", dtype=dtype)
+    pos = 0
+    for s in range(0, slots, chunk):
+        p = torch.arange(s, min(slots, s + chunk), device="cuda", dtype=torch.int64)
+        e = (p * a + b) % slots
+        i, d = e // w, e % w - half
+        j = i + d
+        keep = (j >= 0) & (j < n)
+        i, d, j = i[keep], d[keep], j[keep]
+        k = i.numel()
+        row[pos:pos + k] = i.to(torch.int32)
+        col[pos:pos + k] = j.to(torch.int32)
+        val[pos:pos + k] = band_value(torch, i, d).to(dtype)
+        pos += k
+        del p, e, i, d, j, keep
+    assert pos == cells
+    return row, col, val, cells
+
+
 
 
 def device_view(torch, ptr: int, count: int, dtype):
