@@ -20,11 +20,17 @@
  *  - There is no CPU fallback: without a CUDA device spl_ctx_create fails.
  *  - Limits: dims below 2^32 (device indices are 32 bit).  Positions are 32 bit on the fast
  *    paths; a CsrMatrix / CscMatrix with 2^32 - 65536 stored entries or more ("wide") keeps a 64-bit
- *    pointer array on the device and supports construction + validation, SpMV, transpose, CSR<->CSC,
- *    download and chunked iteration, and COO assembly produces it from 2^32 - 65536 triplets or more
- *    (fewer than that per row of a CSR, per column of a CSC result).  Add/sub/mul/neg and the sharded
- *    calls answer SPL_ERR_UNSUPPORTED for it (their lengths and intermediate products stay below
- *    2^32 - 65536).
+ *    pointer array on the device and supports construction + validation, SpMV (CSR only), transpose,
+ *    CSR<->CSC, download and chunked iteration, and COO assembly produces it from 2^32 - 65536 triplets
+ *    or more (fewer than that per row of a CSR, per column of a CSC result).  Add/sub/mul/neg,
+ *    set_values, to_coo, the windowed and sharded products and SpMV of a wide CSC matrix answer
+ *    SPL_ERR_UNSUPPORTED for it (their lengths and intermediate products stay below 2^32 - 65536).
+ *    Test-only setting: the environment variable SPL_WIDE_MIN_NNZ=<n> makes every matrix created with
+ *    n stored entries or more wide (n clamped to [1, 2^32 - 65536]; a value that is not a number is
+ *    ignored; a matrix without entries is never wide), so that the wide kernels can be compared with
+ *    the usual ones at small sizes.  It applies to spl_mat_from_compressed,
+ *    spl_mat_from_compressed_dev64 and the result of bucketed COO assembly (see
+ *    SPL_ASSEMBLE_BUCKET_MAX); transposes and conversions keep the width of their input.
  */
 #ifndef SPL_H
 #define SPL_H
@@ -216,7 +222,10 @@ int spl_mat_neg(spl_ctx *ctx, const spl_mat *a, spl_mat **out);
  * (same arrays, dims swapped) this is y = B^T x. */
 int spl_spmv(spl_ctx *ctx, const spl_mat *a, const void *x_dev, void *y_dev);
 /* kernel: spl_spmv_kernel in bits 0-7; bits 8-15 optionally force the vector kernel's lanes per
- * row (1, 2, 4, 8, 16 or 32; 0 = planned value). */
+ * row (1, 2, 4, 8, 16 or 32; 0 = planned value).  On a wide matrix the argument is ignored: every
+ * value runs the vector kernel with 64-bit positions and lanes chosen from the mean row length, and
+ * gives the same bytes.  A wide matrix must be CSR: a wide CSC one gives SPL_ERR_UNSUPPORTED (convert
+ * it with spl_mat_convert first). */
 int spl_spmv_ex(spl_ctx *ctx, const spl_mat *a, const void *x_dev, void *y_dev, int kernel);
 /* Host-buffer form (the reference-facing `&A * &x`): uploads x, runs spl_spmv, downloads y,
  * synchronises.  With pinned vectors of a megabyte or more and a matrix for the vector kernel the
@@ -224,7 +233,8 @@ int spl_spmv_ex(spl_ctx *ctx, const spl_mat *a, const void *x_dev, void *y_dev, 
  * behind the kernels), so both directions of the PCIe link work at once; same result bit for bit. */
 int spl_spmv_host(spl_ctx *ctx, const spl_mat *a, const void *x_host, void *y_host);
 /* Which kernel AUTO resolves to for this matrix (SPL_SPMV_VECTOR / _SPLIT) and the vector kernel's
- * lanes per row. */
+ * lanes per row.  A wide matrix answers SPL_SPMV_VECTOR and 0 lanes (its kernel picks the lanes at
+ * each product). */
 int spl_spmv_choice(spl_ctx *ctx, const spl_mat *a, int *kernel, int *lanes_per_row);
 
 /* ---- access --------------------------------------------------------------- */

@@ -315,7 +315,7 @@ int spl_mat_from_compressed(spl_ctx *ctx, int format, int dtype, uint64_t nrows,
     if (val_len != ptr[nmajor]) invalid(ctx, 6, kReasonText[6]);
     const uint64_t nnz = ind_len;
     SPL_REQUIRE(nnz == 0 || (ind && val), SPL_ERR_ARG, "NULL array");
-    if (nnz >= kMaxEntries) {              // 64-bit positions: the pointers go up as they are, the indices narrow in chunks
+    if (nnz >= wide_min_nnz()) {           // 64-bit positions: the pointers go up as they are, the indices narrow in chunks
         spl_mat *w = new_wide_mat(ctx, format, dtype, (uint32_t)nrows, (uint32_t)ncols, nnz);
         try {
             SPL_CUDA(cudaMemcpyAsync(w->ptr64, ptr, (nmajor + 1) * 8, cudaMemcpyHostToDevice, ctx->stream));
@@ -391,7 +391,7 @@ int spl_mat_from_compressed_dev64(spl_ctx *ctx, int format, int dtype, uint64_t 
         if (ends[0] != 0 || ends[1] != 0) invalid(ctx, 4, kReasonText[4]);
         if ((((uint64_t)ends[3] << 32) | ends[2]) != nnz) invalid(ctx, 5, kReasonText[5]);
     }
-    if (nnz < kMaxEntries) {                             // fits 32-bit positions: the usual matrix
+    if (nnz < wide_min_nnz()) {                          // fits 32-bit positions: the usual matrix
         spl_mat *m = new_mat(ctx, format, dtype, (uint32_t)nrows, (uint32_t)ncols, (uint32_t)nnz);
         try {
             SPL_CUDA(cudaMemsetAsync(ctx->d_scratch, 0, sizeof(uint32_t), ctx->stream));
@@ -507,12 +507,12 @@ int spl_mat_transpose(spl_ctx *ctx, const spl_mat *in, spl_mat **out) {
 
 int spl_mat_add(spl_ctx *ctx, const spl_mat *a, const spl_mat *b, spl_mat **out) {
     API_BEGIN(ctx)
+    SPL_REQUIRE(a && b && out, SPL_ERR_ARG, "NULL handle");
+    *out = nullptr;
     require_narrow(a, "spl_mat_add");
     require_narrow(b, "spl_mat_add");
     MatUse use_a(ctx, a);
     MatUse use_b(ctx, b);
-    SPL_REQUIRE(a && b && out, SPL_ERR_ARG, "NULL handle");
-    *out = nullptr;
     *out = addsub(ctx, a, b, 0);
     publish_mat(ctx, *out);
     API_END(ctx)
@@ -520,12 +520,12 @@ int spl_mat_add(spl_ctx *ctx, const spl_mat *a, const spl_mat *b, spl_mat **out)
 
 int spl_mat_sub(spl_ctx *ctx, const spl_mat *a, const spl_mat *b, spl_mat **out) {
     API_BEGIN(ctx)
+    SPL_REQUIRE(a && b && out, SPL_ERR_ARG, "NULL handle");
+    *out = nullptr;
     require_narrow(a, "spl_mat_sub");
     require_narrow(b, "spl_mat_sub");
     MatUse use_a(ctx, a);
     MatUse use_b(ctx, b);
-    SPL_REQUIRE(a && b && out, SPL_ERR_ARG, "NULL handle");
-    *out = nullptr;
     *out = addsub(ctx, a, b, 1);
     publish_mat(ctx, *out);
     API_END(ctx)
@@ -533,12 +533,12 @@ int spl_mat_sub(spl_ctx *ctx, const spl_mat *a, const spl_mat *b, spl_mat **out)
 
 int spl_mat_mul(spl_ctx *ctx, const spl_mat *a, const spl_mat *b, spl_mat **out) {
     API_BEGIN(ctx)
+    SPL_REQUIRE(a && b && out, SPL_ERR_ARG, "NULL handle");
+    *out = nullptr;
     require_narrow(a, "spl_mat_mul");
     require_narrow(b, "spl_mat_mul");
     MatUse use_a(ctx, a);
     MatUse use_b(ctx, b);
-    SPL_REQUIRE(a && b && out, SPL_ERR_ARG, "NULL handle");
-    *out = nullptr;
     *out = spgemm(ctx, a, b);
     publish_mat(ctx, *out);
     API_END(ctx)
@@ -546,10 +546,10 @@ int spl_mat_mul(spl_ctx *ctx, const spl_mat *a, const spl_mat *b, spl_mat **out)
 
 int spl_mat_neg(spl_ctx *ctx, const spl_mat *a, spl_mat **out) {
     API_BEGIN(ctx)
-    require_narrow(a, "spl_mat_neg");
-    MatUse use_a(ctx, a);
     SPL_REQUIRE(a && out, SPL_ERR_ARG, "NULL handle");
     *out = nullptr;
+    require_narrow(a, "spl_mat_neg");
+    MatUse use_a(ctx, a);
     spl_mat *m = new_mat(ctx, a->format, a->dtype, a->nrows, a->ncols, a->nnz);
     try {
         SPL_CUDA(cudaMemcpyAsync(m->ptr, a->ptr, ((size_t)a->nmajor() + 1) * 4,

@@ -7,6 +7,7 @@
 #include <atomic>
 #include <cstdint>
 #include <cstdio>
+#include <cstdlib>
 #include <mutex>
 #include <string>
 #include <type_traits>
@@ -41,6 +42,16 @@ constexpr int kNumSmFallback = 148;
 constexpr uint64_t kMaxEntries = (1ull << 32) - 65536;
 // longest row whose column offsets the SpMV plan keeps as the matrix's row pattern (spl_mat::pattern_off)
 constexpr uint32_t kPatternMax = 64;
+
+// A test-only setting from the environment: true and *v when `name` holds a decimal number and nothing else;
+// false when it is unset, empty or anything else, so that a typo leaves the library's default in place.
+inline bool env_u64(const char *name, unsigned long long *v) {
+    const char *s = std::getenv(name);
+    if (!s || *s < '0' || *s > '9') return false;
+    char *end = nullptr;
+    *v = std::strtoull(s, &end, 10);        // ULLONG_MAX on overflow: clamped by the callers
+    return *end == '\0';
+}
 
 }  // namespace spl
 

@@ -125,6 +125,8 @@ void fill_ptr(spl_ctx *ctx, const uint32_t *sorted_major, uint32_t nnz, uint32_t
 spl_mat *new_mat(spl_ctx *ctx, int format, int dtype, uint32_t nrows, uint32_t ncols, uint32_t nnz);
 
 // wide.cu — matrices with 2^32 - 65536 stored entries or more (64-bit positions, spl_mat::ptr64)
+// Entry count from which a new matrix is stored wide: 2^32 - 65536, or SPL_WIDE_MIN_NNZ when that is set.
+uint64_t wide_min_nnz();
 spl_mat *new_wide_mat(spl_ctx *ctx, int format, int dtype, uint32_t nrows, uint32_t ncols, uint64_t nnz);
 int wide_validate(spl_ctx *ctx, const spl_mat *m);      // 0, or the failing assertion of CsrMatrix::new (7, 8, 9)
 void wide_spmv(spl_ctx *ctx, const spl_mat *a, const void *x, void *y);

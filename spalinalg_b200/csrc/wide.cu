@@ -348,6 +348,14 @@ wide_entry_range_kernel(const uint64_t *__restrict__ ptr, const uint32_t *__rest
 
 }  // namespace
 
+// SPL_WIDE_MIN_NNZ=<n>: matrices with n stored entries or more are created wide (tests of the wide kernels at
+// small sizes), n clamped to [1, 2^32 - 65536]; 2^32 - 65536 when unset or not a number.
+uint64_t wide_min_nnz() {
+    unsigned long long v = 0;
+    if (!env_u64("SPL_WIDE_MIN_NNZ", &v)) return kMaxEntries;
+    return v < 1 ? 1 : (v >= kMaxEntries ? kMaxEntries : (uint64_t)v);
+}
+
 spl_mat *new_wide_mat(spl_ctx *ctx, int format, int dtype, uint32_t nrows, uint32_t ncols, uint64_t nnz) {
     spl_mat *m = new spl_mat();
     m->format = format;

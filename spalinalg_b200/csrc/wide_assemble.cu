@@ -23,7 +23,6 @@
 // buckets run is the input + one bucket's scratch (compacted triplets, the sort's two key/value pairs,
 // its part) + the parts so far; at the stitch it is the input + all parts + the output.
 #include <algorithm>
-#include <cstdlib>
 #include <vector>
 
 #include "kernels.cuh"
@@ -270,7 +269,7 @@ spl_mat *assemble_bucketed(spl_ctx *ctx, int format, int dtype, uint32_t nrows, 
         h_ptr[b] = parts.m[b]->ptr;
     }
     const uint64_t total = h_off[nb];
-    spl_mat *out = total >= kMaxEntries ? new_wide_mat(ctx, format, dtype, nrows, ncols, total)
+    spl_mat *out = total >= wide_min_nnz() ? new_wide_mat(ctx, format, dtype, nrows, ncols, total)
                                         : new_mat(ctx, format, dtype, nrows, ncols, (uint32_t)total);
     try {
         {
@@ -308,11 +307,10 @@ spl_mat *assemble_bucketed(spl_ctx *ctx, int format, int dtype, uint32_t nrows, 
 }
 
 // SPL_ASSEMBLE_BUCKET_MAX=<triplets>: lists longer than that take the bucketed route with buckets of at
-// most that many triplets (tests of the route at small sizes); 0 when unset.
+// most that many triplets (tests of the route at small sizes); 0 when unset or not a number.
 uint64_t bucket_knob() {
-    const char *knob = std::getenv("SPL_ASSEMBLE_BUCKET_MAX");
-    if (!knob || !*knob) return 0;
-    const unsigned long long v = std::strtoull(knob, nullptr, 10);
+    unsigned long long v = 0;
+    if (!env_u64("SPL_ASSEMBLE_BUCKET_MAX", &v)) return 0;
     return v < 1 ? 1 : (v >= kMaxEntries ? kMaxEntries - 1 : (uint64_t)v);
 }
 
