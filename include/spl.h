@@ -352,6 +352,29 @@ int spl_spmv_footprint(spl_ctx *ctx, const spl_mat *a, uint64_t *col_min, uint64
  * place or copy it yourself).  Order it with spl_peer_barrier like spl_spmv_peer. */
 int spl_peer_pull(spl_ctx *ctx, int dtype, int world, int rank, const uint64_t *starts,
                   const void *const *slices, void *x_full_dev);
+/* The exchange of the row-sharded product `&A * &B` (impl Mul for &CsrMatrix, src/csr/ops/mul.rs:5-60;
+ * &CscMatrix, src/csc/ops/mul.rs:5-61).  A compressed matrix of nmajor x nminor (majors = rows for CSR,
+ * columns for CSC) is sharded by major: rank g owns majors [starts[g], starts[g+1]) and its arrays are
+ * readable from this device (mapped with spl_peer_open, the own shard included): ptr_slices[g] = uint32
+ * pointers of its majors (local positions, rows_g + 1 of them), ind_slices[g] = uint32 GLOBAL minor indices,
+ * val_slices[g] = values, shard_nnz[g] entries each.  *out becomes a new ordinary (never wide) matrix of the
+ * same format with nmajor majors and nminor minors (nmajor x nminor for CSR, nminor x nmajor for CSC), sized
+ * exactly, that holds every major named by one of by's stored minor indices, copied bit for bit; every other
+ * major is empty.  So for CSR with by = A_local, spl_mat_mul(A_local, out) gives this rank's rows of A*B, and for CSC
+ * with by = B_local, spl_mat_mul(out, B_local) gives its columns of A*B, bit-identical to the unsharded
+ * product.  The call waits on nobody: bracket it with spl_peer_barrier (before: the peers' arrays are
+ * written; after: nobody overwrites or frees them while they are read).  Long runs of consecutive majors of
+ * one owner travel as TMA bulk copies, short ones as plain loads.  One host synchronisation.
+ * Errors (*out NULL, nothing written): SPL_ERR_SHAPE when by's minor dimension or starts[world] is not
+ * nmajor; SPL_ERR_ARG for world outside 1..8 or rank outside it, starts not rising from 0, a NULL slice of a
+ * rank that owns majors, by of another format or scalar type, or a shard whose pointers (as read on the
+ * device) descend or point past shard_nnz[g]; SPL_ERR_UNSUPPORTED for a wide by, a shard or a gathered total
+ * of 2^32 - 65536 entries or more. */
+int spl_peer_gather_rows(spl_ctx *ctx, int format, int dtype, uint64_t nmajor, uint64_t nminor, int world, int rank,
+                         const uint64_t *starts, const uint64_t *shard_nnz, const void *const *ptr_slices,
+                         const void *const *ind_slices, const void *const *val_slices, const spl_mat *by,
+                         spl_mat **out);
+
 /* Row-sharded y_local = A_local * x with x left where it lives: x_slices[g] is rank
  * g's slice of x (columns [col_starts[g], col_starts[g+1]), own slice included), mapped
  * with spl_peer_open.  One kernel: every gather goes to the slice that owns the column,

@@ -101,6 +101,10 @@ extern "C" {
     pub fn spl_peer_barrier_status(ctx: *mut spl_ctx, timed_out: *mut c_int) -> c_int;
     pub fn spl_peer_pull(ctx: *mut spl_ctx, dtype: c_int, world: c_int, rank: c_int, starts: *const u64,
         slices: *const *const c_void, x_full_dev: *mut c_void) -> c_int;
+    pub fn spl_peer_gather_rows(ctx: *mut spl_ctx, format: c_int, dtype: c_int, nmajor: u64, nminor: u64, world: c_int,
+        rank: c_int, starts: *const u64, shard_nnz: *const u64, ptr_slices: *const *const c_void,
+        ind_slices: *const *const c_void, val_slices: *const *const c_void, by: *const spl_mat,
+        out: *mut *mut spl_mat) -> c_int;
     pub fn spl_spmv_peer(ctx: *mut spl_ctx, a_local: *const spl_mat, world: c_int, rank: c_int,
         col_starts: *const u64, x_slices: *const *const c_void, y_dev: *mut c_void) -> c_int;
     pub fn spl_peer_barrier_halo(ctx: *mut spl_ctx, world: c_int, rank: c_int, flag_ptrs: *const *mut c_void,

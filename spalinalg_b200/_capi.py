@@ -74,6 +74,7 @@ SIGNATURES = {
     "spl_spmv_footprint": (_i, [_vp, _vp, C.POINTER(_u64), C.POINTER(_u64)]),
     "spl_peer_pull": (_i, [_vp, _i, _i, _i, _vp, _vp, _vp]),
     "spl_peer_barrier_status": (_i, [_vp, C.POINTER(_i)]),
+    "spl_peer_gather_rows": (_i, [_vp, _i, _i, _u64, _u64, _i, _i, _vp, _vp, _vp, _vp, _vp, _vp, _pp]),
     "spl_spmv_peer": (_i, [_vp, _vp, _i, _i, _vp, _vp, _vp]),
     "spl_spmv_gather_fused": (_i, [_vp, _i, _u64, _i, _i, _vp, _vp, _i, _vp, _vp, _u64, _vp, _vp, _vp, _vp, _vp, _vp, C.c_uint32, _u64, _vp,
                               C.c_uint32, C.c_uint32, _vp]),

@@ -911,6 +911,37 @@ int spl_peer_pull(spl_ctx *ctx, int dtype, int world, int rank, const uint64_t *
     API_END(ctx)
 }
 
+int spl_peer_gather_rows(spl_ctx *ctx, int format, int dtype, uint64_t nmajor, uint64_t nminor, int world, int rank,
+                         const uint64_t *starts, const uint64_t *shard_nnz, const void *const *ptr_slices,
+                         const void *const *ind_slices, const void *const *val_slices, const spl_mat *by,
+                         spl_mat **out) {
+    API_BEGIN(ctx)
+    SPL_REQUIRE(out, SPL_ERR_ARG, "out is NULL");
+    *out = nullptr;
+    SPL_REQUIRE(by && starts && shard_nnz && ptr_slices && ind_slices && val_slices, SPL_ERR_ARG, "NULL argument");
+    check_enums(format, dtype);
+    SPL_REQUIRE(world >= 1 && world <= SPL_MAX_PEERS && rank >= 0 && rank < world, SPL_ERR_ARG,
+                "world must be 1..8 and rank inside it");
+    require_narrow(by, "spl_peer_gather_rows");
+    SPL_REQUIRE(by->format == format && by->dtype == dtype, SPL_ERR_ARG,
+                "spl_peer_gather_rows: by must have the gathered matrix's format and scalar type");
+    SPL_REQUIRE(starts[0] == 0, SPL_ERR_ARG, "starts must begin at 0");
+    for (int g = 0; g < world; ++g) {
+        SPL_REQUIRE(starts[g] <= starts[g + 1], SPL_ERR_ARG, "starts must be non-decreasing");
+        SPL_REQUIRE(starts[g] == starts[g + 1] || (ptr_slices[g] && ind_slices[g] && val_slices[g]), SPL_ERR_ARG,
+                    "NULL slice of a rank that owns majors");
+        SPL_REQUIRE(shard_nnz[g] < kMaxEntries, SPL_ERR_UNSUPPORTED, "a shard holds 2^32 - 65536 entries or more");
+    }
+    SPL_REQUIRE(starts[world] == nmajor && by->nminor() == nmajor, SPL_ERR_SHAPE,
+                "spl_peer_gather_rows: starts[world] and by's minor dimension must equal nmajor");
+    SPL_REQUIRE(nminor > 0 && nminor < (1ull << 32), SPL_ERR_UNSUPPORTED, "nminor must be in 1 .. 2^32 - 1");
+    MatUse use_by(ctx, by);
+    *out = peer_gather_rows(ctx, format, dtype, (uint32_t)nmajor, (uint32_t)nminor, world, starts, shard_nnz,
+                            ptr_slices, ind_slices, val_slices, by);
+    publish_mat(ctx, *out);
+    API_END(ctx)
+}
+
 int spl_peer_barrier_status(spl_ctx *ctx, int *timed_out) {
     API_BEGIN(ctx)
     uint32_t w = 0;

@@ -96,6 +96,13 @@ void peer_pull(spl_ctx *ctx, int world, int rank, size_t vsize, const uint64_t *
 void peer_barrier_halo(spl_ctx *ctx, int world, int rank, void *const *flag_ptrs, uint32_t epoch, uint32_t timeout_ms,
                        size_t vsize, const uint64_t *starts, void *const *slices, uint32_t halo_left, uint32_t halo_right);
 
+// gather_rows.cu — the exchange of the row-sharded product: every major of a major-sharded matrix (slices of its
+// ranks' ptr / ind / val, peer memory) that one of by's minor indices names, copied into one new full-height matrix
+// (other majors empty).  Arguments checked by the caller, except the shards' pointers (checked on the device).
+spl_mat *peer_gather_rows(spl_ctx *ctx, int format, int dtype, uint32_t nmajor, uint32_t nminor, int world,
+                          const uint64_t *starts, const uint64_t *shard_nnz, const void *const *ptr_slices,
+                          const void *const *ind_slices, const void *const *val_slices, const spl_mat *by);
+
 // addsub.cu — C = A +/- B on compressed arrays of equal format (a-7)
 spl_mat *addsub(spl_ctx *ctx, const spl_mat *a, const spl_mat *b, int subtract);
 

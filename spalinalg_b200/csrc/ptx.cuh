@@ -63,6 +63,11 @@ __device__ __forceinline__ void tma_bulk_s2g(void *dst_gmem, const void *src_sme
                  "r"(smem_u32(src_smem)), "r"(bytes)
                  : "memory");
 }
+// orders this thread's generic-proxy accesses of shared memory before a later bulk copy into the same bytes (a stage
+// the CTA has finished reading is refilled)
+__device__ __forceinline__ void fence_proxy_async_smem() {
+    asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
+}
 __device__ __forceinline__ void bulk_commit() { asm volatile("cp.async.bulk.commit_group;" ::: "memory"); }
 __device__ __forceinline__ void bulk_wait_all() { asm volatile("cp.async.bulk.wait_group 0;" ::: "memory"); }
 __device__ __forceinline__ void bulk_wait_read_but_one() {

@@ -19,6 +19,14 @@ keeps GLOBAL column indices.  What moves between ranks, and how:
              with TMA bulk copies while it multiplies block by block (spl_spmv_gather_fused), or
              x is pulled / all-gathered first (spl_peer_pull, NCCL in sharding.py).
   add/sub/neg  no exchange when the operands share the partition.
+  mul        C = A * B with A, B row-sharded (B with any row partition): rank g's rows of C need exactly the rows
+             of B that its shard's stored columns name.  Every rank copies its shard of B into three peer buffers
+             (pointers, indices, values; sized by one all-gather of the shard sizes), one flag barrier, then
+             spl_peer_gather_rows copies the named rows from their owners over NVLink into one local matrix of
+             B's full height (other rows empty; runs of rows of one owner as TMA bulk copies), a second barrier,
+             and the unsharded product A_local * gathered (spl_mat_mul): bit for bit the rows of the whole
+             product.  Banded / stencil shards move a thin halo; random ones about all of B.  The CSC twin
+             (column-sharded) gathers the columns of A that B's shard names.
 
 torch.distributed is the plumbing (rendezvous, the all-to-all, object exchange of IPC handles);
 the device work goes through the C ABI.  The CPU tests (gloo, world size 2) drive the same host
@@ -280,6 +288,20 @@ class DistCsrMatrix:
     def __neg__(self):
         return DistCsrMatrix(-self.local, self.starts, self.rank, self._nrows, self._ncols)
 
+    def mul(self, rhs: "DistCsrMatrix", dist, torch, group=None) -> "DistCsrMatrix":
+        """Sharded `&A * &B` (impl Mul for &CsrMatrix, src/csr/ops/mul.rs:5-60): this rank's rows of A·B, with A's
+        row partition and rhs.ncols() columns; rhs may have any row partition.  The rows of B this shard needs are
+        gathered from their owners over peer memory (spl_peer_gather_rows), then multiplied locally: bit for bit the
+        rows of the unsharded product.  Collective."""
+        if self._ncols != rhs._nrows:
+            raise Panic("assertion `left == right` failed: self.ncols() == rhs.nrows()")
+        shard = _PeerShard(rhs, dist, torch, group)
+        try:
+            gathered = shard.gather(self.local)
+        finally:
+            shard.close()
+        return DistCsrMatrix(self.local * gathered, self.starts, self.rank, self._nrows, rhs._ncols)
+
     def nnz_global(self, dist, torch, group=None):
         t = torch.tensor([self.local.nnz()], dtype=torch.int64,
                          device="cuda" if torch.cuda.is_available() else "cpu")
@@ -462,6 +484,20 @@ class DistCscMatrix:
     def ncols(self): return self._ncols
     def local_cols(self): return self.starts[self.rank], self.starts[self.rank + 1]
 
+    def mul(self, rhs: "DistCscMatrix", dist, torch, group=None) -> "DistCscMatrix":
+        """Sharded `&A * &B` for column-sharded CSC operands (impl Mul for &CscMatrix, src/csc/ops/mul.rs:5-61):
+        this rank's columns of A·B, with rhs's column partition.  The columns of A (this matrix) that rhs's shard's
+        row indices name are gathered over peer memory, then gathered * rhs.local: bit for bit the columns of the
+        unsharded product.  Collective."""
+        if self._ncols != rhs._nrows:
+            raise Panic("assertion `left == right` failed: self.ncols() == rhs.nrows()")
+        shard = _PeerShard(self, dist, torch, group)
+        try:
+            gathered = shard.gather(rhs.local)
+        finally:
+            shard.close()
+        return DistCscMatrix(gathered * rhs.local, rhs.starts, rhs.rank, self._nrows, rhs._ncols)
+
     def spmv(self, dist, torch, x_local, group=None):
         """y = A x with A column-sharded (this rank holds columns [c0, c1) as a CscMatrix with global row
         indices) and x sharded like the columns: the sharded form of `&A * &X` for a CscMatrix
@@ -572,6 +608,67 @@ class PeerExchange:
             if b is not None:
                 b.close(self.dist, self.group)
         self._keys = self._vals = self._flags = None
+
+
+class _PeerShard:
+    """The sharded product's exchange: a major-sharded matrix (DistCsrMatrix by rows, DistCscMatrix by columns)
+    published in peer memory.  __init__ is collective: one all-gather of every rank's (pointers, entries) sizes
+    the three buffers (the largest shard) and gives the entry counts spl_peer_gather_rows checks the pointers
+    against; the own shard is copied in with plain device-to-device copies.  gather(by) brackets
+    spl_peer_gather_rows with the flag barrier: before (every shard is in place), after (nobody closes a buffer
+    a peer still reads).  Nothing is kept between products."""
+
+    def __init__(self, mat, dist, torch, group=None):
+        from .synthetic_device import device_view
+        L = mat.local
+        self.ctx, self.dist, self.group = L._ctx, dist, group
+        self.world, self.rank = mat.world, mat.rank
+        self.starts = list(mat.starts)
+        self.fmt, self.dtype = L._FORMAT, L.dtype
+        self.nmajor = mat._nrows if self.fmt == capi.SPL_CSR else mat._ncols
+        self.nminor = mat._ncols if self.fmt == capi.SPL_CSR else mat._nrows
+        nloc = self.starts[self.rank + 1] - self.starts[self.rank]      # 0: the local matrix is a phantom major
+        nnz = L.nnz() if nloc else 0
+        dev = "cuda" if torch.cuda.is_available() else "cpu"
+        mine = torch.tensor([nloc + 1, nnz], dtype=torch.int64, device=dev)
+        sizes = torch.empty(2 * self.world, dtype=torch.int64, device=dev)
+        dist.all_gather_into_tensor(sizes, mine, group=group)
+        sizes = sizes.view(self.world, 2).tolist()
+        self.shard_nnz = [int(e) for _, e in sizes]
+        most_p, most_e = max(p for p, _ in sizes), max(max(self.shard_nnz), 1)
+        item = np.dtype(self.dtype).itemsize
+        self.ex = PeerExchange(self.ctx, dist, group)                   # flag block of the barrier
+        self.bufs = [PeerBuffer(self.ctx, dist, n, group) for n in (4 * most_p, 4 * most_e, item * most_e)]
+        self.ctx.sync()                          # L's arrays are final on the context's stream; torch copies below
+        tdt = torch.float32 if self.dtype == np.float32 else torch.float64
+        p_ptr, p_ind, p_val = L.device_ptrs()
+        device_view(torch, self.bufs[0].local, nloc + 1, torch.int32).copy_(device_view(torch, p_ptr, nloc + 1, torch.int32))
+        if nnz:
+            device_view(torch, self.bufs[1].local, nnz, torch.int32).copy_(device_view(torch, p_ind, nnz, torch.int32))
+            device_view(torch, self.bufs[2].local, nnz, tdt).copy_(device_view(torch, p_val, nnz, tdt))
+        torch.cuda.current_stream().synchronize()
+
+    def gather(self, by):
+        """The majors named by `by`'s minor indices, as a new local matrix of the shard's format and full height."""
+        ctx, W = self.ctx, self.world
+        self.ex.barrier()
+        st = (C.c_uint64 * (W + 1))(*self.starts)
+        nz = (C.c_uint64 * W)(*self.shard_nnz)
+        sl = [(C.c_void_p * W)(*b.ptrs) for b in self.bufs]
+        h = C.c_void_p()
+        ctx.check(ctx._lib.spl_peer_gather_rows(
+            ctx._h, self.fmt, _dtype_code(self.dtype), self.nmajor, self.nminor, W, self.rank, C.cast(st, C.c_void_p),
+            C.cast(nz, C.c_void_p), C.cast(sl[0], C.c_void_p), C.cast(sl[1], C.c_void_p), C.cast(sl[2], C.c_void_p),
+            by._h, C.byref(h)))
+        self.ex.barrier()
+        return type(by)._wrap(ctx, h)
+
+    def close(self):
+        self.ctx.sync()
+        self.ex.check()                          # a barrier that gave up is reported, not a half-gathered result
+        for b in self.bufs:
+            b.close(self.dist, self.group)
+        self.ex.close()
 
 
 class PeerVector:
