@@ -346,12 +346,18 @@ struct MatUse {
 };
 
 // Rust's unary minus on floats is a sign-bit flip for every input, NaN included (the GPU's FNEG
-// path may canonicalise NaN), so negate on the integer view.
+// path may canonicalise NaN), so negate on the integer view.  The xor is inline PTX: written in C++
+// the compiler recognises bitcast-xor-bitcast as a float negation, and ptxas may then emit it as
+// FADD -x, -RZ, which returns the canonical NaN (it did in union_block_kernel's staged path).
 __device__ __forceinline__ float flip_sign(float v) {
-    return __uint_as_float(__float_as_uint(v) ^ 0x80000000u);
+    uint32_t u = __float_as_uint(v);
+    asm("xor.b32 %0, %0, 0x80000000;" : "+r"(u));
+    return __uint_as_float(u);
 }
 __device__ __forceinline__ double flip_sign(double v) {
-    return __longlong_as_double(__double_as_longlong(v) ^ (long long)0x8000000000000000ull);
+    unsigned long long u = (unsigned long long)__double_as_longlong(v);
+    asm("xor.b64 %0, %0, 0x8000000000000000;" : "+l"(u));
+    return __longlong_as_double((long long)u);
 }
 
 }  // namespace spl
