@@ -344,6 +344,34 @@ int spl_spmv_window(spl_ctx *ctx, const spl_mat *a, const void *x_window_dev, ui
                     uint64_t window_len, void *y_dev);
 /* Smallest and largest stored column of A (0, 0 for an empty matrix): sizes the halo. */
 int spl_spmv_footprint(spl_ctx *ctx, const spl_mat *a, uint64_t *col_min, uint64_t *col_max);
+/* The row-sharded transposed product y = A^T x: `&A * &X` on the transpose (CsrMatrix::transpose,
+ * src/csr.rs:358-406, then impl Mul for &CsrMatrix, src/csr/ops/mul.rs:5-60).  Rank g owns rows
+ * [rs_g, rs_{g+1}) of A as a CSR shard with global columns and x_g = x[rs_g .. rs_{g+1}); y (ncols values) ends
+ * up sharded by a column partition col_starts.  Two steps per product:
+ *
+ * spl_spmv_transpose_window: the local partial.  y_window_dev[j] = (A^T x)[col_min + j] for j in
+ * [0, col_max - col_min] with (col_min, col_max) = spl_spmv_footprint(a); x_dev has A's nrows values.  Runs on
+ * a CSR form of the transpose restricted to that window (col_max - col_min + 1 rows), built on the first call
+ * and kept with the matrix until its values change; then the planner's row kernels, so with one lane per row
+ * every value is summed over ascending rows of A, bit-identical to the reference.  A without stored entries
+ * writes nothing.  SPL_ERR_UNSUPPORTED for a wide or a CSC a, SPL_ERR_ARG for a NULL pointer; nothing written.
+ *
+ * spl_peer_reduce_windows: the exchange.  windows[2g], windows[2g+1] = rank g's window [first, last + 1)
+ * (empty when equal: a shard without entries); partials[g] = rank g's window buffer, mapped with spl_peer_open
+ * (the own one local; NULL allowed for an empty window).  For every column c of this rank's slice
+ * [col_starts[rank], col_starts[rank+1]), y_local_dev[c - col_starts[rank]] = the partials of the ranks whose
+ * window holds c folded in ascending rank, the first copied, the others added (+0.0 when no window holds c):
+ * deterministic whatever the ranks' timing.  flag_ptrs / epoch / timeout_ms as in spl_peer_barrier: the barrier
+ * runs first, in the same launch (every partial is written before any is read); on a timeout y holds NaN and
+ * spl_peer_barrier_status reports it.  flag_ptrs NULL skips it (order with spl_peer_barrier yourself).  Two
+ * partial buffers per rank alternated by product make one barrier per product enough (a buffer is rewritten
+ * two products after it was read, and every peer finished reading it before arriving at the barrier in between).
+ * SPL_ERR_ARG, nothing written: world outside 1..8 or rank outside it, col_starts not rising from 0, a window
+ * outside [0, col_starts[world]), a NULL partial of a non-empty window, a NULL flag block. */
+int spl_spmv_transpose_window(spl_ctx *ctx, const spl_mat *a, const void *x_dev, void *y_window_dev);
+int spl_peer_reduce_windows(spl_ctx *ctx, int dtype, int world, int rank, const uint64_t *col_starts,
+                            const uint64_t *windows, const void *const *partials, void *const *flag_ptrs,
+                            uint32_t epoch, uint32_t timeout_ms, void *y_local_dev);
 /* All-gather of x by pulling over peer memory, for general (random / power-law) shards whose
  * gathers would be 4-byte NVLink transactions: one kernel copies every peer's slice
  * (slices[g] = x[starts[g] .. starts[g+1]), mapped with spl_peer_open) into the local full-length

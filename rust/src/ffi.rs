@@ -113,6 +113,11 @@ extern "C" {
     pub fn spl_spmv_window(ctx: *mut spl_ctx, a: *const spl_mat, x_window_dev: *const c_void, window_start: u64,
         window_len: u64, y_dev: *mut c_void) -> c_int;
     pub fn spl_spmv_footprint(ctx: *mut spl_ctx, a: *const spl_mat, col_min: *mut u64, col_max: *mut u64) -> c_int;
+    pub fn spl_spmv_transpose_window(ctx: *mut spl_ctx, a: *const spl_mat, x_dev: *const c_void,
+        y_window_dev: *mut c_void) -> c_int;
+    pub fn spl_peer_reduce_windows(ctx: *mut spl_ctx, dtype: c_int, world: c_int, rank: c_int, col_starts: *const u64,
+        windows: *const u64, partials: *const *const c_void, flag_ptrs: *const *mut c_void, epoch: u32,
+        timeout_ms: u32, y_local_dev: *mut c_void) -> c_int;
     pub fn spl_spmv_gather_fused(ctx: *mut spl_ctx, dtype: c_int, nrows_local: u64, world: c_int, rank: c_int,
         col_starts: *const u64, x_slices: *const *const c_void, nblocks: c_int, block_first: *const u32,
         block_ptr: *const u32, block_ptr_stride: u64, tile_entries_max: *const u32, block_ind: *const u32,

@@ -72,6 +72,8 @@ SIGNATURES = {
     "spl_peer_barrier_halo": (_i, [_vp, _i, _i, _vp, C.c_uint32, C.c_uint32, _i, _vp, _vp, _u64, _u64]),
     "spl_spmv_window": (_i, [_vp, _vp, _vp, _u64, _u64, _vp]),
     "spl_spmv_footprint": (_i, [_vp, _vp, C.POINTER(_u64), C.POINTER(_u64)]),
+    "spl_spmv_transpose_window": (_i, [_vp, _vp, _vp, _vp]),
+    "spl_peer_reduce_windows": (_i, [_vp, _i, _i, _i, _vp, _vp, _vp, _vp, C.c_uint32, C.c_uint32, _vp]),
     "spl_peer_pull": (_i, [_vp, _i, _i, _i, _vp, _vp, _vp]),
     "spl_peer_barrier_status": (_i, [_vp, C.POINTER(_i)]),
     "spl_peer_gather_rows": (_i, [_vp, _i, _i, _u64, _u64, _i, _i, _vp, _vp, _vp, _vp, _vp, _vp, _pp]),

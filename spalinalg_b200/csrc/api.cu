@@ -902,6 +902,38 @@ int spl_spmv_footprint(spl_ctx *ctx, const spl_mat *a, uint64_t *col_min, uint64
     API_END(ctx)
 }
 
+int spl_spmv_transpose_window(spl_ctx *ctx, const spl_mat *a, const void *x_dev, void *y_window_dev) {
+    API_BEGIN(ctx)
+    require_narrow(a, "spl_spmv_transpose_window");
+    MatUse use_a(ctx, a);
+    SPL_REQUIRE(a && x_dev && y_window_dev, SPL_ERR_ARG, "NULL argument");
+    spmv_transpose_window(ctx, a, x_dev, y_window_dev);
+    API_END(ctx)
+}
+
+int spl_peer_reduce_windows(spl_ctx *ctx, int dtype, int world, int rank, const uint64_t *col_starts,
+                            const uint64_t *windows, const void *const *partials, void *const *flag_ptrs, uint32_t epoch,
+                            uint32_t timeout_ms, void *y_local_dev) {
+    API_BEGIN(ctx)
+    check_enums(SPL_CSR, dtype);
+    SPL_REQUIRE(col_starts && windows && partials, SPL_ERR_ARG, "NULL argument");
+    SPL_REQUIRE(world >= 1 && world <= SPL_MAX_PEERS && rank >= 0 && rank < world, SPL_ERR_ARG,
+                "world must be 1..8 and rank inside it");
+    SPL_REQUIRE(col_starts[0] == 0, SPL_ERR_ARG, "col_starts must begin at 0");
+    for (int g = 0; g < world; ++g) {
+        SPL_REQUIRE(col_starts[g] <= col_starts[g + 1], SPL_ERR_ARG, "col_starts must be non-decreasing");
+        SPL_REQUIRE(!flag_ptrs || flag_ptrs[g], SPL_ERR_ARG, "NULL flag block");
+    }
+    for (int g = 0; g < world; ++g) {
+        SPL_REQUIRE(windows[2 * g] <= windows[2 * g + 1] && windows[2 * g + 1] <= col_starts[world], SPL_ERR_ARG,
+                    "a window lies outside the columns [0, col_starts[world])");
+        SPL_REQUIRE(partials[g] || windows[2 * g] == windows[2 * g + 1], SPL_ERR_ARG, "NULL partial of a non-empty window");
+    }
+    SPL_REQUIRE(y_local_dev || col_starts[rank] == col_starts[rank + 1], SPL_ERR_ARG, "NULL y");
+    peer_reduce_windows(ctx, dtype, world, rank, col_starts, windows, partials, flag_ptrs, epoch, timeout_ms, y_local_dev);
+    API_END(ctx)
+}
+
 int spl_peer_pull(spl_ctx *ctx, int dtype, int world, int rank, const uint64_t *starts,
                   const void *const *slices, void *x_full_dev) {
     API_BEGIN(ctx)

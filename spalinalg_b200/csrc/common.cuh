@@ -154,6 +154,10 @@ struct spl_mat {
     // and kept: products on a CscMatrix then run the row kernels at full speed and in the reference's
     // summation order.  Owned by this matrix; dropped when the values change.
     std::atomic<spl_mat *> twin{nullptr};
+    // CSR form of the transpose of this CSR matrix restricted to its column footprint: row j is column
+    // col_min + j (col_max - col_min + 1 rows), its columns are this matrix's rows.  Built by the first
+    // spl_spmv_transpose_window and kept (same rules as twin); dropped when the values change.
+    std::atomic<spl_mat *> window_t{nullptr};
     // Sharing across contexts (spl.h: a matrix may be used read-only by several host threads, each
     // with its own context and stream).  `home` is the stream the matrix was created on and `ready`
     // the event recorded there behind the last kernel that wrote it: a context on another stream

@@ -58,6 +58,9 @@ void spmv(spl_ctx *ctx, const spl_mat *a, const void *x, void *y, int kernel, in
 // y = A x where x_window holds only the columns [start, start + len) of x (the matrix's column footprint
 // must lie inside): the product of a row shard next to its halo
 void spmv_window(spl_ctx *ctx, const spl_mat *a, const void *x_window, uint64_t start, uint64_t len, void *y);
+// y_window = rows [col_min, col_max] of A^T x for a CSR matrix (its column footprint), through the cached CSR form
+// of the transpose restricted to the footprint (spl_mat::window_t); an empty matrix writes nothing
+void spmv_transpose_window(spl_ctx *ctx, const spl_mat *a, const void *x, void *y_window);
 // `&A * &x` with host vectors, pipelined: x goes up in prefixes, row chunks run as soon as the prefix
 // they need is there, their part of y goes down while the next chunk runs (PCIe both ways at once).
 // x_dev / y_dev are device buffers of ncols / nrows values.  Returns false (nothing done) when the
@@ -95,6 +98,11 @@ void peer_pull(spl_ctx *ctx, int world, int rank, size_t vsize, const uint64_t *
 // slice are copied from their owners' slices into the padding around slices[rank] (one small kernel)
 void peer_barrier_halo(spl_ctx *ctx, int world, int rank, void *const *flag_ptrs, uint32_t epoch, uint32_t timeout_ms,
                        size_t vsize, const uint64_t *starts, void *const *slices, uint32_t halo_left, uint32_t halo_right);
+// the barrier (when flag_ptrs is given), then y_local[c - col_starts[rank]] = the ranks' window partials of column c
+// folded in ascending rank (windows[2g] .. windows[2g+1] is rank g's window, partials[g] its buffer); arguments checked
+void peer_reduce_windows(spl_ctx *ctx, int dtype, int world, int rank, const uint64_t *col_starts,
+                         const uint64_t *windows, const void *const *partials, void *const *flag_ptrs, uint32_t epoch,
+                         uint32_t timeout_ms, void *y_local);
 
 // gather_rows.cu — the exchange of the row-sharded product: every major of a major-sharded matrix (slices of its
 // ranks' ptr / ind / val, peer memory) that one of by's minor indices names, copied into one new full-height matrix

@@ -225,6 +225,7 @@ void free_mat(spl_ctx *ctx, spl_mat *m) {
     if (m->ready) cudaEventDestroy(m->ready);
     m->ready = nullptr;
     free_mat(ctx, m->twin.exchange(nullptr));
+    free_mat(ctx, m->window_t.exchange(nullptr));
     dfree(ctx, m->ptr);
     dfree(ctx, m->ptr64);
     dfree(ctx, m->ind);

@@ -171,7 +171,99 @@ __global__ void __launch_bounds__(PULL_THREADS) peer_pull_kernel(PullSlices ps, 
     bulk_wait_all();
 }
 
+// The exchange of the row-sharded transposed product y = A^T x.  Rank g's partial A_g^T x_g covers its footprint
+// window [lo_g, hi_g) (spl_spmv_transpose_window) and stays in g's memory; each rank then reads, for every column
+// of its own slice of y, the partials of the ranks whose window holds it and folds them in ascending rank: the
+// first one copied (a lone -0.0 stays -0.0), the others added; a column no window holds is +0.0.  So y does not
+// depend on the ranks' timing.  A banded shard reads its own partial plus two thin halo pieces; a random one the
+// world - 1 peers' pieces of its slice.  Every thread keeps RW_COLS columns in flight (coalesced across the warp,
+// L2-coherent loads: the peers' partials are read over NVLink).  With flag blocks the flag barrier comes first,
+// in every CTA (the arrival stores the same epoch, so repeating it is harmless, and no CTA depends on another
+// being resident); a CTA whose wait timed out, or that finds the timeout flag set, writes NaN.
+struct ReduceWindows {
+    const unsigned char *part[SPL_MAX_PEERS];
+    unsigned long long lo[SPL_MAX_PEERS], hi[SPL_MAX_PEERS];
+    unsigned long long my0, n;
+    int world;
+};
+
+constexpr int RW_COLS = 4;
+constexpr int RW_THREADS = 256;
+
+template <typename T>
+__global__ void __launch_bounds__(RW_THREADS)
+peer_reduce_windows_kernel(FlagBlocks f, bool barrier, int rank, uint32_t epoch, uint64_t timeout_ns, uint32_t *timed_out,
+                           ReduceWindows w, T *__restrict__ y) {
+    __shared__ int s_failed;
+    bool poison = false;
+    if (barrier) {
+        if (threadIdx.x == 0) s_failed = 0;
+        __syncthreads();
+        const int g = threadIdx.x;
+        if (g < w.world && g != rank) {
+            flag_arrive(f.block[g], rank, epoch);
+            if (!flag_wait(f.block[rank] + g, epoch, timeout_ns, 200, timed_out)) s_failed = 1;
+        }
+        __syncthreads();
+        poison = s_failed || *reinterpret_cast<const volatile uint32_t *>(timed_out) != 0u;
+    }
+    const unsigned long long step = (unsigned long long)gridDim.x * RW_THREADS * RW_COLS;
+    for (unsigned long long i0 = (unsigned long long)blockIdx.x * RW_THREADS * RW_COLS + threadIdx.x; i0 < w.n; i0 += step) {
+        T acc[RW_COLS];
+        bool any[RW_COLS];
+#pragma unroll
+        for (int u = 0; u < RW_COLS; ++u) { acc[u] = (T)0; any[u] = false; }
+#pragma unroll
+        for (int g = 0; g < SPL_MAX_PEERS; ++g) {
+            if (g >= w.world) break;
+            const T *p = reinterpret_cast<const T *>(w.part[g]);
+            T v[RW_COLS];
+            bool in[RW_COLS];
+#pragma unroll
+            for (int u = 0; u < RW_COLS; ++u) {
+                const unsigned long long c = w.my0 + i0 + (unsigned long long)u * RW_THREADS;
+                in[u] = i0 + (unsigned long long)u * RW_THREADS < w.n && c >= w.lo[g] && c < w.hi[g];
+                if (in[u]) v[u] = __ldcg(p + (c - w.lo[g]));
+            }
+#pragma unroll
+            for (int u = 0; u < RW_COLS; ++u)
+                if (in[u]) { acc[u] = any[u] ? acc[u] + v[u] : v[u]; any[u] = true; }
+        }
+#pragma unroll
+        for (int u = 0; u < RW_COLS; ++u) {
+            const unsigned long long i = i0 + (unsigned long long)u * RW_THREADS;
+            if (i < w.n) y[i] = poison ? (T)NAN : acc[u];
+        }
+    }
+}
+
 }  // namespace
+
+void peer_reduce_windows(spl_ctx *ctx, int dtype, int world, int rank, const uint64_t *col_starts,
+                         const uint64_t *windows, const void *const *partials, void *const *flag_ptrs, uint32_t epoch,
+                         uint32_t timeout_ms, void *y_local) {
+    FlagBlocks f{};
+    ReduceWindows w{};
+    w.world = world;
+    w.my0 = col_starts[rank];
+    w.n = col_starts[rank + 1] - col_starts[rank];
+    for (int g = 0; g < world; ++g) {
+        w.part[g] = static_cast<const unsigned char *>(partials[g]);
+        w.lo[g] = windows[2 * g];
+        w.hi[g] = windows[2 * g + 1];
+        if (flag_ptrs) f.block[g] = static_cast<uint32_t *>(flag_ptrs[g]);
+    }
+    const bool barrier = flag_ptrs != nullptr && world > 1;
+    const unsigned grid = std::max(1u, std::min(div_up(w.n, (uint64_t)RW_THREADS * RW_COLS), (unsigned)ctx->num_sms * 4u));
+    const uint64_t timeout_ns = (uint64_t)(timeout_ms ? timeout_ms : 2000) * 1000000ull;
+    if (dtype == SPL_F32)
+        peer_reduce_windows_kernel<float><<<grid, RW_THREADS, 0, ctx->stream>>>(f, barrier, rank, epoch, timeout_ns,
+                                                                               ctx->d_scratch + 32, w, (float *)y_local);
+    else
+        peer_reduce_windows_kernel<double><<<grid, RW_THREADS, 0, ctx->stream>>>(f, barrier, rank, epoch, timeout_ns,
+                                                                                ctx->d_scratch + 32, w, (double *)y_local);
+    check_launch(ctx, "peer_reduce_windows");
+}
 
 void peer_pull(spl_ctx *ctx, int world, int rank, size_t vsize, const uint64_t *starts,
                const void *const *slices, void *x_full) {

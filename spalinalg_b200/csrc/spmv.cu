@@ -1389,6 +1389,7 @@ const spl_mat *csr_form(spl_ctx *ctx, const spl_mat *a) {
 void drop_value_copies(spl_ctx *ctx, spl_mat *m) {
     std::lock_guard<std::mutex> lock(m->plan_mu);
     free_mat(ctx, m->twin.exchange(nullptr));
+    free_mat(ctx, m->window_t.exchange(nullptr));
     dfree(ctx, m->slice_ptr); dfree(ctx, m->slice_ind); dfree(ctx, m->slice_val);
     m->slice_ptr = m->slice_ind = nullptr;
     m->slice_val = nullptr;
@@ -1643,6 +1644,50 @@ void spmv_window(spl_ctx *ctx, const spl_mat *a, const void *x_window, uint64_t 
                 "the matrix has stored columns outside the window of x");
     const unsigned char *base = static_cast<const unsigned char *>(x_window) - start * a->vsize();
     spmv(ctx, a, base, y, SPL_SPMV_AUTO, 0, (uint32_t)start, (uint32_t)(start + len));
+}
+
+// ------------------------------------------------------------------ transposed product over the footprint
+// y = A^T x of a row shard only has values in the shard's column footprint [col_min, col_max].  The transpose
+// restricted to it is a CSR matrix of col_max - col_min + 1 rows (pointer array sized by the window, not by
+// ncols), built once by rebasing the column indices to the window and re-compressing (recompress: stable, so
+// every row of the transpose keeps the shard's rows in ascending order), then multiplied by the planner's row
+// kernels like any matrix: with one lane per row, y[c] is summed over ascending rows, the reference's order.
+namespace {
+__global__ void rebase_kernel(const uint32_t *__restrict__ in, uint32_t n, uint32_t base, uint32_t *__restrict__ out) {
+    for (uint64_t i = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (uint64_t)gridDim.x * blockDim.x)
+        out[i] = in[i] - base;
+}
+
+// a: CSR, narrow, planned, nnz > 0
+const spl_mat *transpose_window_form(spl_ctx *ctx, const spl_mat *a) {
+    spl_mat *m = const_cast<spl_mat *>(a);
+    if (spl_mat *t = m->window_t.load(std::memory_order_acquire)) return t;
+    std::lock_guard<std::mutex> lock(m->plan_mu);
+    if (spl_mat *t = m->window_t.load(std::memory_order_relaxed)) return t;
+    const uint32_t len = a->col_max - a->col_min + 1;
+    spl_mat *t = new_mat(ctx, SPL_CSR, a->dtype, len, a->nrows, a->nnz);
+    try {
+        Tmp<uint32_t> rebased(ctx, a->nnz);
+        rebase_kernel<<<std::min(div_up(a->nnz, 256), (unsigned)ctx->num_sms * 8u), 256, 0, ctx->stream>>>(
+            a->ind, a->nnz, a->col_min, rebased);
+        check_launch(ctx, "rebase");
+        recompress(ctx, a->dtype, a->nrows, len, a->nnz, a->ptr, rebased, a->val, t->ptr, t->ind, t->val);
+        publish_mat(ctx, t);
+        SPL_CUDA(cudaStreamSynchronize(ctx->stream));          // visible to any other stream from here on
+    } catch (...) {
+        free_mat(ctx, t);
+        throw;
+    }
+    m->window_t.store(t, std::memory_order_release);
+    return t;
+}
+}  // namespace
+
+void spmv_transpose_window(spl_ctx *ctx, const spl_mat *a, const void *x, void *y_window) {
+    SPL_REQUIRE(a->format == SPL_CSR, SPL_ERR_UNSUPPORTED, "spl_spmv_transpose_window needs a CSR matrix");
+    spmv_plan(ctx, const_cast<spl_mat *>(a));
+    if (a->nnz == 0) return;                                   // empty footprint: nothing to write
+    spmv(ctx, transpose_window_form(ctx, a), x, y_window, SPL_SPMV_AUTO, 0);
 }
 
 // The row-sharded `&A * &x` with HOST vectors (the reference-facing call on one rank of a sharded

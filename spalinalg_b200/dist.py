@@ -18,6 +18,11 @@ keeps GLOBAL column indices.  What moves between ranks, and how:
              (random / power-law) shards need the whole of x: ONE kernel pulls the peers' slices
              with TMA bulk copies while it multiplies block by block (spl_spmv_gather_fused), or
              x is pulled / all-gathered first (spl_peer_pull, NCCL in sharding.py).
+  A^T x      each rank multiplies x's slice by its shard's transpose over the shard's column footprint only
+             (spl_spmv_transpose_window) into one of two peer-visible partial buffers; one kernel then runs the
+             flag barrier and sums, for every column of the rank's slice of y, the partials of the ranks whose
+             footprint holds it, in ascending rank (spl_peer_reduce_windows): deterministic, and y lands in a
+             column partition of the caller's choice (x's own for a square matrix).
   add/sub/neg  no exchange when the operands share the partition.
   mul        C = A * B with A, B row-sharded (B with any row partition): rank g's rows of C need exactly the rows
              of B that its shard's stored columns name.  Every rank copies its shard of B into three peer buffers
@@ -384,6 +389,71 @@ class DistCsrMatrix:
         item = x.dtype.itemsize
         ctx.check(ctx._lib.spl_spmv_window(ctx._h, self.local._h, C.c_void_p(x.published_ptr - (r0 - w0) * item),
                                            w0, w1 - w0, C.c_void_p(y_dev)))
+
+    def prepare_transpose(self, dist, torch, col_starts: Optional[Sequence[int]] = None, group=None):
+        """One-time set-up of spmv_transpose (collective).  Every rank's footprint window [col_min, col_max + 1)
+        (spl_spmv_footprint; empty for a shard without entries) travels in one all-gather; two PeerBuffers of the
+        longest window hold the partials and a flag block carries the barrier.  col_starts is the column partition
+        y is left in: default partition_starts(ncols, world), which is `starts` for a square matrix, so that y can
+        be written straight into a PeerVector of x's partition."""
+        ctx = self.local._ctx
+        world = self.world
+        cs = list(col_starts) if col_starts is not None else partition_starts(self._ncols, world)
+        if len(cs) != world + 1 or cs[0] != 0 or cs[-1] != self._ncols or any(a > b for a, b in zip(cs, cs[1:])):
+            raise ValueError("col_starts must rise from 0 to ncols in world + 1 steps")
+        lo, hi = C.c_uint64(), C.c_uint64()
+        ctx.check(ctx._lib.spl_spmv_footprint(ctx._h, self.local._h, C.byref(lo), C.byref(hi)))
+        r0, r1 = self.local_rows()
+        mine = [lo.value, hi.value + 1] if r1 > r0 and self.local.nnz() else [0, 0]
+        dev = "cuda" if torch.cuda.is_available() else "cpu"
+        allw = torch.empty(2 * world, dtype=torch.int64, device=dev)
+        dist.all_gather_into_tensor(allw, torch.tensor(mine, dtype=torch.int64, device=dev), group=group)
+        windows = [int(v) for v in allw.tolist()]
+        longest = max(windows[2 * g + 1] - windows[2 * g] for g in range(world))
+        item = np.dtype(self.local.dtype).itemsize
+        self._transpose = {"col_starts": cs, "windows": windows, "epoch": 0,
+                           "parts": [PeerBuffer(ctx, dist, max(longest, 1) * item, group) for _ in range(2)],
+                           "flags": PeerBuffer(ctx, dist, 4 * capi.SPL_MAX_PEERS, group)}
+        dist.barrier(group=group)              # every flag block exists (and is zero) before first use
+
+    def spmv_transpose(self, x_local_dev: int, y_local_dev: int, timeout_ms: int = 2000):
+        """y = A^T x, sharded: x_local_dev holds this rank's rows' slice of x, y_local_dev receives the columns
+        [col_starts[rank], col_starts[rank+1]) of y (e.g. a PeerVector's local_ptr).  Two launches on the context's
+        stream, no host synchronisation: this rank's partial A_local^T x_local over its footprint window
+        (spl_spmv_transpose_window), then the barrier and the sum of the ranks' partials of the own columns in
+        ascending rank (spl_peer_reduce_windows).  Call prepare_transpose once first; check() reports a barrier
+        that timed out (y then holds NaN).
+        Product t writes partial buffer t % 2.  That buffer was last read by the peers' reduces of product t - 2,
+        which every peer finished before it arrived at barrier t - 1 (stream order), and this rank passed barrier
+        t - 1 before it got here: so one barrier per product is enough, as for PeerVector."""
+        T = self._transpose
+        ctx, world = self.local._ctx, self.world
+        T["epoch"] += 1
+        part = T["parts"][T["epoch"] % 2]
+        ctx.check(ctx._lib.spl_spmv_transpose_window(ctx._h, self.local._h, C.c_void_p(x_local_dev),
+                                                     C.c_void_p(part.local)))
+        cs = (C.c_uint64 * (world + 1))(*T["col_starts"])
+        win = (C.c_uint64 * (2 * world))(*T["windows"])
+        pp = (C.c_void_p * world)(*part.ptrs)
+        fl = (C.c_void_p * world)(*T["flags"].ptrs)
+        ctx.check(ctx._lib.spl_peer_reduce_windows(
+            ctx._h, _dtype_code(self.local.dtype), world, self.rank, C.cast(cs, C.c_void_p), C.cast(win, C.c_void_p),
+            C.cast(pp, C.c_void_p), C.cast(fl, C.c_void_p), T["epoch"], int(timeout_ms), C.c_void_p(y_local_dev)))
+
+    def check(self):
+        """Raises if a device barrier of this rank's context timed out (synchronises the stream)."""
+        t = C.c_int()
+        self.local._ctx.check(self.local._ctx._lib.spl_peer_barrier_status(self.local._ctx._h, C.byref(t)))
+
+    def close_transpose(self, dist=None, group=None):
+        """Frees what prepare_transpose set up (collective when dist is given)."""
+        T = getattr(self, "_transpose", None)
+        if T is None:
+            return
+        self.local._ctx.sync()
+        for b in T["parts"] + [T["flags"]]:
+            b.close(dist, group)
+        self._transpose = None
 
     @staticmethod
     def gather_groups(world: int):
@@ -789,6 +859,27 @@ def route_numpy(nrows: int, ncols: int, row, col, val, starts):
     keys = ((row - base) << np.uint64(bits_for(ncols))) | col
     counts = np.bincount(owner, minlength=len(starts) - 1).tolist()
     return keys[order].astype(np.uint64), np.asarray(val)[order], counts
+
+
+def reduce_windows_numpy(col_starts, windows, partials, rank: int, dtype):
+    """What spl_peer_reduce_windows writes on `rank`, in numpy: for every column c of the rank's slice, the partials
+    of the ranks whose window [windows[2g], windows[2g+1]) holds c, folded in ascending rank (the first copied, the
+    others added in `dtype`), +0.0 where no window holds c.  partials[g][j] is rank g's value of column
+    windows[2g] + j."""
+    c0, c1 = int(col_starts[rank]), int(col_starts[rank + 1])
+    y = np.zeros(c1 - c0, dtype)
+    have = np.zeros(c1 - c0, bool)
+    for g in range(len(col_starts) - 1):
+        lo, hi = int(windows[2 * g]), int(windows[2 * g + 1])
+        a, b = max(lo, c0), min(hi, c1)
+        if a >= b:
+            continue
+        seg = np.asarray(partials[g], dtype)[a - lo:b - lo]
+        s = slice(a - c0, b - c0)
+        with np.errstate(invalid="ignore", over="ignore"):
+            y[s] = np.where(have[s], y[s] + seg, seg)
+        have[s] = True
+    return y
 
 
 def unpack_keys(keys, ncols: int):
