@@ -144,9 +144,10 @@ struct spl_mat {
     // such r (a shard's local matrix: local rows, global columns, offsets shifted by its first row).  A stream
     // tile is regular when each of its rows r has K entries at columns r + pattern_off[j]: the stream kernel
     // then fetches its values only.  stream_tile_reg[slot] = 1 for a regular tile (layout of stream_tile_lo),
-    // stream_regular = how many tiles of the grid are regular.
+    // stream_regular = how many tiles of the grid are regular.  pattern_breaks = how many rows do not follow the
+    // pattern (plan): with few of them the band kernel takes the matrix (spmv.cu, band_eligible).
     uint32_t pattern_off[spl::kPatternMax] = {};
-    uint32_t pattern_len = 0;
+    uint32_t pattern_len = 0, pattern_breaks = 0;
     uint32_t *stream_tile_reg = nullptr;
     uint32_t stream_regular = 0;
 

@@ -451,6 +451,9 @@ void spmv_merge(spl_ctx *ctx, const spl_mat *a, const T *x, T *y) {
 //     the reference's `&A * &X` (src/csr/ops/mul.rs:25-40).
 // The tile layout and the consumers' row loop are those of stream_tile.cuh (shared with the fused
 // gather kernel, gather.cu); the copy and barrier primitives are those of ptx.cuh.
+// Bands do not run this kernel: a matrix with a row pattern at most kBandWidthMax columns wide and at most one row
+// off it per 64 tiles, with x as one local array, runs spmv_band_kernel (below), whose stages hold a regular tile's
+// values and x window only.
 constexpr uint32_t kStreamXEdgeMax = 1u << 15;     // longest leading edge of x one tile prefetches (elements)
 
 // largest number of stored entries in any window of `rows` consecutive rows (bounds every tile)
@@ -496,6 +499,14 @@ struct RowPattern {
     uint32_t len;
 };
 
+// whether row r, stored at positions [lo, hi), has pat.len entries at columns r + pat.off[j]
+__device__ __forceinline__ bool row_follows(const uint32_t *__restrict__ ind, uint32_t lo, uint32_t hi, uint32_t r,
+                                            const RowPattern &pat) {
+    bool fits = hi - lo == pat.len;
+    for (uint32_t j = 0; fits && j < pat.len; ++j) fits = ind[lo + j] == r + pat.off[j];
+    return fits;
+}
+
 // Per CTA b, slots [b * (max_tiles + 1) ...]: tile_lo[k] = position of tile k's first stored entry
 // (k = number of tiles: the end of the range); xhi[k] = 1 + the largest column of tile k (rows are
 // column-sorted: the last entry of a row), 0 if the tile has no entry; xlo0[b] = the smallest column of
@@ -517,11 +528,7 @@ __global__ void stream_edges_kernel(const uint32_t *__restrict__ ptr, const uint
     for (uint32_t r = rs + threadIdx.x; r < re; r += blockDim.x) {
         const uint32_t lo = ptr[r], hi = ptr[r + 1];
         const uint32_t k = (r - rs) / rows_per_tile;
-        if (pat.len) {                                  // reg[] holds "irregular" until the pass below
-            bool fits = hi - lo == pat.len;
-            for (uint32_t j = 0; fits && j < pat.len; ++j) fits = ind[lo + j] == r + pat.off[j];
-            if (!fits) reg[base + k] = 1u;
-        }
+        if (pat.len && !row_follows(ind, lo, hi, r, pat)) reg[base + k] = 1u;   // "irregular" until the pass below
         if (hi == lo) continue;
         atomicMax(xhi + base + k, ind[hi - 1] + 1u);
         if (k == 0) atomicMin(xlo0 + b, ind[lo]);
@@ -745,6 +752,23 @@ uint32_t stream_resident(K k, size_t smem, std::atomic<size_t> &smem_set, std::a
     return (uint32_t)(oc & 0xff);
 }
 
+// The dynamic shared memory, at least `smem`, with which no more than `ctas` CTAs fit on an SM.  Under programmatic
+// dependent launch the next product's CTAs would otherwise take a spare slot early, which was measured slower (C1,
+// one L2-resident copy: 12.7 against 11.0 us per product, profiles/r3_spmv_notes.md).
+size_t smem_for_ctas(size_t smem, uint32_t ctas) {
+    static const size_t sm_bytes = [] {
+        int dev = 0, per_sm = 0, reserved = 0;
+        cudaGetDevice(&dev);
+        cudaDeviceGetAttribute(&per_sm, cudaDevAttrMaxSharedMemoryPerMultiprocessor, dev);
+        cudaDeviceGetAttribute(&reserved, cudaDevAttrReservedSharedMemoryPerBlock, dev);
+        return ((size_t)per_sm << 16) | (size_t)reserved;
+    }();
+    const size_t per_sm = sm_bytes >> 16, reserved = sm_bytes & 0xffff;
+    const size_t one_more = per_sm / (ctas + 1) + 1;            // ctas + 1 CTAs of this size do not fit
+    if (one_more > reserved) return std::max(smem, std::min<size_t>(one_more - reserved, 227 * 1024));
+    return smem;
+}
+
 // x_edge: array indexable by column over [x_lo, x_hi) in local memory (the whole x, or this rank's own
 // slice of a sharded x with the pointer moved back by the slice's first column), or NULL
 template <typename T, int LPR, int U, bool TIGHT, typename XG>
@@ -776,16 +800,7 @@ void launch_stream(spl_ctx *ctx, const spl_mat *a, const XG &xg, T *y, const T *
     bool pat = a->stream_regular && env_int("SPL_STREAM_PATTERN", 1) != 0;
     size_t smem_pat_run = smem_pat;
     if (pat) {
-        static const size_t sm_bytes = [] {
-            int dev = 0, per_sm = 0, reserved = 0;
-            cudaGetDevice(&dev);
-            cudaDeviceGetAttribute(&per_sm, cudaDevAttrMaxSharedMemoryPerMultiprocessor, dev);
-            cudaDeviceGetAttribute(&reserved, cudaDevAttrReservedSharedMemoryPerBlock, dev);
-            return ((size_t)per_sm << 16) | (size_t)reserved;
-        }();
-        const size_t per_sm = sm_bytes >> 16, reserved = sm_bytes & 0xffff;
-        const size_t one_more = per_sm / (ctas + 1) + 1;            // ctas + 1 CTAs of this size do not fit
-        if (one_more > reserved) smem_pat_run = std::max(smem_pat, std::min<size_t>(one_more - reserved, 227 * 1024));
+        smem_pat_run = smem_for_ctas(smem_pat, ctas);
         pat = smem_pat_run <= 227 * 1024 && stream_resident(k_pat, smem_pat_run, smem_set_pat, occ_pat) >= ctas;
     }
     cudaLaunchConfig_t cfg{};
@@ -831,6 +846,213 @@ void spmv_stream(spl_ctx *ctx, const spl_mat *a, const XG &xg, T *y, const T *x_
         case 8: spmv_stream_u<T, 8>(ctx, a, xg, y, x_edge, x_lo, x_hi); break;
         case 16: spmv_stream_u<T, 16>(ctx, a, xg, y, x_edge, x_lo, x_hi); break;
         default: spmv_stream_u<T, 32>(ctx, a, xg, y, x_edge, x_lo, x_hi); break;
+    }
+}
+
+// ------------------------------------------------------------------ band kernel
+// The stream kernel for matrices whose rows, all but a few, follow the row pattern (bands; band_eligible).  A regular
+// tile of rows [r0, r1) needs its values and the x window [r0 + pat.off[0], r1 - 1 + pat.off[K-1] + 1) and nothing
+// else, so a stage holds just those two: the producer copies both into shared memory and the consumers never wait on
+// global memory (in the stream kernel they gather x with __ldg while they hold the stage).  The stages are sized for
+// a regular tile, not for the CSR slices of the stream kernel, so more CTAs and stages fit on an SM.  Irregular tiles
+// take no stage: their consumers run the same row loop over the global CSR arrays and x, and the producer skips them
+// (both read tile_reg[k]).  The row loop is tile_row_sum / row_lanes_sum: y has the bits of the vector kernel.
+//   * x may be the output of the launch before this one (x_{t+1} = A x_t under programmatic dependent launch): the
+//     producer reads no x byte before griddepcontrol.wait; before it, it only prefetches the first values into L2.
+//   * the x copy stays inside the caller's [x_lo, x_hi) (spmv_window passes a buffer that need not be 16-byte
+//     aligned and may end at the footprint): lane 0 bulk-copies the 16-byte aligned inside of the window, lanes 1
+//     and 2 load its ragged head and tail (under 16 bytes each) with plain loads, store them and arrive on the
+//     stage's full barrier.
+constexpr uint32_t kBandWidthMax = 4096;     // widest row pattern (last column - first column) the band kernel takes
+
+// The x window of the regular tile of rows [r0, r1): columns [*a, *b), clamped to [x_lo, x_hi); its stage area starts
+// at the 16-byte boundary at or below x + *a, which is column *xb.
+template <typename T>
+__device__ __forceinline__ void band_window(const T *x, uint32_t r0, uint32_t r1, uint32_t off0, uint32_t off_last,
+                                            uint32_t x_lo, uint32_t x_hi, uint32_t *a, uint32_t *b, uint32_t *xb) {
+    const uint32_t c0 = r0 + off0, c1 = r1 - 1u + off_last + 1u;    // mod 2^32: a shard's columns are global
+    *a = c0 > x_lo ? c0 : x_lo;
+    *b = c1 < x_hi ? c1 : x_hi;
+    *xb = *a - (uint32_t)((reinterpret_cast<uintptr_t>(x + *a) & 15u) / sizeof(T));
+}
+
+template <typename T, int LPR, int U>
+__global__ void __launch_bounds__(TILE_CONSUMERS + 32, 3)
+spmv_band_kernel(const uint32_t *__restrict__ ptr, const uint32_t *__restrict__ ind, const T *__restrict__ val,
+                 const T *__restrict__ x, T *__restrict__ y, const uint32_t *__restrict__ cta_rows,
+                 const uint32_t *__restrict__ tile_lo, const uint32_t *__restrict__ tile_reg, uint32_t max_tiles,
+                 uint32_t val_cap, uint32_t x_cap, uint32_t stages, uint32_t x_lo, uint32_t x_hi, int l2_hint,
+                 const __grid_constant__ RowPattern pat) {
+    constexpr uint32_t CONS = TILE_CONSUMERS;
+    constexpr uint32_t R = tile_rows(LPR);
+    extern __shared__ __align__(128) unsigned char st_raw[];
+    // per stage: [val_cap] values, then [x_cap] elements of x (both multiples of 16 bytes); then the barriers, the
+    // first entry position of the tile in each stage, and the row pattern
+    const uint32_t stage_bytes = (val_cap + x_cap) * (uint32_t)sizeof(T);
+    uint64_t *full = reinterpret_cast<uint64_t *>(st_raw + (size_t)stages * stage_bytes);
+    uint64_t *empty = full + stages;
+    uint32_t *s_lo = reinterpret_cast<uint32_t *>(empty + stages);
+    uint32_t *s_pat = s_lo + stages;
+    if (threadIdx.x == 0) {
+        for (uint32_t s = 0; s < stages; ++s) {
+            mbar_init(full + s, 3);                 // producer lanes 0 (with the copies' bytes), 1 and 2
+            mbar_init(empty + s, CONS / 32);
+        }
+        mbar_init_fence();
+    }
+    if (threadIdx.x < pat.len) s_pat[threadIdx.x] = pat.off[threadIdx.x];
+    __syncthreads();
+    const uint32_t rs = __ldg(cta_rows + blockIdx.x), re = __ldg(cta_rows + blockIdx.x + 1);
+    const uint32_t ntiles = (re - rs + R - 1) / R;
+    const size_t base = (size_t)blockIdx.x * (max_tiles + 1);
+    const uint32_t *t_lo = tile_lo + base, *t_reg = tile_reg + base;
+    const uint32_t K = pat.len, off0 = pat.off[0], off_last = pat.off[K - 1];
+
+    if (threadIdx.x >= CONS) {
+        // ---- producer: lanes 0-2 of the last warp, up to S regular tiles ahead of the consumers ----
+        const uint32_t lane = threadIdx.x - CONS;
+        if (lane > 2 || ntiles == 0) return;
+        const uint64_t pol = l2_policy_evict_first();
+        if (lane == 0) {                                           // the matrix does not change: start it early
+            for (uint32_t k = 0, n = 0; k < ntiles && n < stages; ++k) {
+                if (!__ldg(t_reg + k)) continue;
+                const uint32_t za = slice_lo(__ldg(t_lo + k));
+                l2_prefetch_bulk(val + za, (slice_hi(__ldg(t_lo + k + 1)) - za) * (uint32_t)sizeof(T));
+                ++n;
+            }
+        }
+        griddep_wait();                                            // no x byte before this
+        uint32_t s = 0, phase = 0, filled = 0;
+        for (uint32_t k = 0; k < ntiles; ++k) {
+            if (!__ldg(t_reg + k)) continue;
+            if (filled++ >= stages) mbar_wait(empty + s, phase ^ 1u);   // the consumers are done with this stage
+            const uint32_t r0 = rs + k * R, r1 = r0 + R < re ? r0 + R : re;
+            uint32_t a, b, xb;
+            band_window(x, r0, r1, off0, off_last, x_lo, x_hi, &a, &b, &xb);
+            unsigned char *sx = st_raw + (size_t)s * stage_bytes + (size_t)val_cap * sizeof(T);
+            const uintptr_t pa = reinterpret_cast<uintptr_t>(x + a), pb = reinterpret_cast<uintptr_t>(x + b);
+            const uintptr_t p16 = pa & ~(uintptr_t)15;                // stage byte 0 of the x area
+            const uintptr_t a16 = (pa + 15) & ~(uintptr_t)15, b16 = pb & ~(uintptr_t)15;
+            if (lane == 0) {
+                const uint32_t lo = __ldg(t_lo + k), za = slice_lo(lo), cnt = slice_hi(__ldg(t_lo + k + 1)) - za;
+                const uint32_t xbytes = b16 > a16 ? (uint32_t)(b16 - a16) : 0u;
+                s_lo[s] = lo;                                          // published by the arrive below (release)
+                T *sv = reinterpret_cast<T *>(st_raw + (size_t)s * stage_bytes);
+                mbar_expect_tx(full + s, cnt * (uint32_t)sizeof(T) + xbytes);
+                if (l2_hint) tma_bulk_g2s_hint(sv, val + za, cnt * (uint32_t)sizeof(T), full + s, pol);
+                else tma_bulk_g2s(sv, val + za, cnt * (uint32_t)sizeof(T), full + s);
+                if (xbytes) tma_bulk_g2s(sx + (a16 - p16), reinterpret_cast<const void *>(a16), xbytes, full + s);
+            } else {
+                // lane 1: the head [pa, min(a16, pb)); lane 2: the tail [max(a16, b16), pb)
+                uintptr_t p = lane == 1 ? pa : (a16 > b16 ? a16 : b16);
+                const uintptr_t e = lane == 1 ? (a16 < pb ? a16 : pb) : pb;
+                for (; p < e; p += sizeof(T))
+                    *reinterpret_cast<T *>(sx + (p - p16)) = __ldcg(reinterpret_cast<const T *>(p));
+                mbar_arrive(full + s);                                 // release: the stores above
+            }
+            if (++s == stages) { s = 0; phase ^= 1u; }
+        }
+        return;
+    }
+
+    // ---- consumers: CONS threads, LPR lanes per row; a regular tile reads nothing but its flag from global memory ----
+    const uint32_t rl = threadIdx.x / LPR, sub = threadIdx.x % LPR;
+    uint32_t s = 0, phase = 0;
+    griddep_wait();                    // x (and y's previous readers) belong to the launch before this one
+    if (threadIdx.x == 0) griddep_launch();
+    for (uint32_t k = 0; k < ntiles; ++k) {
+        const uint32_t r0 = rs + k * R, r = r0 + rl;
+        T acc = (T)0;
+        if (__ldg(t_reg + k)) {
+            const uint32_t r1 = r0 + R < re ? r0 + R : re;
+            uint32_t a, b, xb;
+            band_window(x, r0, r1, off0, off_last, x_lo, x_hi, &a, &b, &xb);
+            const T *sv = reinterpret_cast<const T *>(st_raw + (size_t)s * stage_bytes);
+            const T *sx = sv + val_cap;
+            mbar_wait(full + s, phase);
+            // stage position j holds the value of column s_pat[j - p0] + r
+            uint32_t p0 = 0, e = 0;
+            if (r < re) { p0 = (s_lo[s] & 3u) + rl * K; e = p0 + K; }
+            tile_row_sum<T, LPR, U>(acc, s_pat - p0, r, sv, p0, e, sub, [&](uint32_t c) { return sx[c - xb]; });
+            __syncwarp();
+            if (lane_id() == 0) mbar_arrive(empty + s);
+            if (++s == stages) { s = 0; phase ^= 1u; }
+        } else if (r < re) {
+            tile_row_sum<T, LPR, U>(acc, ind, 0u, val, __ldg(ptr + r), __ldg(ptr + r + 1), sub,
+                                    [&](uint32_t c) { return __ldg(x + c); });
+        }
+        acc = row_lanes_sum<LPR>(acc);
+        if (sub == 0 && r < re) y[r] = acc;
+    }
+}
+
+// The band kernel takes a matrix with a row pattern at most kBandWidthMax columns wide and at most one row off the
+// pattern per 64 tiles (a band: the rows at its two ends).  Stencils (boundary rows in most tiles) and matrices
+// without a pattern do not qualify.  Decided per matrix, never per grid: the partition is cached for one grid.
+bool band_eligible(const spl_mat *a) {
+    if (!a->pattern_len || !a->stream_rows) return false;
+    const uint32_t width = a->pattern_off[a->pattern_len - 1] - a->pattern_off[0];
+    const uint64_t ntiles = div_up(a->nrows, a->stream_rows);
+    return width <= kBandWidthMax && (uint64_t)a->pattern_breaks * 64u <= ntiles;
+}
+
+// x: array indexable by column over [x_lo, x_hi)
+template <typename T, int LPR, int U>
+void launch_band(spl_ctx *ctx, const spl_mat *a, const T *x, T *y, uint32_t x_lo, uint32_t x_hi) {
+    auto k = spmv_band_kernel<T, LPR, U>;
+    constexpr uint32_t R = tile_rows(LPR);
+    const uint32_t val_cap = stage_capacity(R * a->pattern_len);
+    const uint32_t width = a->pattern_off[a->pattern_len - 1] - a->pattern_off[0];
+    // the window's R + width columns and up to 15 bytes below it (the aligned start), in whole 16-byte units
+    const uint32_t x_cap = (uint32_t)(((R + width) * sizeof(T) + 15 + 15) / 16 * 16 / sizeof(T));
+    // shape (measured, profiles/r7_band_notes.md): three stages, three CTAs per SM
+    const uint32_t stages = (uint32_t)std::max(2, env_int("SPL_STREAM_STAGES", 3));
+    const size_t smem = (size_t)stages * (val_cap + x_cap) * sizeof(T) + (size_t)stages * (2 * sizeof(uint64_t) + 4) +
+                        kPatternMax * sizeof(uint32_t);
+    SPL_REQUIRE(smem <= 227 * 1024, SPL_ERR_UNSUPPORTED, "band SpMV: the stages do not fit in shared memory");
+    static std::atomic<size_t> smem_set{0};
+    static std::atomic<uint64_t> occ{0}, occ_run{0};
+    const uint32_t resident = stream_resident(k, smem, smem_set, occ);
+    uint32_t ctas = (uint32_t)env_int("SPL_STREAM_CTAS", 0);
+    if (ctas == 0 || ctas > resident) ctas = resident;
+    const size_t smem_run = smem_for_ctas(smem, ctas);
+    stream_resident(k, smem_run, smem_set, occ_run);             // sets the kernel's shared-memory size
+    const uint32_t grid = (uint32_t)ctx->num_sms * ctas;
+    stream_partition(ctx, const_cast<spl_mat *>(a), grid);
+    cudaLaunchConfig_t cfg{};
+    cfg.gridDim = dim3(grid);
+    cfg.blockDim = dim3(TILE_CONSUMERS + 32);
+    cfg.dynamicSmemBytes = smem_run;
+    cfg.stream = ctx->stream;
+    cudaLaunchAttribute attr[1];
+    attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
+    attr[0].val.programmaticStreamSerializationAllowed = 1;
+    cfg.attrs = attr;
+    cfg.numAttrs = (ctx->pdl_prev && !std::getenv("SPL_NO_PDL")) ? 1 : 0;     // only behind another stream-kernel product
+    SPL_CUDA(cudaLaunchKernelEx(&cfg, k, (const uint32_t *)a->ptr, (const uint32_t *)a->ind,
+                                static_cast<const T *>(a->val), x, y, (const uint32_t *)a->stream_cta_rows,
+                                (const uint32_t *)a->stream_tile_lo, (const uint32_t *)a->stream_tile_reg,
+                                a->stream_max_tiles, val_cap, x_cap, stages, x_lo, x_hi,
+                                env_int("SPL_STREAM_L2HINT", 1), row_pattern(a)));
+    check_launch(ctx, "spmv_band");
+    ctx->pdl_chain = true;
+}
+
+template <typename T, int LPR>
+void spmv_band_u(spl_ctx *ctx, const spl_mat *a, const T *x, T *y, uint32_t x_lo, uint32_t x_hi) {
+    if ((a->max_row_len + LPR - 1) / LPR > 4) launch_band<T, LPR, 8>(ctx, a, x, y, x_lo, x_hi);   // as spmv_stream_u
+    else launch_band<T, LPR, 4>(ctx, a, x, y, x_lo, x_hi);
+}
+
+template <typename T>
+void spmv_band(spl_ctx *ctx, const spl_mat *a, const T *x, T *y, uint32_t x_lo, uint32_t x_hi) {
+    switch (a->plan_lanes) {
+        case 1: spmv_band_u<T, 1>(ctx, a, x, y, x_lo, x_hi); break;
+        case 2: spmv_band_u<T, 2>(ctx, a, x, y, x_lo, x_hi); break;
+        case 4: spmv_band_u<T, 4>(ctx, a, x, y, x_lo, x_hi); break;
+        case 8: spmv_band_u<T, 8>(ctx, a, x, y, x_lo, x_hi); break;
+        case 16: spmv_band_u<T, 16>(ctx, a, x, y, x_lo, x_hi); break;
+        default: spmv_band_u<T, 32>(ctx, a, x, y, x_lo, x_hi); break;
     }
 }
 
@@ -1277,10 +1499,23 @@ __global__ void pattern_row_kernel(const uint32_t *__restrict__ ptr, uint32_t fr
     }
 }
 
+// *count += the rows that do not follow the row pattern
+__global__ void pattern_breaks_kernel(const uint32_t *__restrict__ ptr, const uint32_t *__restrict__ ind, uint32_t nrows,
+                                      const __grid_constant__ RowPattern pat, uint32_t *count) {
+    uint32_t m = 0;
+    for (uint64_t r = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x; r < nrows; r += (uint64_t)gridDim.x * blockDim.x)
+        m += row_follows(ind, ptr[r], ptr[r + 1], (uint32_t)r, pat) ? 0u : 1u;
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) m += __shfl_xor_sync(0xffffffffu, m, o);
+    if (lane_id() == 0 && m) atomicAdd(count, m);
+}
+
 // The row pattern (spl_mat::pattern_off): the column offsets of the first row at or after nrows / 2 with the
-// longest length, taken from the middle because the first rows of bands and stencils are boundary rows.
+// longest length, taken from the middle because the first rows of bands and stencils are boundary rows.  Then the
+// number of rows that do not follow it (spl_mat::pattern_breaks).
 void plan_pattern(spl_ctx *ctx, spl_mat *a) {
     a->pattern_len = 0;
+    a->pattern_breaks = 0;
     const uint32_t len = a->max_row_len;
     if (len == 0 || len > kPatternMax) return;
     SPL_CUDA(cudaMemsetAsync(ctx->d_scratch, 0xff, sizeof(uint32_t), ctx->stream));
@@ -1295,6 +1530,11 @@ void plan_pattern(spl_ctx *ctx, spl_mat *a) {
     read_back(ctx, a->ind + p, a->pattern_off, (int)len);
     for (uint32_t j = 0; j < len; ++j) a->pattern_off[j] -= row;
     a->pattern_len = len;
+    SPL_CUDA(cudaMemsetAsync(ctx->d_scratch, 0, sizeof(uint32_t), ctx->stream));
+    pattern_breaks_kernel<<<std::min<unsigned>(div_up(a->nrows, 256), (unsigned)ctx->num_sms * 8u), 256, 0, ctx->stream>>>(
+        a->ptr, a->ind, a->nrows, row_pattern(a), ctx->d_scratch);
+    check_launch(ctx, "pattern_breaks");
+    read_back(ctx, ctx->d_scratch, &a->pattern_breaks, 1);
 }
 
 }  // namespace
@@ -1463,6 +1703,13 @@ void spmv(spl_ctx *ctx, const spl_mat *a, const void *x, void *y, int kernel, in
                     "stream SpMV: a tile of rows does not fit in shared memory (skewed rows: use SPLIT)");
         if (a->nnz == 0) {
             SPL_CUDA(cudaMemsetAsync(y, 0, a->vsize() * (size_t)a->nrows, ctx->stream));
+            return;
+        }
+        // a band: its own kernel (SPL_STREAM_BAND=0, or SPL_STREAM_PATTERN=0 with the other row-pattern path, turns it
+        // off for A/B measurements)
+        if (band_eligible(a) && env_int("SPL_STREAM_BAND", 1) != 0 && env_int("SPL_STREAM_PATTERN", 1) != 0) {
+            if (a->dtype == SPL_F32) spmv_band<float>(ctx, a, (const float *)x, (float *)y, x_lo, x_hi);
+            else spmv_band<double>(ctx, a, (const double *)x, (double *)y, x_lo, x_hi);
             return;
         }
         if (a->dtype == SPL_F32) spmv_stream<float>(ctx, a, XLocal<float>{(const float *)x}, (float *)y, (const float *)x, x_lo, x_hi);
