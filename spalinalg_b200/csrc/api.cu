@@ -665,7 +665,7 @@ int spl_mat_set_values(spl_ctx *ctx, spl_mat *m, const void *val) {
     if (m->nnz) {
         SPL_CUDA(cudaMemcpyAsync(m->val, val, (size_t)m->nnz * m->vsize(), cudaMemcpyHostToDevice, ctx->stream));
         SPL_CUDA(cudaStreamSynchronize(ctx->stream));      // the caller may reuse its buffer at once
-        drop_value_copies(ctx, m);                         // copies of the old values: CSR twin, sliced SpMV copy
+        drop_value_copies(ctx, m);                         // copies of the old values: CSR twin, sliced SpMV copy, band value codes
     }
     API_END(ctx)
 }

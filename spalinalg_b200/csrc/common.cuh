@@ -42,6 +42,8 @@ constexpr int kNumSmFallback = 148;
 constexpr uint64_t kMaxEntries = (1ull << 32) - 65536;
 // longest row whose column offsets the SpMV plan keeps as the matrix's row pattern (spl_mat::pattern_off)
 constexpr uint32_t kPatternMax = 64;
+// most distinct values a matrix may hold for the band kernel to stream one-byte codes of them (spl_mat::val_codes)
+constexpr uint32_t kCodesMax = 256;
 
 // A test-only setting from the environment: true and *v when `name` holds a decimal number and nothing else;
 // false when it is unset, empty or anything else, so that a typo leaves the library's default in place.
@@ -150,6 +152,16 @@ struct spl_mat {
     uint32_t pattern_len = 0, pattern_breaks = 0;
     uint32_t *stream_tile_reg = nullptr;
     uint32_t stream_regular = 0;
+    // one-byte value codes for the band kernel (spmv.cu, band_codes), a derived copy of the values like slice_val: a
+    // matrix with at most kCodesMax distinct values (by bit pattern) keeps them in code_dict (device, code_count of
+    // them; code_bits: their bit patterns on the host, ascending, which is the code order) and the code of entry j of
+    // every row r with pattern_len = K entries at byte (r / 32) * 32 K + 32 j + r % 32 of val_codes (planar by 32-row
+    // group).  code_state: 0 not tried, 2 decided (val_codes set or not); built by the first band product.
+    uint8_t *val_codes = nullptr;
+    void *code_dict = nullptr;
+    uint64_t code_bits[spl::kCodesMax] = {};
+    uint32_t code_count = 0;
+    std::atomic<int> code_state{0};
 
     // CSR form of a CSC matrix (same matrix, other format), built by the first product y = A x on it
     // and kept: products on a CscMatrix then run the row kernels at full speed and in the reference's

@@ -286,8 +286,9 @@ spmv_gather_fused_kernel(uint32_t nloc, const uint32_t *__restrict__ bptr, uint3
             T acc = (T)0;
             // block 0 reads the published slice (constant for the whole kernel); x_full is written by this very kernel,
             // behind the acquire that let this block start: L2 loads
-            if (k == 0) tile_row_sum<T, LPR, U>(acc, ci, 0, cv, p0, e, sub, [&](uint32_t col) { return __ldg(own + col); });
-            else tile_row_sum<T, LPR, U>(acc, ci, 0, cv, p0, e, sub, [&](uint32_t col) { return __ldcg(x_full + col); });
+            const auto vals = [&](uint32_t j) { return cv[j]; };
+            if (k == 0) tile_row_sum<T, LPR, U>(acc, ci, 0, vals, p0, e, sub, [&](uint32_t col) { return __ldg(own + col); });
+            else tile_row_sum<T, LPR, U>(acc, ci, 0, vals, p0, e, sub, [&](uint32_t col) { return __ldcg(x_full + col); });
             __syncwarp();
             if (lane == 0) mbar_arrive(empty + s);
             acc = row_lanes_sum<LPR>(acc);

@@ -242,6 +242,8 @@ void free_mat(spl_ctx *ctx, spl_mat *m) {
     dfree(ctx, m->stream_xlo0);
     dfree(ctx, m->stream_tile_lo);
     dfree(ctx, m->stream_tile_reg);
+    dfree(ctx, m->val_codes);
+    dfree(ctx, m->code_dict);
     delete m;
 }
 

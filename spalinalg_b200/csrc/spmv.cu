@@ -652,10 +652,11 @@ spmv_stream_kernel(uint32_t nrows, const uint32_t *__restrict__ ptr, const uint3
         }
         T acc = (T)0;
         // the row's columns are sorted: first and last entry bound them
+        const auto vals = [&](uint32_t j) { return cv[j]; };
         if (e <= p0 || xg.all_local(cb[p0] + cadd, cb[e - 1] + cadd))
-            tile_row_sum<T, LPR, U>(acc, cb, cadd, cv, p0, e, sub, [&](uint32_t c) { return xg.local(c); });
+            tile_row_sum<T, LPR, U>(acc, cb, cadd, vals, p0, e, sub, [&](uint32_t c) { return xg.local(c); });
         else
-            tile_row_sum<T, LPR, U>(acc, cb, cadd, cv, p0, e, sub, [&](uint32_t c) { return xg(c); });
+            tile_row_sum<T, LPR, U>(acc, cb, cadd, vals, p0, e, sub, [&](uint32_t c) { return xg(c); });
         __syncwarp();
         if (lane_id() == 0) mbar_arrive(empty + s);
         acc = row_lanes_sum<LPR>(acc);
@@ -863,6 +864,12 @@ void spmv_stream(spl_ctx *ctx, const spl_mat *a, const XG &xg, T *y, const T *x_
 //     aligned and may end at the footprint): lane 0 bulk-copies the 16-byte aligned inside of the window, lanes 1
 //     and 2 load its ragged head and tail (under 16 bytes each) with plain loads, store them and arrive on the
 //     stage's full barrier.
+//   * a matrix with at most kCodesMax distinct values (band_codes) runs spmv_band_codes_kernel: its stages hold the
+//     tile's one-byte value codes (spl_mat::val_codes) in place of the values, and a dictionary of the values sits in
+//     shared memory from the CTA's start (the matrix does not change, so it is read before griddepcontrol.wait).  A
+//     consumer reads dict[code], the very value, so y keeps its bits.  The codes are planar by 32-row group: a warp
+//     reads the codes of its 32 rows for one entry as 32 consecutive bytes.  A tile copies the whole groups its rows
+//     touch (32-byte aligned, one group more than R / 32 when the tile does not start on a group).
 constexpr uint32_t kBandWidthMax = 4096;     // widest row pattern (last column - first column) the band kernel takes
 
 // The x window of the regular tile of rows [r0, r1): columns [*a, *b), clamped to [x_lo, x_hi); its stage area starts
@@ -876,23 +883,38 @@ __device__ __forceinline__ void band_window(const T *x, uint32_t r0, uint32_t r1
     *xb = *a - (uint32_t)((reinterpret_cast<uintptr_t>(x + *a) & 15u) / sizeof(T));
 }
 
-template <typename T, int LPR, int U>
-__global__ void __launch_bounds__(TILE_CONSUMERS + 32, 3)
-spmv_band_kernel(const uint32_t *__restrict__ ptr, const uint32_t *__restrict__ ind, const T *__restrict__ val,
-                 const T *__restrict__ x, T *__restrict__ y, const uint32_t *__restrict__ cta_rows,
-                 const uint32_t *__restrict__ tile_lo, const uint32_t *__restrict__ tile_reg, uint32_t max_tiles,
-                 uint32_t val_cap, uint32_t x_cap, uint32_t stages, uint32_t x_lo, uint32_t x_hi, int l2_hint,
-                 const __grid_constant__ RowPattern pat) {
+// The stage bytes of the code groups of rows [r0, r1) of a K-entry pattern: [*at, *at + *bytes) of val_codes
+__device__ __forceinline__ void band_code_groups(uint32_t r0, uint32_t r1, uint32_t K, uint64_t *at, uint32_t *bytes) {
+    *at = (uint64_t)(r0 / 32u) * 32u * K;
+    *bytes = ((r1 - 1u) / 32u - r0 / 32u + 1u) * 32u * K;
+}
+
+// The band kernel's body.  CODES = false: a stage holds the tile's values (spmv_band_kernel), val_cap of them;
+// CODES = true: its code groups (spmv_band_codes_kernel), val_cap bytes, and the ndict values of `dict` are in shared
+// memory.
+template <typename T, int LPR, int U, bool CODES>
+__device__ __forceinline__ void band_body(const uint32_t *__restrict__ ptr, const uint32_t *__restrict__ ind,
+                                          const T *__restrict__ val, const uint8_t *__restrict__ codes,
+                                          const T *__restrict__ dict, uint32_t ndict, const T *__restrict__ x,
+                                          T *__restrict__ y, const uint32_t *__restrict__ cta_rows,
+                                          const uint32_t *__restrict__ tile_lo, const uint32_t *__restrict__ tile_reg,
+                                          uint32_t max_tiles, uint32_t val_cap, uint32_t x_cap, uint32_t stages,
+                                          uint32_t x_lo, uint32_t x_hi, int l2_hint, const RowPattern &pat) {
     constexpr uint32_t CONS = TILE_CONSUMERS;
     constexpr uint32_t R = tile_rows(LPR);
     extern __shared__ __align__(128) unsigned char st_raw[];
-    // per stage: [val_cap] values, then [x_cap] elements of x (both multiples of 16 bytes); then the barriers, the
-    // first entry position of the tile in each stage, and the row pattern
-    const uint32_t stage_bytes = (val_cap + x_cap) * (uint32_t)sizeof(T);
-    uint64_t *full = reinterpret_cast<uint64_t *>(st_raw + (size_t)stages * stage_bytes);
+    // per stage: [val_cap] values (CODES: val_cap bytes of codes), then [x_cap] elements of x (both multiples of 16
+    // bytes); then (CODES) the dictionary, kCodesMax values; then the barriers, the first entry position of the tile
+    // in each stage, and the row pattern
+    const uint32_t stage_bytes = CODES ? val_cap + x_cap * (uint32_t)sizeof(T) : (val_cap + x_cap) * (uint32_t)sizeof(T);
+    T *s_dict = reinterpret_cast<T *>(st_raw + (size_t)stages * stage_bytes);
+    uint64_t *full = reinterpret_cast<uint64_t *>(st_raw + (size_t)stages * stage_bytes + (CODES ? kCodesMax * sizeof(T) : 0));
     uint64_t *empty = full + stages;
     uint32_t *s_lo = reinterpret_cast<uint32_t *>(empty + stages);
     uint32_t *s_pat = s_lo + stages;
+    if constexpr (CODES) {
+        for (uint32_t i = threadIdx.x; i < ndict; i += blockDim.x) s_dict[i] = __ldg(dict + i);
+    }
     if (threadIdx.x == 0) {
         for (uint32_t s = 0; s < stages; ++s) {
             mbar_init(full + s, 3);                 // producer lanes 0 (with the copies' bytes), 1 and 2
@@ -916,8 +938,16 @@ spmv_band_kernel(const uint32_t *__restrict__ ptr, const uint32_t *__restrict__ 
         if (lane == 0) {                                           // the matrix does not change: start it early
             for (uint32_t k = 0, n = 0; k < ntiles && n < stages; ++k) {
                 if (!__ldg(t_reg + k)) continue;
-                const uint32_t za = slice_lo(__ldg(t_lo + k));
-                l2_prefetch_bulk(val + za, (slice_hi(__ldg(t_lo + k + 1)) - za) * (uint32_t)sizeof(T));
+                if constexpr (CODES) {
+                    const uint32_t r0 = rs + k * R;
+                    uint64_t at;
+                    uint32_t bytes;
+                    band_code_groups(r0, r0 + R < re ? r0 + R : re, K, &at, &bytes);
+                    l2_prefetch_bulk(codes + at, bytes);
+                } else {
+                    const uint32_t za = slice_lo(__ldg(t_lo + k));
+                    l2_prefetch_bulk(val + za, (slice_hi(__ldg(t_lo + k + 1)) - za) * (uint32_t)sizeof(T));
+                }
                 ++n;
             }
         }
@@ -929,11 +959,21 @@ spmv_band_kernel(const uint32_t *__restrict__ ptr, const uint32_t *__restrict__ 
             const uint32_t r0 = rs + k * R, r1 = r0 + R < re ? r0 + R : re;
             uint32_t a, b, xb;
             band_window(x, r0, r1, off0, off_last, x_lo, x_hi, &a, &b, &xb);
-            unsigned char *sx = st_raw + (size_t)s * stage_bytes + (size_t)val_cap * sizeof(T);
+            unsigned char *sx = st_raw + (size_t)s * stage_bytes + (CODES ? (size_t)val_cap : (size_t)val_cap * sizeof(T));
             const uintptr_t pa = reinterpret_cast<uintptr_t>(x + a), pb = reinterpret_cast<uintptr_t>(x + b);
             const uintptr_t p16 = pa & ~(uintptr_t)15;                // stage byte 0 of the x area
             const uintptr_t a16 = (pa + 15) & ~(uintptr_t)15, b16 = pb & ~(uintptr_t)15;
-            if (lane == 0) {
+            if (lane == 0 && CODES) {
+                uint64_t at;
+                uint32_t bytes;
+                band_code_groups(r0, r1, K, &at, &bytes);
+                const uint32_t xbytes = b16 > a16 ? (uint32_t)(b16 - a16) : 0u;
+                unsigned char *sc = st_raw + (size_t)s * stage_bytes;
+                mbar_expect_tx(full + s, bytes + xbytes);
+                if (l2_hint) tma_bulk_g2s_hint(sc, codes + at, bytes, full + s, pol);
+                else tma_bulk_g2s(sc, codes + at, bytes, full + s);
+                if (xbytes) tma_bulk_g2s(sx + (a16 - p16), reinterpret_cast<const void *>(a16), xbytes, full + s);
+            } else if (lane == 0) {
                 const uint32_t lo = __ldg(t_lo + k), za = slice_lo(lo), cnt = slice_hi(__ldg(t_lo + k + 1)) - za;
                 const uint32_t xbytes = b16 > a16 ? (uint32_t)(b16 - a16) : 0u;
                 s_lo[s] = lo;                                          // published by the arrive below (release)
@@ -967,23 +1007,66 @@ spmv_band_kernel(const uint32_t *__restrict__ ptr, const uint32_t *__restrict__ 
             const uint32_t r1 = r0 + R < re ? r0 + R : re;
             uint32_t a, b, xb;
             band_window(x, r0, r1, off0, off_last, x_lo, x_hi, &a, &b, &xb);
-            const T *sv = reinterpret_cast<const T *>(st_raw + (size_t)s * stage_bytes);
-            const T *sx = sv + val_cap;
-            mbar_wait(full + s, phase);
-            // stage position j holds the value of column s_pat[j - p0] + r
-            uint32_t p0 = 0, e = 0;
-            if (r < re) { p0 = (s_lo[s] & 3u) + rl * K; e = p0 + K; }
-            tile_row_sum<T, LPR, U>(acc, s_pat - p0, r, sv, p0, e, sub, [&](uint32_t c) { return sx[c - xb]; });
+            if constexpr (CODES) {
+                const unsigned char *sc = st_raw + (size_t)s * stage_bytes;
+                const T *sx = reinterpret_cast<const T *>(sc + val_cap);
+                mbar_wait(full + s, phase);
+                // entry j of row r: column s_pat[j] + r (x at sx[r - xb + s_pat[j]], mod 2^32), code at stage byte
+                // q + 32 j.  Lane sub sums entries sub, sub + LPR, ... in order, the lane order of tile_row_sum.  A
+                // regular row has all K entries, so there is no masked slot, whose explicit +0 leaves acc unchanged
+                // anyway (acc starts at +0 and a sum never turns it to -0).  Without the masks and the column
+                // sentinel, an entry costs a third fewer instructions than in tile_row_sum, and the consumers bound
+                // this kernel (r8_band_codes_notes.md).
+                if (r < re) {
+                    const uint32_t q = (r / 32u - r0 / 32u) * 32u * K + r % 32u, rx = r - xb;
+#pragma unroll 4
+                    for (uint32_t j = sub; j < K; j += LPR) acc += s_dict[sc[q + 32u * j]] * sx[rx + s_pat[j]];
+                }
+            } else {
+                const T *sv = reinterpret_cast<const T *>(st_raw + (size_t)s * stage_bytes);
+                const T *sx = sv + val_cap;
+                mbar_wait(full + s, phase);
+                // stage position j holds the value of column s_pat[j - p0] + r
+                uint32_t p0 = 0, e = 0;
+                if (r < re) { p0 = (s_lo[s] & 3u) + rl * K; e = p0 + K; }
+                tile_row_sum<T, LPR, U>(acc, s_pat - p0, r, [&](uint32_t j) { return sv[j]; }, p0, e, sub,
+                                        [&](uint32_t c) { return sx[c - xb]; });
+            }
             __syncwarp();
             if (lane_id() == 0) mbar_arrive(empty + s);
             if (++s == stages) { s = 0; phase ^= 1u; }
         } else if (r < re) {
-            tile_row_sum<T, LPR, U>(acc, ind, 0u, val, __ldg(ptr + r), __ldg(ptr + r + 1), sub,
-                                    [&](uint32_t c) { return __ldg(x + c); });
+            tile_row_sum<T, LPR, U>(acc, ind, 0u, [&](uint32_t j) { return val[j]; }, __ldg(ptr + r), __ldg(ptr + r + 1),
+                                    sub, [&](uint32_t c) { return __ldg(x + c); });
         }
         acc = row_lanes_sum<LPR>(acc);
         if (sub == 0 && r < re) y[r] = acc;
     }
+}
+
+template <typename T, int LPR, int U>
+__global__ void __launch_bounds__(TILE_CONSUMERS + 32, 3)
+spmv_band_kernel(const uint32_t *__restrict__ ptr, const uint32_t *__restrict__ ind, const T *__restrict__ val,
+                 const T *__restrict__ x, T *__restrict__ y, const uint32_t *__restrict__ cta_rows,
+                 const uint32_t *__restrict__ tile_lo, const uint32_t *__restrict__ tile_reg, uint32_t max_tiles,
+                 uint32_t val_cap, uint32_t x_cap, uint32_t stages, uint32_t x_lo, uint32_t x_hi, int l2_hint,
+                 const __grid_constant__ RowPattern pat) {
+    band_body<T, LPR, U, false>(ptr, ind, val, nullptr, nullptr, 0u, x, y, cta_rows, tile_lo, tile_reg, max_tiles,
+                                val_cap, x_cap, stages, x_lo, x_hi, l2_hint, pat);
+}
+
+// Its stages are a quarter of the value kernel's or less (C5: 4.7 against 20.6 KB), so deeper rings and more CTAs
+// fit: four CTAs of 288 threads, at most 56 registers each (48 or fewer, no spills).
+template <typename T, int LPR, int U>
+__global__ void __launch_bounds__(TILE_CONSUMERS + 32, 4)
+spmv_band_codes_kernel(const uint32_t *__restrict__ ptr, const uint32_t *__restrict__ ind, const T *__restrict__ val,
+                       const uint8_t *__restrict__ codes, const T *__restrict__ dict, uint32_t ndict,
+                       const T *__restrict__ x, T *__restrict__ y, const uint32_t *__restrict__ cta_rows,
+                       const uint32_t *__restrict__ tile_lo, const uint32_t *__restrict__ tile_reg, uint32_t max_tiles,
+                       uint32_t code_cap, uint32_t x_cap, uint32_t stages, uint32_t x_lo, uint32_t x_hi, int l2_hint,
+                       const __grid_constant__ RowPattern pat) {
+    band_body<T, LPR, U, true>(ptr, ind, val, codes, dict, ndict, x, y, cta_rows, tile_lo, tile_reg, max_tiles,
+                               code_cap, x_cap, stages, x_lo, x_hi, l2_hint, pat);
 }
 
 // The band kernel takes a matrix with a row pattern at most kBandWidthMax columns wide and at most one row off the
@@ -996,20 +1079,233 @@ bool band_eligible(const spl_mat *a) {
     return width <= kBandWidthMax && (uint64_t)a->pattern_breaks * 64u <= ntiles;
 }
 
-// x: array indexable by column over [x_lo, x_hi)
-template <typename T, int LPR, int U>
-void launch_band(spl_ctx *ctx, const spl_mat *a, const T *x, T *y, uint32_t x_lo, uint32_t x_hi) {
-    auto k = spmv_band_kernel<T, LPR, U>;
-    constexpr uint32_t R = tile_rows(LPR);
-    const uint32_t val_cap = stage_capacity(R * a->pattern_len);
-    const uint32_t width = a->pattern_off[a->pattern_len - 1] - a->pattern_off[0];
+// ------------------------------------------------------------------ one-byte value codes (band kernel)
+// A matrix with at most kCodesMax distinct values, told apart by bit pattern (+0.0 and -0.0 are two values, a NaN
+// keeps its payload), stores a dictionary of them and a one-byte code per entry of every row with K = pattern_len
+// entries (spl_mat::val_codes); the band kernel then streams 1 byte per entry in place of 4 or 8.  value_set_kernel
+// collects the distinct values: a set per CTA in shared memory, merged into one global table at the CTA's end.  A CTA
+// that sees more than kCodesMax values raises a flag that every CTA polls once per round of 8 values per thread, so a
+// matrix with many values costs about one round of reads.  The codes follow the ascending bit patterns (sorted on the
+// host): the same matrix always gets the same codes.
+constexpr uint64_t kNoKey = ~0ull;                  // an empty slot (the one value with these bits is flagged apart)
+// 1024 slots per CTA: a thread stops at its first insert past kCodesMax, so at most kCodesMax + 256 keys (one per
+// thread) go in and the set stays at most half full; 1024 in the global table
+constexpr uint32_t kSetBits = 10, kTableBits = 10;
+
+__device__ __forceinline__ uint64_t value_key(float v) { return __float_as_uint(v); }
+__device__ __forceinline__ uint64_t value_key(double v) { return (uint64_t)__double_as_longlong(v); }
+__device__ __forceinline__ uint32_t key_hash(uint64_t k, uint32_t bits) {
+    return (uint32_t)((k * 0x9E3779B97F4A7C15ull) >> (64 - bits));
+}
+
+// Puts k (not kNoKey) into the open-addressing set of 2^bits slots (shared or global memory): 1 when it was not there,
+// 0 when it was, -1 when the set is full.
+__device__ __forceinline__ int key_insert(unsigned long long *set, uint32_t bits, uint64_t k) {
+    const uint32_t mask = (1u << bits) - 1u;
+    uint32_t h = key_hash(k, bits);
+    for (uint32_t i = 0; i <= mask; ++i, h = (h + 1u) & mask) {
+        unsigned long long cur = *reinterpret_cast<volatile unsigned long long *>(set + h);
+        if (cur == kNoKey) cur = atomicCAS(set + h, kNoKey, (unsigned long long)k);
+        if (cur == kNoKey) return 1;
+        if (cur == k) return 0;
+    }
+    return -1;
+}
+
+// table: 2^kTableBits slots, all kNoKey.  state[0] = keys in the table, state[1] = 1 when there are more than
+// kCodesMax distinct values (the table is then incomplete), state[2] = 1 when the value with bits kNoKey occurs.
+template <typename T>
+__global__ void __launch_bounds__(256)
+value_set_kernel(const T *__restrict__ val, uint32_t nnz, unsigned long long *table, uint32_t *state) {
+    constexpr uint32_t kRound = 8;
+    __shared__ unsigned long long set[1u << kSetBits];
+    __shared__ uint32_t s_count;
+    for (uint32_t i = threadIdx.x; i < (1u << kSetBits); i += blockDim.x) set[i] = kNoKey;
+    if (threadIdx.x == 0) s_count = 0;
+    __syncthreads();
+    const uint64_t stride = (uint64_t)gridDim.x * blockDim.x;
+    bool nokey = false;
+    for (uint64_t b0 = (uint64_t)blockIdx.x * blockDim.x; b0 < nnz; b0 += kRound * stride) {
+        T v[kRound];
+#pragma unroll
+        for (uint32_t u = 0; u < kRound; ++u) {
+            const uint64_t i = b0 + threadIdx.x + u * stride;
+            v[u] = i < nnz ? val[i] : val[0];
+        }
+        bool over = false;
+#pragma unroll
+        for (uint32_t u = 0; u < kRound; ++u) {
+            const uint64_t k = value_key(v[u]);
+            if (over) continue;                         // this thread is past kCodesMax: no more inserts
+            if (k == kNoKey) { nokey = true; continue; }
+            const int fresh = key_insert(set, kSetBits, k);
+            if (fresh < 0 || (fresh > 0 && atomicAdd(&s_count, 1u) >= kCodesMax)) over = true;
+        }
+        if (__syncthreads_or(over || (threadIdx.x == 0 && *reinterpret_cast<volatile uint32_t *>(state + 1)))) {
+            if (over) atomicExch(state + 1, 1u);
+            return;
+        }
+    }
+    if (nokey) atomicExch(state + 2, 1u);
+    for (uint32_t h = threadIdx.x; h < (1u << kSetBits); h += blockDim.x) {
+        const unsigned long long k = set[h];
+        if (k == kNoKey) continue;
+        const int fresh = key_insert(table, kTableBits, k);
+        if (fresh < 0 || (fresh > 0 && atomicAdd(state, 1u) >= kCodesMax)) atomicExch(state + 1, 1u);
+    }
+}
+
+// codes[(r / 32) * 32 K + 32 j + r % 32] = the code of entry j of row r, for every row with K entries (the others are
+// off the pattern: their tiles never read codes); dict: the ndict values in code order
+template <typename T>
+__global__ void __launch_bounds__(256)
+encode_codes_kernel(const uint32_t *__restrict__ ptr, const T *__restrict__ val, uint32_t nrows, uint32_t K,
+                    const T *__restrict__ dict, uint32_t ndict, uint8_t *__restrict__ codes) {
+    constexpr uint32_t mask = (1u << kSetBits) - 1u;
+    __shared__ unsigned long long set[1u << kSetBits];
+    __shared__ uint8_t code_at[1u << kSetBits];
+    __shared__ uint8_t nokey_code;
+    for (uint32_t i = threadIdx.x; i <= mask; i += blockDim.x) set[i] = kNoKey;
+    __syncthreads();
+    if (threadIdx.x == 0) {
+        for (uint32_t c = 0; c < ndict; ++c) {
+            const uint64_t k = value_key(dict[c]);
+            if (k == kNoKey) { nokey_code = (uint8_t)c; continue; }
+            uint32_t h = key_hash(k, kSetBits);
+            while (set[h] != kNoKey) h = (h + 1u) & mask;
+            set[h] = k;
+            code_at[h] = (uint8_t)c;
+        }
+    }
+    __syncthreads();
+    for (uint64_t r = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x; r < nrows; r += (uint64_t)gridDim.x * blockDim.x) {
+        const uint32_t lo = ptr[r];
+        if (ptr[r + 1] - lo != K) continue;
+        uint8_t *out = codes + (r / 32u) * 32u * K + r % 32u;
+        for (uint32_t j = 0; j < K; ++j) {
+            const uint64_t k = value_key(val[lo + j]);
+            uint8_t c = nokey_code;
+            if (k != kNoKey) {
+                uint32_t h = key_hash(k, kSetBits);
+                for (uint32_t i = 0; i < mask && set[h] != k; ++i) h = (h + 1u) & mask;
+                c = code_at[h];
+            }
+            out[32u * j] = c;
+        }
+    }
+}
+
+// The dictionary and the codes of a band matrix (spl_mat::val_codes), or none when it has more than kCodesMax
+// distinct values or the codes do not fit in memory.
+template <typename T>
+void plan_codes(spl_ctx *ctx, spl_mat *a) {
+    const uint32_t K = a->pattern_len;
+    Tmp<unsigned long long> table(ctx, 1u << kTableBits);
+    SPL_CUDA(cudaMemsetAsync(table, 0xff, sizeof(unsigned long long) << kTableBits, ctx->stream));
+    SPL_CUDA(cudaMemsetAsync(ctx->d_scratch, 0, 3 * sizeof(uint32_t), ctx->stream));
+    value_set_kernel<T><<<std::min<unsigned>(div_up(a->nnz, 256), (unsigned)ctx->num_sms * 8u), 256, 0, ctx->stream>>>(
+        static_cast<const T *>(a->val), a->nnz, table, ctx->d_scratch);
+    check_launch(ctx, "value_set");
+    uint32_t st[3];
+    read_back(ctx, ctx->d_scratch, st, 3);
+    if (st[1] || st[0] + st[2] > kCodesMax) return;
+    std::vector<unsigned long long> slots(1u << kTableBits);
+    SPL_CUDA(cudaMemcpyAsync(slots.data(), table, sizeof(unsigned long long) << kTableBits, cudaMemcpyDeviceToHost,
+                             ctx->stream));
+    SPL_CUDA(cudaStreamSynchronize(ctx->stream));
+    std::vector<uint64_t> keys;
+    for (unsigned long long k : slots)
+        if (k != kNoKey) keys.push_back(k);
+    if (st[2]) keys.push_back(kNoKey);
+    std::sort(keys.begin(), keys.end());
+    std::vector<T> dict(keys.size());
+    for (size_t c = 0; c < keys.size(); ++c) {
+        if constexpr (sizeof(T) == 4) {
+            const uint32_t b = (uint32_t)keys[c];
+            std::memcpy(&dict[c], &b, 4);
+        } else {
+            std::memcpy(&dict[c], &keys[c], 8);
+        }
+    }
+    const uint64_t code_bytes = (uint64_t)div_up(a->nrows, 32) * 32u * K;
+    T *d_dict = nullptr;
+    uint8_t *codes = nullptr;
+    try {
+        d_dict = dalloc<T>(ctx, dict.size());
+        codes = dalloc<uint8_t>(ctx, code_bytes);
+    } catch (const Error &e) {
+        if (e.status != SPL_ERR_OOM) throw;
+        cudaGetLastError();
+        dfree(ctx, d_dict);
+        return;                                         // the band kernel streams the values instead
+    }
+    SPL_CUDA(cudaMemcpyAsync(d_dict, dict.data(), dict.size() * sizeof(T), cudaMemcpyHostToDevice, ctx->stream));
+    encode_codes_kernel<T><<<std::min<unsigned>(div_up(a->nrows, 256), (unsigned)ctx->num_sms * 8u), 256, 0, ctx->stream>>>(
+        a->ptr, static_cast<const T *>(a->val), a->nrows, K, d_dict, (uint32_t)dict.size(), codes);
+    check_launch(ctx, "encode_codes");
+    SPL_CUDA(cudaStreamSynchronize(ctx->stream));      // visible to any other stream from here on
+    a->code_dict = d_dict;
+    a->val_codes = codes;
+    a->code_count = (uint32_t)keys.size();
+    std::copy(keys.begin(), keys.end(), a->code_bits);
+}
+
+// Whether the band matrix a has value codes: planned by its first band product, and again after set_values
+// (drop_value_copies)
+bool band_codes(spl_ctx *ctx, spl_mat *a) {
+    if (a->code_state.load(std::memory_order_acquire) != 2) {
+        std::lock_guard<std::mutex> lock(a->plan_mu);
+        if (a->code_state.load(std::memory_order_relaxed) != 2) {
+            if (a->dtype == SPL_F32) plan_codes<float>(ctx, a);
+            else plan_codes<double>(ctx, a);
+            a->code_state.store(2, std::memory_order_release);
+        }
+    }
+    return a->val_codes != nullptr;
+}
+
+constexpr size_t kBandSmemMax = 227 * 1024;
+
+// The band kernel's shared memory for matrix a and tiles of R rows.  A stage holds the values (CODES: the code groups)
+// and the x window, and comes with two barriers and a word; the rest is the row pattern and (CODES) the dictionary.
+struct BandShape {
+    uint32_t val_cap, x_cap;
+    size_t stage_bytes, fixed;
+    size_t smem(uint32_t stages) const { return (size_t)stages * (stage_bytes + 2 * sizeof(uint64_t) + 4) + fixed; }
+};
+
+template <typename T, bool CODES>
+BandShape band_shape(const spl_mat *a, uint32_t R) {
+    const uint32_t K = a->pattern_len;
+    BandShape sh;
+    // CODES: bytes of the largest run of 32-row groups a tile touches (it starts on a multiple of 4 rows)
+    sh.val_cap = CODES ? ((R + 27) / 32 + 1) * 32 * K : stage_capacity(R * K);
+    const uint32_t width = a->pattern_off[K - 1] - a->pattern_off[0];
     // the window's R + width columns and up to 15 bytes below it (the aligned start), in whole 16-byte units
-    const uint32_t x_cap = (uint32_t)(((R + width) * sizeof(T) + 15 + 15) / 16 * 16 / sizeof(T));
-    // shape (measured, profiles/r7_band_notes.md): three stages, three CTAs per SM
-    const uint32_t stages = (uint32_t)std::max(2, env_int("SPL_STREAM_STAGES", 3));
-    const size_t smem = (size_t)stages * (val_cap + x_cap) * sizeof(T) + (size_t)stages * (2 * sizeof(uint64_t) + 4) +
-                        kPatternMax * sizeof(uint32_t);
-    SPL_REQUIRE(smem <= 227 * 1024, SPL_ERR_UNSUPPORTED, "band SpMV: the stages do not fit in shared memory");
+    sh.x_cap = (uint32_t)(((R + width) * sizeof(T) + 15 + 15) / 16 * 16 / sizeof(T));
+    sh.stage_bytes = CODES ? sh.val_cap + (size_t)sh.x_cap * sizeof(T) : (size_t)(sh.val_cap + sh.x_cap) * sizeof(T);
+    sh.fixed = (CODES ? kCodesMax * sizeof(T) : 0) + kPatternMax * sizeof(uint32_t);
+    return sh;
+}
+
+// x: array indexable by column over [x_lo, x_hi).  CODES: the code kernel (a->val_codes is set)
+template <typename T, int LPR, int U, bool CODES>
+void launch_band(spl_ctx *ctx, const spl_mat *a, const T *x, T *y, uint32_t x_lo, uint32_t x_hi) {
+    constexpr uint32_t R = tile_rows(LPR);
+    const BandShape sh = band_shape<T, CODES>(a, R);
+    const uint32_t val_cap = sh.val_cap, x_cap = sh.x_cap;
+    // shape (measured, profiles/r7_band_notes.md and r8_band_codes_notes.md): values: three stages, three CTAs per
+    // SM; codes: eight stages, four CTAs.  The x window of a wide pattern (up to kBandWidthMax columns) leaves room for
+    // fewer stages: the code kernel then runs as many as fit, two at least (spmv_band checked that two fit).
+    uint32_t stages = (uint32_t)std::max(2, env_int("SPL_STREAM_STAGES", CODES ? 8 : 3));
+    if (CODES)
+        while (stages > 2 && sh.smem(stages) > kBandSmemMax) --stages;
+    const size_t smem = sh.smem(stages);
+    SPL_REQUIRE(smem <= kBandSmemMax, SPL_ERR_UNSUPPORTED, "band SpMV: the stages do not fit in shared memory");
+    const auto k = [] {
+        if constexpr (CODES) return spmv_band_codes_kernel<T, LPR, U>;
+        else return spmv_band_kernel<T, LPR, U>;
+    }();
     static std::atomic<size_t> smem_set{0};
     static std::atomic<uint64_t> occ{0}, occ_run{0};
     const uint32_t resident = stream_resident(k, smem, smem_set, occ);
@@ -1029,31 +1325,55 @@ void launch_band(spl_ctx *ctx, const spl_mat *a, const T *x, T *y, uint32_t x_lo
     attr[0].val.programmaticStreamSerializationAllowed = 1;
     cfg.attrs = attr;
     cfg.numAttrs = (ctx->pdl_prev && !std::getenv("SPL_NO_PDL")) ? 1 : 0;     // only behind another stream-kernel product
-    SPL_CUDA(cudaLaunchKernelEx(&cfg, k, (const uint32_t *)a->ptr, (const uint32_t *)a->ind,
-                                static_cast<const T *>(a->val), x, y, (const uint32_t *)a->stream_cta_rows,
-                                (const uint32_t *)a->stream_tile_lo, (const uint32_t *)a->stream_tile_reg,
-                                a->stream_max_tiles, val_cap, x_cap, stages, x_lo, x_hi,
-                                env_int("SPL_STREAM_L2HINT", 1), row_pattern(a)));
+    const int l2_hint = env_int("SPL_STREAM_L2HINT", 1);
+    if constexpr (CODES)
+        SPL_CUDA(cudaLaunchKernelEx(&cfg, k, (const uint32_t *)a->ptr, (const uint32_t *)a->ind,
+                                    static_cast<const T *>(a->val), (const uint8_t *)a->val_codes,
+                                    static_cast<const T *>(a->code_dict), a->code_count, x, y,
+                                    (const uint32_t *)a->stream_cta_rows, (const uint32_t *)a->stream_tile_lo,
+                                    (const uint32_t *)a->stream_tile_reg, a->stream_max_tiles, val_cap, x_cap, stages,
+                                    x_lo, x_hi, l2_hint, row_pattern(a)));
+    else
+        SPL_CUDA(cudaLaunchKernelEx(&cfg, k, (const uint32_t *)a->ptr, (const uint32_t *)a->ind,
+                                    static_cast<const T *>(a->val), x, y, (const uint32_t *)a->stream_cta_rows,
+                                    (const uint32_t *)a->stream_tile_lo, (const uint32_t *)a->stream_tile_reg,
+                                    a->stream_max_tiles, val_cap, x_cap, stages, x_lo, x_hi, l2_hint, row_pattern(a)));
     check_launch(ctx, "spmv_band");
     ctx->pdl_chain = true;
 }
 
-template <typename T, int LPR>
+// The code kernel takes 4 entries per lane in flight: with 8 it needs more than the 56 registers four CTAs leave
+// (spills).  U sets no bit of y: a lane sums its positions in order either way.
+template <typename T, int LPR, bool CODES>
 void spmv_band_u(spl_ctx *ctx, const spl_mat *a, const T *x, T *y, uint32_t x_lo, uint32_t x_hi) {
-    if ((a->max_row_len + LPR - 1) / LPR > 4) launch_band<T, LPR, 8>(ctx, a, x, y, x_lo, x_hi);   // as spmv_stream_u
-    else launch_band<T, LPR, 4>(ctx, a, x, y, x_lo, x_hi);
+    if constexpr (CODES) launch_band<T, LPR, 4, true>(ctx, a, x, y, x_lo, x_hi);
+    else if ((a->max_row_len + LPR - 1) / LPR > 4) launch_band<T, LPR, 8, false>(ctx, a, x, y, x_lo, x_hi);   // as spmv_stream_u
+    else launch_band<T, LPR, 4, false>(ctx, a, x, y, x_lo, x_hi);
 }
 
+template <typename T, bool CODES>
+void spmv_band_c(spl_ctx *ctx, const spl_mat *a, const T *x, T *y, uint32_t x_lo, uint32_t x_hi) {
+    switch (a->plan_lanes) {
+        case 1: spmv_band_u<T, 1, CODES>(ctx, a, x, y, x_lo, x_hi); break;
+        case 2: spmv_band_u<T, 2, CODES>(ctx, a, x, y, x_lo, x_hi); break;
+        case 4: spmv_band_u<T, 4, CODES>(ctx, a, x, y, x_lo, x_hi); break;
+        case 8: spmv_band_u<T, 8, CODES>(ctx, a, x, y, x_lo, x_hi); break;
+        case 16: spmv_band_u<T, 16, CODES>(ctx, a, x, y, x_lo, x_hi); break;
+        default: spmv_band_u<T, 32, CODES>(ctx, a, x, y, x_lo, x_hi); break;
+    }
+}
+
+// the code kernel when the matrix has value codes (SPL_STREAM_BAND_CODES=0 turns it off for A/B measurements: no codes
+// are planned then) and two of its stages fit in shared memory (they do whenever three stages of the value kernel fit: a code stage is
+// the smaller one)
 template <typename T>
 void spmv_band(spl_ctx *ctx, const spl_mat *a, const T *x, T *y, uint32_t x_lo, uint32_t x_hi) {
-    switch (a->plan_lanes) {
-        case 1: spmv_band_u<T, 1>(ctx, a, x, y, x_lo, x_hi); break;
-        case 2: spmv_band_u<T, 2>(ctx, a, x, y, x_lo, x_hi); break;
-        case 4: spmv_band_u<T, 4>(ctx, a, x, y, x_lo, x_hi); break;
-        case 8: spmv_band_u<T, 8>(ctx, a, x, y, x_lo, x_hi); break;
-        case 16: spmv_band_u<T, 16>(ctx, a, x, y, x_lo, x_hi); break;
-        default: spmv_band_u<T, 32>(ctx, a, x, y, x_lo, x_hi); break;
-    }
+    if (env_int("SPL_STREAM_BAND_CODES", 1) != 0 &&
+        band_shape<T, true>(a, tile_rows(a->plan_lanes)).smem(2) <= kBandSmemMax &&
+        band_codes(ctx, const_cast<spl_mat *>(a)))
+        spmv_band_c<T, true>(ctx, a, x, y, x_lo, x_hi);
+    else
+        spmv_band_c<T, false>(ctx, a, x, y, x_lo, x_hi);
 }
 
 template <typename T>
@@ -1635,6 +1955,11 @@ void drop_value_copies(spl_ctx *ctx, spl_mat *m) {
     m->slice_val = nullptr;
     m->slice_entries = 0;
     m->slice_state.store(0, std::memory_order_release);
+    dfree(ctx, m->val_codes); dfree(ctx, m->code_dict);
+    m->val_codes = nullptr;
+    m->code_dict = nullptr;
+    m->code_count = 0;
+    m->code_state.store(0, std::memory_order_release);
 }
 
 namespace {

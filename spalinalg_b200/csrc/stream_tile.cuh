@@ -24,10 +24,11 @@ constexpr uint32_t stage_capacity(uint32_t max_window) { return (max_window + 6u
 
 // acc += the row's products over stage positions [p0, e): lane `sub` of LPR takes positions p0 + sub, p0 + sub + LPR,
 // ..., U of them in flight (all columns, then all U gathers of x, then the values).  Position j holds column
-// cols[j] + cadd and value vals[j]; gather(c) returns x[c].  A masked slot adds an explicit 0, never 0 * x (x may hold
-// an inf).  These lines fix the bits of y: the vector kernel takes a row's entries in the same lane order.
-template <typename T, int LPR, int U, typename G>
-__device__ __forceinline__ void tile_row_sum(T &acc, const uint32_t *cols, uint32_t cadd, const T *vals, uint32_t p0,
+// cols[j] + cadd and value vals(j) (an array read, or a dictionary read through a one-byte code); gather(c) returns
+// x[c].  A masked slot adds an explicit 0, never 0 * x (x may hold an inf).  These lines fix the bits of y: the
+// vector kernel takes a row's entries in the same lane order.
+template <typename T, int LPR, int U, typename V, typename G>
+__device__ __forceinline__ void tile_row_sum(T &acc, const uint32_t *cols, uint32_t cadd, V vals, uint32_t p0,
                                              uint32_t e, uint32_t sub, G gather) {
     for (uint32_t j = p0 + sub; j < e; j += U * LPR) {
         uint32_t c[U];
@@ -37,7 +38,7 @@ __device__ __forceinline__ void tile_row_sum(T &acc, const uint32_t *cols, uint3
 #pragma unroll
         for (int u = 0; u < U; ++u) xv[u] = c[u] != 0xffffffffu ? gather(c[u]) : (T)0;
 #pragma unroll
-        for (int u = 0; u < U; ++u) v[u] = j + u * LPR < e ? vals[j + u * LPR] : (T)0;
+        for (int u = 0; u < U; ++u) v[u] = j + u * LPR < e ? vals(j + u * LPR) : (T)0;
 #pragma unroll
         for (int u = 0; u < U; ++u) acc += j + u * LPR < e ? v[u] * xv[u] : (T)0;      // 0, never 0 * inf
     }
